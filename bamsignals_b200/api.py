@@ -10,11 +10,16 @@ CUDA library is missing or no GPU is present the calls raise.
   flagMask / tlenFilter helpers          R/wrappers.R:76-98
   CountSignals                           R/zzzCountSignals.R:27-113
   GRanges                                the slots parseRegions reads (src/bamsignals.cpp:92-135)
+
+Results on the GPU (beyond the R interface): `device=` on bamCount / bamProfile / bamCoverage, and `out=` (any int32
+device array with __cuda_array_interface__) on pileup_core / coverage_core / Stage, count straight into device memory
+through the bsg_*_device entry points; nothing of the result crosses PCIe.  torch is imported only for those.
 """
 from __future__ import annotations
 
 import ctypes as C
 import os
+import sys
 import warnings
 from dataclasses import dataclass
 from typing import List, Optional, Sequence
@@ -90,12 +95,27 @@ class GRanges:
 # ------------------------------------------------------------------------------------------------------------------
 # CountSignals container (R/zzzCountSignals.R)
 # ------------------------------------------------------------------------------------------------------------------
+def _is_tensor(x):
+    torch = sys.modules.get("torch")            # a tensor exists only if torch was imported: never import it here
+    return torch is not None and isinstance(x, torch.Tensor)
+
+
+def _pairs(v):
+    """(2, w) view [sense; antisense] of an interleaved slice [s_0, a_0, s_1, ...]: R's IntegerMatrix(2, w) memory order."""
+    return v.view(-1, 2).t() if _is_tensor(v) else v.reshape((2, -1), order="F")
+
+
+def _permute(a, axes):
+    return a.permute(*axes) if _is_tensor(a) else a.transpose(axes)
+
+
 class CountSignals:
     """List-like container: signal i is a (w,) int32 vector, or a (2, w) matrix [sense; antisense] when ss.
 
     The (2, w) matrices are Fortran-ordered views into the flat result buffer, i.e. the memory layout of R's
     IntegerMatrix(2, w) (src/bamsignals.cpp:178-181): [sense_0, antisense_0, sense_1, ...].  When built from the
-    library's flat result (`flat` + `offsets`) the per-region views are created on first use."""
+    library's flat result (`flat` + `offsets`) the per-region views are created on first use.  `flat` may be a torch
+    tensor (device=): the views, alignSignals and as_list are then tensors of the same shapes and element order."""
 
     rownames = ("sense", "antisense")
 
@@ -112,8 +132,8 @@ class CountSignals:
                     raise ValueError("signals must be vectors")
 
     def _view(self, i):
-        v = self._flat[self._offsets[i]:self._offsets[i + 1]]
-        return v.reshape((2, -1), order="F") if self.ss else v
+        v = self._flat[int(self._offsets[i]):int(self._offsets[i + 1])]
+        return _pairs(v) if self.ss else v
 
     @property
     def signals(self):
@@ -145,10 +165,14 @@ class CountSignals:
         if len(w) and (w != w[0]).any():
             raise ValueError("all signals must have the same width")
         if len(self) == 0:
-            return np.zeros((0,), dtype=np.int32)
+            return self._flat.new_zeros((0,)) if _is_tensor(self._flat) else np.zeros((0,), dtype=np.int32)
         if self._signals is None:                            # contiguous result: one reshape, no copies
-            a = self._flat.reshape((len(self), -1))
-            return a.T if not self.ss else a.reshape((len(self), -1, 2)).transpose(2, 1, 0)
+            R, w0 = len(self), int(w[0])
+            if not self.ss:
+                return _permute(self._flat.reshape((R, w0)), (1, 0))
+            return _permute(self._flat.reshape((R, w0, 2)), (2, 1, 0))
+        if _is_tensor(self._signals[0]):
+            return sys.modules["torch"].stack(self._signals, dim=-1)
         return np.stack(self._signals, axis=-1)              # [w, R] or [2, w, R] like simplify2array
 
     def __repr__(self):
@@ -254,6 +278,10 @@ def lib():
     L.bsg_coverage.argtypes = region_args + [i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                              i32p, i64p, C.POINTER(C.POINTER(C.c_int32)), C.POINTER(BsgOpts)]
     L.bsg_coverage.restype = C.c_int
+    L.bsg_pileup_device.argtypes = region_args + [i32p] + [C.c_int32] * 8 + [C.c_void_p, i64p, C.c_void_p, C.POINTER(BsgOpts)]
+    L.bsg_pileup_device.restype = C.c_int
+    L.bsg_coverage_device.argtypes = region_args + [i32p] + [C.c_int32] * 5 + [C.c_void_p, i64p, C.c_void_p, C.POINTER(BsgOpts)]
+    L.bsg_coverage_device.restype = C.c_int
     L.bsg_last_error.restype = C.c_char_p
     L.bsg_version.restype = C.c_char_p
     L.bsg_get_timings.argtypes = [C.POINTER(BsgTimings)]
@@ -268,6 +296,10 @@ def lib():
     L.bsg_pileup_staged.restype = C.c_int
     L.bsg_coverage_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 4 + [i32p, i64p]
     L.bsg_coverage_staged.restype = C.c_int
+    L.bsg_pileup_staged_device.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 7 + [C.c_void_p, i64p, C.c_void_p]
+    L.bsg_pileup_staged_device.restype = C.c_int
+    L.bsg_coverage_staged_device.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 4 + [C.c_void_p, i64p, C.c_void_p]
+    L.bsg_coverage_staged_device.restype = C.c_int
     L.bsg_stage_close.argtypes = [C.c_void_p]
     L.bsg_stage_close.restype = None
     L.bsg_debug_plan.argtypes = region_args + [C.c_int64, i64p, i64p, i64p, i32p, i32p, C.c_int64]
@@ -326,14 +358,73 @@ def timings() -> dict:
     return {f: getattr(t, f) for f, _ in BsgTimings._fields_ if f not in ("reserved", "pad")}
 
 
+def device_buffer(out, total):
+    """(pointer, stream) of a caller's device buffer for the bsg_*_device entry points.  `out` is anything with
+    __cuda_array_interface__ (a torch CUDA tensor, a CuPy array): one-dimensional, int32, C-contiguous, at least `total`
+    elements.  The stream is the one the library orders its writes after: torch's current stream for a tensor, else the
+    interface's `stream` entry (0, the legacy default stream, when absent)."""
+    if _is_tensor(out):
+        import torch
+        if not out.is_cuda:
+            raise TypeError(f"out must be a CUDA tensor, not one on {out.device}")
+        if out.dtype != torch.int32:
+            raise TypeError(f"out must be an int32 tensor, not {out.dtype}")
+        if out.dim() != 1:
+            raise ValueError(f"out must be one-dimensional, not of shape {tuple(out.shape)}")
+        if not out.is_contiguous():
+            raise ValueError("out must be C-contiguous")
+        if out.numel() < total:
+            raise ValueError(f"out has {out.numel()} elements, the result needs {total}")
+        return out.data_ptr(), torch.cuda.current_stream(out.device).cuda_stream
+    try:
+        cai = out.__cuda_array_interface__
+    except (AttributeError, TypeError):
+        raise TypeError("out must be a device array with __cuda_array_interface__ (a torch CUDA tensor, a CuPy array)") from None
+    if np.dtype(cai["typestr"]) != np.int32:
+        raise TypeError(f"out must be int32, not {np.dtype(cai['typestr'])}")
+    shape = tuple(cai["shape"])
+    if len(shape) != 1:
+        raise ValueError(f"out must be one-dimensional, not of shape {shape}")
+    strides = cai.get("strides")
+    if strides is not None and shape[0] > 1 and tuple(strides) != (4,):
+        raise ValueError("out must be C-contiguous")
+    if shape[0] < total:
+        raise ValueError(f"out has {shape[0]} elements, the result needs {total}")
+    ptr, readonly = cai["data"]
+    if readonly:
+        raise ValueError("out is read-only")
+    return ptr, cai.get("stream") or 0
+
+
+def _empty_on(device, gr, binsize, ss):
+    """The flat int32 result buffer of a call, allocated by torch on `device` (a torch.device, "cuda:1" or 1)."""
+    import torch
+    if not isinstance(gr, GRanges):
+        raise TypeError("must provide a GRanges object")             # src/bamsignals.cpp:94
+    dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
+    if dev.type != "cuda":
+        raise TypeError(f"device must be a CUDA device, not {dev}")
+    n = int(output_layout(gr.width, int(binsize), bool(ss))[-1])
+    return torch.empty(n, dtype=torch.int32, device=dev)
+
+
 def pileup_core(bampath, gr, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1,
-                pe_mid=False, maxgap=16385, opts: Optional[BsgOpts] = None, _lazy=False):
+                pe_mid=False, maxgap=16385, opts: Optional[BsgOpts] = None, _lazy=False, out=None):
     """The .Call('bamsignals_pileup_core') entry point (src/bamsignals.cpp:444-461); binsize <= 0 means bamCount.
-    Returns the R `List`: one flat vector / (2,R) matrix for bamCount, else one array per region."""
+    Returns the R `List`: one flat vector / (2,R) matrix for bamCount, else one array per region.
+    With `out` (a device array, see device_buffer) the flat result is written there on the GPU and `out` is returned."""
     m = marshal_regions(gr)
     off = output_layout(m.width, int(binsize), bool(ss))
-    flat = np.empty(int(off[-1]), dtype=np.int32)
     tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+    if out is not None:
+        ptr, stream = device_buffer(out, int(off[-1]))
+        _check(lib().bsg_pileup_device(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                       _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                       None if tl is None else _p(tl, C.c_int32), int(mapqual), int(binsize), int(shift),
+                                       int(bool(ss)), int(requiredF), int(filteredF), int(bool(pe_mid)), int(maxgap),
+                                       ptr, _p(off, C.c_int64), stream, None if opts is None else C.byref(opts)))
+        return (out, off) if _lazy else out
+    flat = np.empty(int(off[-1]), dtype=np.int32)
     rc = lib().bsg_pileup(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
                           _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
                           None if tl is None else _p(tl, C.c_int32), int(mapqual), int(binsize), int(shift),
@@ -349,12 +440,20 @@ def pileup_core(bampath, gr, tlen_filter, mapqual=0, binsize=1, shift=0, ss=Fals
 
 
 def coverage_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, maxgap=16385,
-                  opts: Optional[BsgOpts] = None, _lazy=False):
-    """The .Call('bamsignals_coverage_core') entry point (src/bamsignals.cpp:474-494)."""
+                  opts: Optional[BsgOpts] = None, _lazy=False, out=None):
+    """The .Call('bamsignals_coverage_core') entry point (src/bamsignals.cpp:474-494).  `out`: as for pileup_core."""
     m = marshal_regions(gr)
     off = output_layout(m.width, 1, False)
-    flat = np.empty(int(off[-1]), dtype=np.int32)
     tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+    if out is not None:
+        ptr, stream = device_buffer(out, int(off[-1]))
+        _check(lib().bsg_coverage_device(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                         _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                         None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
+                                         int(filteredF), int(bool(tspan)), int(maxgap), ptr, _p(off, C.c_int64), stream,
+                                         None if opts is None else C.byref(opts)))
+        return (out, off) if _lazy else out
+    flat = np.empty(int(off[-1]), dtype=np.int32)
     rc = lib().bsg_coverage(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
                             _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
                             None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF), int(filteredF),
@@ -369,7 +468,8 @@ def coverage_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1
 class Stage:
     """Resident session (bsg_stage_*): the byte ranges `gr` needs (with halo `ext_hint`) are fetched, inflated and
     uploaded once; every pileup()/coverage() call then runs the device path only.  want_output=False leaves the
-    result in HBM (kernel-only timing)."""
+    result in HBM (kernel-only timing); `out` (a device array, see device_buffer) receives it on the GPU and is
+    returned."""
 
     def __init__(self, bampath, gr, ext_hint=0, opts: Optional[BsgOpts] = None):
         self._m = marshal_regions(gr)
@@ -380,19 +480,31 @@ class Stage:
                                     _p(m.strand, C.c_int8), int(ext_hint), None if opts is None else C.byref(opts)))
 
     def pileup(self, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1, pe_mid=False,
-               want_output=True):
+               want_output=True, out=None):
         off = output_layout(self._m.width, int(binsize), bool(ss))
-        flat = np.empty(int(off[-1]), dtype=np.int32) if want_output else None
         tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+        if out is not None:
+            ptr, stream = device_buffer(out, int(off[-1]))
+            _check(lib().bsg_pileup_staged_device(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                                  int(binsize), int(shift), int(bool(ss)), int(requiredF), int(filteredF),
+                                                  int(bool(pe_mid)), ptr, _p(off, C.c_int64), stream))
+            return out
+        flat = np.empty(int(off[-1]), dtype=np.int32) if want_output else None
         _check(lib().bsg_pileup_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual), int(binsize),
                                        int(shift), int(bool(ss)), int(requiredF), int(filteredF), int(bool(pe_mid)),
                                        None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
         return flat
 
-    def coverage(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, want_output=True):
+    def coverage(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, want_output=True, out=None):
         off = output_layout(self._m.width, 1, False)
-        flat = np.empty(int(off[-1]), dtype=np.int32) if want_output else None
         tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+        if out is not None:
+            ptr, stream = device_buffer(out, int(off[-1]))
+            _check(lib().bsg_coverage_staged_device(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                                    int(requiredF), int(filteredF), int(bool(tspan)), ptr,
+                                                    _p(off, C.c_int64), stream))
+            return out
+        flat = np.empty(int(off[-1]), dtype=np.int32) if want_output else None
         _check(lib().bsg_coverage_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
                                          int(requiredF), int(filteredF), int(bool(tspan)),
                                          None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
@@ -431,12 +543,17 @@ def _trunc(x):
     return int(x)          # Rcpp's input_parameter<int> truncates R doubles
 
 
+# device=None: host numpy results (the R interface).  device= a torch device ("cuda:1", 1, torch.device): the result is
+# counted into a torch int32 tensor on that device (bsg_*_device) and stays there.
 def bamCount(bampath, gr, mapqual=0, shift=0, ss=False, paired_end=("ignore", "filter", "midpoint"),
-             tlenFilter=None, filteredFlag=-1, verbose=False, opts=None):
+             tlenFilter=None, filteredFlag=-1, verbose=False, opts=None, device=None):
     pe = _match_arg(paired_end, ("ignore", "filter", "midpoint"))
     bampath = os.path.expanduser(bampath)
+    out = None if device is None else _empty_on(device, gr, -1, ss)
     pu = pileup_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), -1, _trunc(shift), ss, flagMask(pe),
-                     _trunc(filteredFlag), pe == "midpoint", opts=opts)
+                     _trunc(filteredFlag), pe == "midpoint", opts=opts, out=out)
+    if out is not None:
+        return _pairs(out) if ss else out                                            # (R,) or the (2, R) view
     return pu[0]                                                                      # R/wrappers.R:118
 
 
@@ -454,7 +571,7 @@ def _tlen(tf, pe):
 
 
 def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=("ignore", "filter", "midpoint"),
-               tlenFilter=None, filteredFlag=-1, verbose=False, opts=None):
+               tlenFilter=None, filteredFlag=-1, verbose=False, opts=None, device=None):
     if binsize < 1:
         raise ValueError("provide a binsize greater or equal to 1")                  # R/wrappers.R:136-137
     if binsize > 1 and isinstance(gr, GRanges) and (gr.width % int(binsize) != 0).any():
@@ -462,15 +579,17 @@ def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=
                       "some bins will correspond to less than binsize basepairs")     # R/wrappers.R:138-141
     pe = _match_arg(paired_end, ("ignore", "filter", "midpoint"))
     bampath = os.path.expanduser(bampath)
+    out = None if device is None else _empty_on(device, gr, _trunc(binsize), ss)
     flat, off = pileup_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), _trunc(binsize), _trunc(shift), ss,
-                            flagMask(pe), _trunc(filteredFlag), pe == "midpoint", opts=opts, _lazy=True)
+                            flagMask(pe), _trunc(filteredFlag), pe == "midpoint", opts=opts, _lazy=True, out=out)
     return CountSignals(None, ss, flat=flat, offsets=off)
 
 
 def bamCoverage(bampath, gr, mapqual=0, paired_end=("ignore", "extend"), tlenFilter=None, filteredFlag=-1,
-                verbose=False, opts=None):
+                verbose=False, opts=None, device=None):
     pe = _match_arg(paired_end, ("ignore", "extend"))
     bampath = os.path.expanduser(bampath)
+    out = None if device is None else _empty_on(device, gr, 1, False)
     flat, off = coverage_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), flagMask(pe), _trunc(filteredFlag),
-                              pe == "extend", opts=opts, _lazy=True)
+                              pe == "extend", opts=opts, _lazy=True, out=out)
     return CountSignals(None, False, flat=flat, offsets=off)

@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <atomic>
 #include <climits>
+#include <cstddef>
 #include <condition_variable>
 #include <deque>
 #include <functional>
@@ -106,6 +107,7 @@ struct DeviceCtx {
     PinBuf h_scalars, h_out[kOutSlots], h_tiles, h_front, h_ovf[kOutSlots], h_pack_cnt;
     DevBuf g_pack[kOutSlots], g_pack_cnt;       // result narrowing (opts.result_pack): packed bytes per ring slot, overflow counters
     cudaEvent_t ev_d2h[kOutSlots] = {}, ev_front[2] = {}, ev_order = nullptr;
+    cudaEvent_t ev_caller = nullptr;            // device-output calls: the caller's stream at entry
     std::vector<cudaEvent_t> ev_pool;
     size_t ev_next = 0;
 
@@ -126,6 +128,7 @@ struct DeviceCtx {
             BSG_CUDA(cudaStreamCreateWithPriority(&s_hi, cudaStreamNonBlocking, hi_p));
         }
         BSG_CUDA(cudaEventCreateWithFlags(&ev_order, cudaEventDisableTiming));
+        BSG_CUDA(cudaEventCreateWithFlags(&ev_caller, cudaEventDisableTiming));
         for (int i = 0; i < kSlots; ++i) {
             BSG_CUDA(cudaEventCreateWithFlags(&ev_h2d[i], cudaEventDisableTiming));
             BSG_CUDA(cudaEventCreateWithFlags(&ev_free[i], cudaEventDisableTiming));
@@ -182,6 +185,7 @@ struct DeviceCtx {
         for (auto e : ev_pool) cudaEventDestroy(e);
         ev_pool.clear(); ev_next = 0;
         cudaStreamDestroy(s_copy); cudaStreamDestroy(s_comp); cudaStreamDestroy(s_aux); cudaStreamDestroy(s_walk); cudaStreamDestroy(s_walk2); cudaStreamDestroy(s_d2h); cudaStreamDestroy(s_hi); cudaEventDestroy(ev_order);
+        cudaEventDestroy(ev_caller);
         init = false;
     }
 };
@@ -394,14 +398,15 @@ struct Batch {
 // ---------------------------------------------------------------------------------------------------------------
 class Session {
 public:
+    // dev >= 0 overrides the device opts names (device-output calls run where the caller's buffer is)
     Session(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
-            const int32_t* loc, const int32_t* width, const int8_t* strand, const bsg_opts* opts)
+            const int32_t* loc, const int32_t* width, const int8_t* strand, const bsg_opts* opts, int dev = -1)
         : bamp_(open_bam(bampath)), bam_(*bamp_), opts_(effective_opts(opts)) {
         resolve_regions(bam_, R, seq_levels, n_levels, seq_idx, loc, width, strand, &rg_);
         int ndev = 0;
         if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1)
             fail(BSG_ECUDA, "no CUDA device available (libbamsignals_cuda has no CPU fallback)");
-        int dev = opts_.n_devices > 0 ? opts_.devices[0] : 0;
+        if (dev < 0) dev = opts_.n_devices > 0 ? opts_.devices[0] : 0;
         if (dev < 0 || dev >= ndev || dev >= 16) fail(BSG_EARG, "invalid CUDA device index");
         ctx_ = &g_ctx[dev];
         ctx_->ensure_init(dev);
@@ -651,6 +656,8 @@ public:
         }
     }
     // up: the stream the tile table is uploaded on (and waited for); not the compute stream once inflates are queued on it
+    // The tiles' out_off depends on where the kernels write: DeviceCtx::out in tile order, or the caller's device buffer
+    // in the caller's layout (use_device_output) - the cached table is only reused for the same kind.
     void prepare_tiles(Mode mode, int32_t binsize, int ss, const int64_t* out_offsets, cudaStream_t up = nullptr) {
         Nvtx r("bsg:tiles");
         DeviceCtx& c = *ctx_;
@@ -658,7 +665,8 @@ public:
         if (!up) up = c.s_comp;
         if (!out_offsets) fail(BSG_EARG, "out_offsets is required");
         if (tiles_valid_ && my_tiles_gen_ == c.tiles_gen && tiles_mode_ == mode && tiles_binsize_ == binsize && tiles_ss_ == ss &&
-            tiles_offsets_.size() == size_t(R + 1) && memcmp(tiles_offsets_.data(), out_offsets, size_t(R + 1) * 8) == 0)
+            tiles_caller_ == dev_out_.on && tiles_offsets_.size() == size_t(R + 1) &&
+            memcmp(tiles_offsets_.data(), out_offsets, size_t(R + 1) * 8) == 0)
             return;
         validate_layout(mode, binsize, ss, out_offsets);
         HostTiles& ht = ht_;
@@ -683,7 +691,7 @@ public:
             uint8_t* h = c.h_tiles.as<uint8_t>();
             memcpy(h, ht.rid.data(), nt * 4); memcpy(h + nt * 4, ht.loc.data(), nt * 4);
             memcpy(h + nt * 8, ht.len.data(), nt * 4); memcpy(h + nt * 12, ht.strand.data(), nt * 4);
-            memcpy(h + nt * 16, tile_dev_off_.data(), nt * 8);
+            memcpy(h + nt * 16, dev_out_.on ? ht.out_off.data() : tile_dev_off_.data(), nt * 8);
             BSG_CUDA(cudaMemcpyAsync(ti, h, nt * 16, cudaMemcpyHostToDevice, up));
             BSG_CUDA(cudaMemcpyAsync(tl, h + nt * 16, nt * 8, cudaMemcpyHostToDevice, up));
             BSG_CUDA(cudaStreamSynchronize(up));         // h_tiles is reused by the next call; the kernels that read the tiles are launched after this
@@ -691,7 +699,7 @@ public:
         my_tiles_gen_ = ++c.tiles_gen;
         n_tiles_ = nt;
         max_tile_ints_ = ht.max_tile_ints;
-        tiles_mode_ = mode; tiles_binsize_ = binsize; tiles_ss_ = ss;
+        tiles_mode_ = mode; tiles_binsize_ = binsize; tiles_ss_ = ss; tiles_caller_ = dev_out_.on;
         tiles_offsets_.assign(out_offsets, out_offsets + R + 1);
         tiles_valid_ = true;
     }
@@ -710,11 +718,16 @@ public:
         cnt_.active = true; cnt_.mode = mode; cnt_.fp = fp; cnt_.binsize = binsize; cnt_.ss = ss;
         cnt_.out = out; cnt_.out_offsets = out_offsets; cnt_.out_ptrs = out_ptrs;
         const int64_t total = out_offsets[R];
-        cnt_.want_output = want_output && total > 0;
+        cnt_.want_output = want_output && total > 0 && !dev_out_.on;
         if (cnt_.want_output && !out && !out_ptrs) fail(BSG_EARG, "either out or out_ptrs must be given");
         tm_.n_tiles = n_tiles_;
         tm_.out_elems = total;
-        c.out.ensure(size_t(total) * sizeof(int32_t) + 64);
+        if (dev_out_.on) {
+            cnt_.dst = dev_out_.ptr;
+        } else {
+            c.out.ensure(size_t(total) * sizeof(int32_t) + 64);
+            cnt_.dst = c.out.as<int32_t>();
+        }
         // (rid, end + ext) as one key, prefix-maxed over the tile order: tiles [0, t) are final iff final_key[t-1] <= frontier
         tile_final_key_.resize(size_t(n_tiles_));
         uint64_t run = 0;
@@ -747,14 +760,25 @@ public:
         if (n_tiles_ > cnt_.t_done) count_tiles(cnt_.t_done, n_tiles_);
         DeviceScalars* sc = c.scalars.as<DeviceScalars>();
         BSG_CUDA(cudaGetLastError());
-        BSG_CUDA(cudaMemcpyAsync(c.h_scalars.p, sc, sizeof(DeviceScalars), cudaMemcpyDeviceToHost, cnt_stream()));
+        double scalar_bytes = double(sizeof(DeviceScalars));
+        if (dev_out_.on) {
+            // nothing of the result comes back: only the header (status, candidates) and the used kept[] slots
+            DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
+            const size_t head = offsetof(DeviceScalars, pad2), pitch = kKeptStride * sizeof(unsigned long long);
+            BSG_CUDA(cudaMemcpyAsync(hs, sc, head, cudaMemcpyDeviceToHost, cnt_stream()));
+            BSG_CUDA(cudaMemcpy2DAsync(hs->kept, pitch, sc->kept, pitch, sizeof(unsigned long long), kKeptSlots,
+                                       cudaMemcpyDeviceToHost, cnt_stream()));
+            scalar_bytes = double(head + kKeptSlots * sizeof(unsigned long long));
+        } else {
+            BSG_CUDA(cudaMemcpyAsync(c.h_scalars.p, sc, sizeof(DeviceScalars), cudaMemcpyDeviceToHost, cnt_stream()));
+        }
         const double t_d2h = now_ms();
         stop_streamer(false);
         BSG_CUDA(cudaStreamSynchronize(cnt_stream()));
         BSG_CUDA(cudaStreamSynchronize(c.s_comp));
         hi_prio_ = false;
         tm_.ms_d2h = now_ms() - t_d2h;
-        tm_.bytes_d2h = os_bytes_ + double(sizeof(DeviceScalars));
+        tm_.bytes_d2h = os_bytes_ + scalar_bytes;
         cnt_.active = false;
         const DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
         check_status(hs->status);
@@ -770,6 +794,18 @@ public:
         finish_count();
     }
 
+    // Where the counting kernels of the next call write.  use_device_output: straight into the caller's device buffer
+    // d_out at the caller's offsets (no DeviceCtx::out, no result streamer, nothing of the result crosses PCIe); every
+    // library stream that writes d_out first waits for what `caller` had queued at this point (e.g. work on memory the
+    // caller's allocator just handed out again).  use_host_output: the default, DeviceCtx::out in tile order + streamer.
+    void use_device_output(int32_t* d_out, cudaStream_t caller) {
+        BSG_CUDA(cudaEventRecord(ctx_->ev_caller, caller));
+        dev_out_ = DeviceOutput{true, d_out};
+    }
+    void use_host_output() { dev_out_ = DeviceOutput{}; }
+    int device() const { return ctx_->dev; }
+    int64_t regions() const { return rg_.R; }
+
 private:
     struct CountState {
         bool active = false, want_output = false;
@@ -780,8 +816,10 @@ private:
         int32_t* out = nullptr;
         const int64_t* out_offsets = nullptr;
         int32_t* const* out_ptrs = nullptr;
+        int32_t* dst = nullptr;                  // what the counting kernels write: DeviceCtx::out or the caller's d_out
         int64_t rows_ready = 0, t_done = 0;
     };
+    struct DeviceOutput { bool on = false; int32_t* ptr = nullptr; };
     struct OutJob { int slot; int64_t t0, t1; cudaEvent_t computed; };
 
     cudaStream_t cnt_stream() const { return hi_prio_ ? ctx_->s_hi : ctx_->s_comp; }
@@ -805,12 +843,13 @@ private:
             BSG_CUDA(cudaEventRecord(sp.b, st));
             kt_.join.push_back(sp); kt_.launches += 1;
         }
+        if (dev_out_.on) BSG_CUDA(cudaStreamWaitEvent(st, c.ev_caller, 0));
         {
             Span sp{c.timing_event(), c.timing_event()};
             BSG_CUDA(cudaEventRecord(sp.a, st));
-            if (cnt_.mode == MODE_COUNT) launch_count(tt, n, c0, c1, cnt_.ss, c.out.as<int32_t>(), sc, st);
-            else if (cnt_.mode == MODE_PROFILE) launch_profile(tt, n, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, c.out.as<int32_t>(), sc, st);
-            else launch_coverage(tt, n, c0, c1, max_tile_ints_, c.out.as<int32_t>(), sc, st);
+            if (cnt_.mode == MODE_COUNT) launch_count(tt, n, c0, c1, cnt_.ss, cnt_.dst, sc, st);
+            else if (cnt_.mode == MODE_PROFILE) launch_profile(tt, n, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, cnt_.dst, sc, st);
+            else launch_coverage(tt, n, c0, c1, max_tile_ints_, cnt_.dst, sc, st);
             BSG_CUDA(cudaEventRecord(sp.b, st));
             kt_.count.push_back(sp); kt_.launches += 1;
             if (cnt_.want_output) ship_tiles(t0, t1, sp.b);
@@ -1574,7 +1613,8 @@ private:
     Error os_err_{0, ""};
     double os_wait_ms_ = 0, os_scatter_ms_ = 0, os_bytes_ = 0;
     // cached tiles
-    bool tiles_valid_ = false;
+    bool tiles_valid_ = false, tiles_caller_ = false;
+    DeviceOutput dev_out_;
     Mode tiles_mode_ = MODE_COUNT;
     int32_t tiles_binsize_ = 0;
     int tiles_ss_ = 0;
@@ -1713,6 +1753,52 @@ void validate_devices(const bsg_opts& o) {
             if (o.devices[a] == o.devices[b]) fail(BSG_EARG, "the same CUDA device is listed twice");
 }
 
+// Device-output calls (bsg_*_device): the device that owns d_out, or -1 when d_out is NULL and the layout is empty.
+// Everything the caller could get wrong is refused before anything is written.
+int output_device(const int32_t* d_out, int64_t R, const int64_t* out_offsets) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev < 1) {
+        cudaGetLastError();
+        fail(BSG_ECUDA, "no CUDA device available (libbamsignals_cuda has no CPU fallback)");
+    }
+    if (!out_offsets) fail(BSG_EARG, "out_offsets is required");
+    if (R < 0) fail(BSG_EARG, "negative region count");
+    if (!d_out) {
+        if (out_offsets[R] == 0) return -1;
+        fail(BSG_EARG, "d_out is NULL but the layout has " + std::to_string(out_offsets[R]) + " elements");
+    }
+    if (reinterpret_cast<uintptr_t>(d_out) & 3) fail(BSG_EARG, "d_out must be 4-byte aligned");
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, d_out) != cudaSuccess) {
+        cudaGetLastError();
+        fail(BSG_EARG, "d_out is not a pointer CUDA knows");
+    }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+        fail(BSG_EARG, std::string("d_out must be device or managed memory, not ") +
+                       (a.type == cudaMemoryTypeHost ? "page-locked host memory" : "unregistered host memory"));
+    return a.device;
+}
+
+// The device a bsg_*_device call runs on: the one that owns d_out; opts may name it, but only that one.
+int device_for_output(const int32_t* d_out, int64_t R, const int64_t* out_offsets, const bsg_opts* opts) {
+    const int dev = output_device(d_out, R, out_offsets);
+    const bsg_opts o = effective_opts(opts);
+    validate_devices(o);
+    if (o.n_devices > 1) fail(BSG_EARG, "device output runs on one device: n_devices must be 0 or 1");
+    if (o.n_devices == 1 && dev >= 0 && o.devices[0] != dev)
+        fail(BSG_EARG, "d_out is on CUDA device " + std::to_string(dev) + ", opts.devices[0] names device " + std::to_string(o.devices[0]));
+    return dev >= 0 ? dev : (o.n_devices == 1 ? o.devices[0] : 0);
+}
+
+// Device-output calls run with the buffer's device current - `stream` 0 is that device's legacy stream - and give the
+// calling thread its current device back when they return (a torch caller's current device must not change under it).
+struct KeepCurrentDevice {
+    int prev = -1;
+    KeepCurrentDevice() { if (cudaGetDevice(&prev) != cudaSuccess) { cudaGetLastError(); prev = -1; } }
+    ~KeepCurrentDevice() { if (prev >= 0) cudaSetDevice(prev); }
+    KeepCurrentDevice(const KeepCurrentDevice&) = delete;
+};
+
 template <class F>
 int guarded(F&& f) {
     try {
@@ -1745,6 +1831,13 @@ namespace {
 // open staged sessions: bsg_shutdown() ends them (their device memory and streams are about to go away); the handles stay
 // valid to pass to bsg_stage_close(), every other use is refused
 std::vector<bsg_stage*> g_stages;
+
+// the device that owns d_out must be the session's (-1: empty layout, nothing is written)
+void check_staged_output(const bsg_stage* st, const int32_t* d_out, const int64_t* out_offsets) {
+    const int dev = output_device(d_out, st->s->regions(), out_offsets);
+    if (dev >= 0 && dev != st->s->device())
+        fail(BSG_EARG, "d_out is on CUDA device " + std::to_string(dev) + ", the staged session on device " + std::to_string(st->s->device()));
+}
 }
 
 extern "C" {
@@ -1815,6 +1908,52 @@ int bsg_coverage(const char* bampath, int64_t R, const char* const* seq_levels, 
     });
 }
 
+int bsg_pileup_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                      const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                      int32_t mapqual, int32_t binsize, int32_t shift, int32_t ss, int32_t requiredF, int32_t filteredF,
+                      int32_t pe_mid, int32_t /*maxgap*/, int32_t* d_out, const int64_t* out_offsets, void* stream,
+                      const bsg_opts* opts) {
+    return guarded([&] {
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        const int dev = device_for_output(d_out, R, out_offsets, opts);
+        Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts, dev);
+        const int64_t ext = ext_pileup(tlen_filter, shift, pe_mid);
+        const Mode mode = binsize <= 0 ? MODE_COUNT : MODE_PROFILE;
+        s.start_plan(ext);
+        s.validate_layout(mode, binsize, ss != 0, out_offsets);
+        s.use_device_output(d_out, static_cast<cudaStream_t>(stream));
+        const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
+        s.defer_setup([&] { s.begin_count(mode, fp, binsize, ss != 0, ext, nullptr, out_offsets, nullptr, false, s.setup_stream()); });
+        s.stage(ext, false);
+        s.finish_count();
+        s.finish_timings(t0);
+        s.kick_page_locking();
+    });
+}
+
+int bsg_coverage_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                        const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                        int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t /*maxgap*/,
+                        int32_t* d_out, const int64_t* out_offsets, void* stream, const bsg_opts* opts) {
+    return guarded([&] {
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        const int dev = device_for_output(d_out, R, out_offsets, opts);
+        Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts, dev);
+        const int64_t ext = ext_coverage(tlen_filter, tspan);
+        s.start_plan(ext);
+        s.validate_layout(MODE_COVERAGE, 1, 0, out_offsets);
+        s.use_device_output(d_out, static_cast<cudaStream_t>(stream));
+        const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
+        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, 0, ext, nullptr, out_offsets, nullptr, false, s.setup_stream()); });
+        s.stage(ext, false);
+        s.finish_count();
+        s.finish_timings(t0);
+        s.kick_page_locking();
+    });
+}
+
 int64_t bsg_output_layout(int64_t R, const int32_t* width, int32_t binsize, int32_t ss, int64_t* offsets) {
     const int64_t mult = ss ? 2 : 1;
     int64_t acc = 0;
@@ -1852,6 +1991,7 @@ int bsg_pileup_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual
         const double t0 = now_ms();
         st->s->reset_counters();
         st->s->require_ext(ext_pileup(tlen_filter, shift, pe_mid));
+        st->s->use_host_output();
         st->s->prepare_tiles(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, binsize, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
         st->s->decode_resident(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, fp);
@@ -1868,10 +2008,53 @@ int bsg_coverage_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqu
         const double t0 = now_ms();
         st->s->reset_counters();
         st->s->require_ext(ext_coverage(tlen_filter, tspan));
+        st->s->use_host_output();
         st->s->prepare_tiles(MODE_COVERAGE, 1, 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
         st->s->decode_resident(MODE_COVERAGE, fp);
         st->s->count(MODE_COVERAGE, fp, 1, 0, out, out_offsets, nullptr, out != nullptr);
+        st->s->finish_timings(t0);
+    });
+}
+
+int bsg_pileup_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift,
+                             int32_t ss, int32_t requiredF, int32_t filteredF, int32_t pe_mid, int32_t* d_out,
+                             const int64_t* out_offsets, void* stream) {
+    if (!st) { g_err = "null stage"; return BSG_EARG; }
+    return guarded([&] {
+        if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        check_staged_output(st, d_out, out_offsets);
+        BSG_CUDA(cudaSetDevice(st->s->device()));
+        const Mode mode = binsize <= 0 ? MODE_COUNT : MODE_PROFILE;
+        st->s->reset_counters();
+        st->s->require_ext(ext_pileup(tlen_filter, shift, pe_mid));
+        st->s->use_device_output(d_out, static_cast<cudaStream_t>(stream));
+        st->s->prepare_tiles(mode, binsize, ss != 0, out_offsets);
+        const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
+        st->s->decode_resident(mode, fp);
+        st->s->count(mode, fp, binsize, ss != 0, nullptr, out_offsets, nullptr, false);
+        st->s->finish_timings(t0);
+    });
+}
+
+int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                               int32_t filteredF, int32_t tspan, int32_t* d_out, const int64_t* out_offsets, void* stream) {
+    if (!st) { g_err = "null stage"; return BSG_EARG; }
+    return guarded([&] {
+        if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        check_staged_output(st, d_out, out_offsets);
+        BSG_CUDA(cudaSetDevice(st->s->device()));
+        st->s->reset_counters();
+        st->s->require_ext(ext_coverage(tlen_filter, tspan));
+        st->s->use_device_output(d_out, static_cast<cudaStream_t>(stream));
+        st->s->prepare_tiles(MODE_COVERAGE, 1, 0, out_offsets);
+        const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
+        st->s->decode_resident(MODE_COVERAGE, fp);
+        st->s->count(MODE_COVERAGE, fp, 1, 0, nullptr, out_offsets, nullptr, false);
         st->s->finish_timings(t0);
     });
 }

@@ -338,6 +338,12 @@ __device__ __forceinline__ void copy_out(int32_t* __restrict__ dst, const int32_
     for (int k = head + 4 * body + threadIdx.x; k < n; k += blockDim.x) __stcs(dst + k, sm[k]);
 }
 
+// Position of an int32 destination inside its 16-byte line.  Taken from the ADDRESS, not from the offset: the base of a
+// caller's buffer (bsg_*_device) is only 4-byte aligned, e.g. a tensor slice big[1:].
+__device__ __forceinline__ int out_phase(const int32_t* dst) {
+    return int((reinterpret_cast<uintptr_t>(dst) >> 2) & 3);
+}
+
 // exact floor(n / d) for 0 <= n < 2^31 with a precomputed multiplier (host: magic_for())
 __device__ __forceinline__ uint32_t fast_div(uint32_t n, uint64_t magic, uint32_t shift) {
     return uint32_t((uint64_t(n) * magic) >> shift);
@@ -360,7 +366,7 @@ __global__ void __launch_bounds__(kThreads) k_profile(TileTable tiles, const int
     const int64_t off = tiles.out_off[tix];
     const int nbins = BIN1 ? len : int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize));
     const int nout = SS ? 2 * nbins : nbins;
-    int32_t* hist = smem + (off & 3);                      // same 16-byte phase as the destination
+    int32_t* hist = smem + out_phase(out + off);           // same 16-byte phase as the destination
     for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
     __syncthreads();
     for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
@@ -395,7 +401,7 @@ __global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const
     const int64_t off = tiles.out_off[tix];
     const int nbins = int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize));
     const int nout = SS ? 2 * nbins : nbins;
-    int32_t* hist = smem + (off & 3);
+    int32_t* hist = smem + out_phase(out + off);
     for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
     __syncthreads();
     const int lane = threadIdx.x & 31;
@@ -469,7 +475,7 @@ __global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const in
     const int32_t rend = loc + len;                          // region end, exclusive
     // d[j] <-> out[off + j]; d sits `ph` ints into the 16-byte aligned buffer so that shared and global addresses
     // have the same phase; the ph leading ints are zeros and simply take part in the scan.
-    const int ph = int(off & 3);
+    const int ph = out_phase(out + off);
     int32_t* d = smem + ph;
     const int total = ph + len;
     const int nquads = (total + 3) >> 2;

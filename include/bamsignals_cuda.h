@@ -27,6 +27,7 @@
  *                       ints, interleaved [sense_0, antisense_0, sense_1, ...] when ss (:172-191).  mult = ss ? 2 : 1.
  *   out_ptrs          : R pointers, out_ptrs[i] receives region i's slice (the R shim passes INTEGER(sig_i));
  *                       used when `out` is NULL.  out_offsets is still required (it carries the sizes).
+ * The *_device variants below write the same flat layout into the caller's DEVICE memory instead ("results on the GPU").
  *
  * Errors: functions return 0 or a negative BSG_E* code; bsg_last_error() returns the message (thread-local).  The
  * messages for BSG_EOPEN / BSG_ENOINDEX / BSG_ENOCHROM are the reference's own Rcpp::stop strings
@@ -126,6 +127,34 @@ int bsg_coverage(const char* bampath, int64_t R, const char* const* seq_levels, 
                  int32_t maxgap, int32_t* out, const int64_t* out_offsets, int32_t* const* out_ptrs,
                  const bsg_opts* opts);
 
+/* ---- results on the GPU: count into device memory the caller owns ------------------------------------------------
+ * bsg_pileup_device / bsg_coverage_device take the arguments of bsg_pileup / bsg_coverage up to maxgap and write the
+ * result into d_out instead of host memory, for callers that consume it on the device (a torch / CuPy tensor, ...).
+ *   Layout   d_out receives exactly bsg_output_layout()'s layout, as the host `out` does; out_offsets stays in host
+ *            memory and is validated the same way.  Every element of [0, out_offsets[R]) is written exactly once,
+ *            nothing outside it is touched.  d_out may be NULL only when out_offsets[R] == 0.
+ *   Device   the call runs on the device that owns d_out (cudaPointerGetAttributes).  BSG_EARG, before any write, for:
+ *            device or managed memory on another device than opts->devices[0] (opts with n_devices == 1);
+ *            n_devices > 1; host memory of any kind (page-locked, registered or not); a pointer that is not 4-byte
+ *            aligned.  Without a device: BSG_ECUDA ("no CUDA device").
+ *   Stream   `stream` is a cudaStream_t of that device (0 = the legacy default stream).  The library's writes to d_out
+ *            are ordered after everything queued on `stream` when the call begins (e.g. a kernel still using memory the
+ *            caller's allocator has just handed out again).  The call is synchronous like the others: when it returns,
+ *            every write to d_out is complete and the buffer may be used on any stream.
+ *   Transfer nothing of the result crosses PCIe: no pinned staging, no host scatter, opts->result_pack is ignored;
+ *            bsg_timings.bytes_d2h counts only the control scalars.  opts->stream_min_ints still decides when finished
+ *            tiles are counted while later batches are still inflating.
+ * Multi-device calls, out_ptrs and output types other than int32 have no device variant. */
+int bsg_pileup_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                      const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                      const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift, int32_t ss,
+                      int32_t requiredF, int32_t filteredF, int32_t pe_mid, int32_t maxgap,
+                      int32_t* d_out, const int64_t* out_offsets, void* stream, const bsg_opts* opts);
+int bsg_coverage_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                        const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                        const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
+                        int32_t maxgap, int32_t* d_out, const int64_t* out_offsets, void* stream, const bsg_opts* opts);
+
 /* allocateList's sizes (src/bamsignals.cpp:139-192): fills offsets[0..R], returns the total element count. */
 int64_t bsg_output_layout(int64_t R, const int32_t* width, int32_t binsize, int32_t ss, int64_t* offsets);
 
@@ -133,7 +162,9 @@ int64_t bsg_output_layout(int64_t R, const int32_t* width, int32_t binsize, int3
  * bsg_stage() fetches, inflates and uploads the byte ranges a region set needs and keeps the RAW record bytes and
  * record offsets resident in HBM.  bsg_pileup_staged()/bsg_coverage_staged() then run the device path only
  * (decode -> filter -> join -> count) and leave the result on the device unless `out` is given.  This is how the
- * kernel-only throughput is measured, and how an application amortises inflate over many parameter settings.
+ * kernel-only throughput is measured.  bsg_pileup_staged_device()/bsg_coverage_staged_device() write the result into
+ * the caller's device memory with the contract of bsg_pileup_device (d_out must be on the session's device): this is
+ * how an application amortises inflate over many parameter settings and keeps every result on the GPU.
  * ext_hint is the halo fetched around every region, the `ext` of src/bamsignals.cpp:457,487: a staged call needs
  * |shift| (+ tlen_filter[1] when pe_mid) for pileups and tlen_filter[1] when tspan for coverage; a call that needs
  * more than the session was staged with is refused with BSG_EARG instead of silently missing reads.
@@ -151,6 +182,11 @@ int bsg_pileup_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual
                       int32_t* out, const int64_t* out_offsets);
 int bsg_coverage_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
                         int32_t filteredF, int32_t tspan, int32_t* out, const int64_t* out_offsets);
+int bsg_pileup_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift,
+                             int32_t ss, int32_t requiredF, int32_t filteredF, int32_t pe_mid,
+                             int32_t* d_out, const int64_t* out_offsets, void* stream);
+int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                               int32_t filteredF, int32_t tspan, int32_t* d_out, const int64_t* out_offsets, void* stream);
 void bsg_stage_close(bsg_stage* st);
 
 /*

@@ -4,7 +4,8 @@
     compute-sanitizer --tool racecheck python tools/sanitize_smoke.py
 Covers K0a inflate, K0b CRC32, K0c walk (speculate / link / scan / write), K1 decode (pileup and coverage
 instantiations), K3 join, K4 count, K4 profile (binsize 1 and the aggregated binsize >= 4 kernel, ss and not), K5
-coverage, the result-narrowing kernels and the one-thread publishers; results are checked against the oracle so that a
+coverage, the result-narrowing kernels and the one-thread publishers, and (where torch is installed) the tile kernels writing
+into a caller's device buffer at every 16-byte phase (bsg_*_device); results are checked against the oracle so that a
 sanitizer-clean run is also a correct one.  (The device-inflate path is forced: a job this small would otherwise be
 inflated by the host pool.)"""
 import os
@@ -47,5 +48,29 @@ for rp in (0, 2):
     a, b = B.bamCoverage(bam, big, paired_end="extend", opts=o2).as_list(), O.bamCoverage(bam, big, paired_end="extend").as_list()
     assert all(np.array_equal(x, y) for x, y in zip(a, b))
     launches += B.timings()["n_launches"]
+# device output (bsg_*_device) into slices of every 16-byte phase of one allocation: the tile kernels place their shared
+# buffers and 128-bit stores by the destination ADDRESS, which a caller's buffer only guarantees to 4 bytes
+try:
+    import torch
+except ImportError:
+    torch = None
+if torch is not None:
+    import warnings
+    for fn, kw in (("bamProfile", dict(binsize=1, ss=True)), ("bamProfile", dict(binsize=5, ss=True)),
+                   ("bamProfile", dict(binsize=3)), ("bamCount", dict(ss=True)), ("bamCoverage", dict(paired_end="extend"))):
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            ref = getattr(O, fn)(bam, gr, **kw)
+        want = ref.ravel(order="F") if fn == "bamCount" else np.concatenate([x.ravel(order="F") for x in ref.as_list()])
+        args = B.core_args(fn, **kw)
+        buf = torch.full((len(want) + 8,), -7, dtype=torch.int32, device="cuda:0")
+        for k in range(4):
+            view = buf[k:k + len(want)]
+            if fn == "bamCoverage":
+                B.coverage_core(bam, gr, opts=opts, out=view, **args)
+            else:
+                B.pileup_core(bam, gr, opts=opts, out=view, **args)
+            assert np.array_equal(view.cpu().numpy(), want), (fn, kw, k)
+            launches += B.timings()["n_launches"]
 B.lib().bsg_shutdown()
 print(f"sanitize_smoke ok: {launches} kernel launches, results equal to the oracle")

@@ -49,7 +49,8 @@ struct WsCtl {
     uint8_t qn[2][kWsStreams];                       // tokens in q[buf] of every stream (<= 32)
     uint32_t pos[kWsStreams];                        // bytes materialised so far (owned by the stream's copy warp)
     uint32_t out_off[kWsStreams];
-    uint32_t produced[2][kWsDecWarps];               // did the decode warp hand over anything in round buf?
+    uint32_t produced[2][kWsDecWarps];               // did the decode warp hand over anything in round buf, or has it a
+                                                     // stream that is not finished?
     alignas(8) uint8_t stage[kWsCopyWarps][256];     // a copy warp's chunk of output being built (also its bitmap scratch)
 };
 constexpr size_t kWsSmem = sizeof(WsStream) * kWsStreams + sizeof(WsCtl);
@@ -409,7 +410,10 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_inflate_ws(const InflateBlock
                     }
                 }
                 ctl.qn[buf][s] = uint8_t(nq);
-                const bool any = __any_sync(FULL, nq > 0);
+                // a stream that is not finished keeps the generation going even when it handed over nothing this round (a
+                // non-final block that is empty, or whose end-of-block code starts the round); it consumes header bits or
+                // meets the end_bit check every round, so the loop stays finite on corrupt input
+                const bool any = __any_sync(FULL, nq > 0 || !fin);
                 if (lane == 0) ctl.produced[buf][wid] = any ? 1u : 0u;
             } else if (wid == kWsChainWarp) {
                 if (spec.offs) chain_follow(false, buf ^ 1, r > 0);
@@ -442,7 +446,8 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_inflate_ws(const InflateBlock
             bool more = false;
 #pragma unroll
             for (int w = 0; w < kWsDecWarps; ++w) more = more || ctl.produced[buf][w] != 0;
-            if (!more) break;                        // nothing was handed over in round r: round r - 1 was the last one
+            if (!more) break;                        // every stream finished and nothing was handed over in round r: round r - 1
+                                                     // was the last one with tokens
         }
         // every stream must have produced exactly ISIZE bytes
         if (threadIdx.x < kWsStreams && b0 + s < n_blocks && ctl.pos[s] != out_len) atomicOr(&sc->status, STATUS_BAD_DEFLATE);

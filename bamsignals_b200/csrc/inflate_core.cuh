@@ -203,8 +203,13 @@ uint32_t slow_entry(uint32_t v, const A& acc) {
     return 15u | kDistBad;
 }
 
+// Which literal/length and distance codes a block may use, as zlib (inftrees.c) decides it: not over-subscribed, and
+// complete - except a code whose codes all have length 1, i.e. a single code of one bit (or, for distances, no code at
+// all).  `left` is the unused code space after lengths 1..15, `nlong` the number of codes longer than one bit.
+BSG_HD bool code_accepted(int left, int nlong) { return left == 0 || nlong == 0; }
+
 // Serial table construction by the owning thread.  is_dist selects the entry format.  Returns false when the code
-// is over-subscribed.
+// is over-subscribed or incomplete (code_accepted).
 BSG_HD bool build_table(const uint8_t* lens, int n, uint16_t* primary, int bits, uint16_t* count, uint16_t* sorted, bool is_dist,
                         uint16_t* first_out, uint16_t* index_out) {
     const uint16_t unset = is_dist ? uint16_t(0) : uint16_t(kLitUnset);      // code length 0 = not in the primary table
@@ -213,8 +218,13 @@ BSG_HD bool build_table(const uint8_t* lens, int n, uint16_t* primary, int bits,
     for (int l = 0; l < 16; ++l) cnt[l] = 0;
     for (int s = 0; s < n; ++s) cnt[lens[s] & 15]++;
     cnt[0] = 0;
-    int left = 1, ok = 1;
-    for (int l = 1; l <= 15; ++l) { left = left * 2 - cnt[l]; if (left < 0) { ok = 0; left = 0; } }    // over-subscribed
+    int left = 1, ok = 1, nlong = 0;
+    for (int l = 1; l <= 15; ++l) {
+        left = left * 2 - cnt[l];
+        if (left < 0) { ok = 0; left = 0; }                                  // over-subscribed
+        nlong += l > 1 ? cnt[l] : 0;
+    }
+    ok = ok && code_accepted(left, nlong);
     int next[16], offs[16];
     next[0] = 0; offs[0] = 0; next[1] = 0; offs[1] = 0;
     for (int l = 1; l < 15; ++l) { next[l + 1] = (next[l] + cnt[l]) << 1; offs[l + 1] = offs[l] + cnt[l]; }
@@ -238,7 +248,8 @@ BSG_HD bool build_table(const uint8_t* lens, int n, uint16_t* primary, int bits,
 }
 
 // Literal/length tables of one block: 10-bit primary table + second-level tables for the longer codes.
-// Returns false when the code is over-subscribed or (corrupt input only) the second level overflows.
+// Returns false when the code is over-subscribed or incomplete (code_accepted) or (corrupt input only) the second
+// level overflows.
 BSG_HD bool build_lit_table(const uint8_t* lens, Tables& T) {
     constexpr int n = 288, kRoot = kLitBits;
     for (int i = 0; i < (1 << kRoot); ++i) T.lit[i] = uint16_t(kLitUnset);
@@ -246,8 +257,13 @@ BSG_HD bool build_lit_table(const uint8_t* lens, Tables& T) {
     for (int l = 0; l < 16; ++l) cnt[l] = 0;
     for (int s = 0; s < n; ++s) cnt[lens[s] & 15]++;
     cnt[0] = 0;
-    int left = 1, ok = 1;
-    for (int l = 1; l <= 15; ++l) { left = left * 2 - cnt[l]; if (left < 0) { ok = 0; left = 0; } }    // over-subscribed
+    int left = 1, ok = 1, nlong = 0;
+    for (int l = 1; l <= 15; ++l) {
+        left = left * 2 - cnt[l];
+        if (left < 0) { ok = 0; left = 0; }                                  // over-subscribed
+        nlong += l > 1 ? cnt[l] : 0;
+    }
+    ok = ok && code_accepted(left, nlong);
     if (!ok) return false;
     int first_code[16], next[16];
     first_code[0] = 0; first_code[1] = 0;
@@ -339,6 +355,10 @@ BSG_HD int read_block_header(BR& br, Tables& T, uint8_t* dlens, int* last) {
         for (int i = 0; i < 19; ++i) cnt[cll[i]]++;
         cnt[0] = 0;
         next[1] = 0;
+        // the code-length code must be complete (zlib refuses an incomplete one, even a single code): once the unused
+        // code space goes negative (over-subscribed) it stays negative
+        int cl_left = 1;
+        for (int l = 1; l <= 7; ++l) cl_left = cl_left * 2 - cnt[l];
         for (int l = 1; l < 7; ++l) next[l + 1] = (next[l] + cnt[l]) << 1;
         for (int i = 0; i < 128; ++i) cl[i] = 0;
         for (int s = 0; s < 19; ++s) {
@@ -347,7 +367,7 @@ BSG_HD int read_block_header(BR& br, Tables& T, uint8_t* dlens, int* last) {
             const uint32_t r = rev_bits(uint32_t(next[l]++), uint32_t(l));
             for (uint32_t k = r; k < 128; k += (1u << l)) cl[k] = uint8_t(s | (l << 5));
         }
-        if (nlit > 286 || ndist > 30) return 2;
+        if (nlit > 286 || ndist > 30 || cl_left != 0) return 2;
         const int total = nlit + ndist;
         int i = 0;
         while (i < total) {

@@ -14,6 +14,10 @@ CUDA library is missing or no GPU is present the calls raise.
 Results on the GPU (beyond the R interface): `device=` on bamCount / bamProfile / bamCoverage, and `out=` (any int32
 device array with __cuda_array_interface__) on pileup_core / coverage_core / Stage, count straight into device memory
 through the bsg_*_device entry points; nothing of the result crosses PCIe.  torch is imported only for those.
+
+Coverage as runs (beyond the R interface): `bamCoverage(..., runs=True)`, `coverage_runs_core` and
+`Stage.coverage_runs` return a CoverageRuns - run-length (length, value) pairs per region, counted on the GPU through
+bsg_coverage_runs, on the host or (device=) in torch tensors.
 """
 from __future__ import annotations
 
@@ -180,6 +184,51 @@ class CountSignals:
         return f"CountSignals object with {len(self)} {kind} signals"
 
 
+class CoverageRuns:
+    """bamCoverage as runs: region i's coverage (in region orientation) is lengths[offsets[i]:offsets[i+1]] bases of
+    values[offsets[i]:offsets[i+1]].  `lengths` / `values` are flat int32 numpy arrays or torch tensors on one device;
+    `offsets` is numpy int64 (R + 1).  Adjacent runs of a region differ in value, every length is >= 1, a zero-width
+    region has no runs.  The same thing as an RleList of GenomicAlignments::coverage, one Rle per region."""
+
+    def __init__(self, lengths, values, offsets):
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        if offsets.ndim != 1 or len(offsets) < 1 or offsets[0] != 0 or (np.diff(offsets) < 0).any():
+            raise ValueError("offsets must be a non-decreasing int64 vector that starts at 0")
+        if len(lengths) != offsets[-1] or len(values) != offsets[-1]:
+            raise ValueError(f"lengths and values must have offsets[-1] = {int(offsets[-1])} elements")
+        self.lengths, self.values, self.offsets = lengths, values, offsets
+
+    def __len__(self):
+        return len(self.offsets) - 1
+
+    def __getitem__(self, i):
+        if not isinstance(i, (int, np.integer)):
+            raise TypeError("CoverageRuns indices must be integers")
+        if i < 0 or i >= len(self):
+            raise IndexError("subscript out of bounds")
+        a, b = int(self.offsets[i]), int(self.offsets[i + 1])
+        return self.lengths[a:b], self.values[a:b]
+
+    def to_dense(self) -> CountSignals:
+        """The bamCoverage result these runs describe (a CountSignals over one flat buffer on the runs' device)."""
+        if _is_tensor(self.lengths):
+            torch = sys.modules["torch"]
+            lengths = self.lengths.long()
+            flat = torch.repeat_interleave(self.values, lengths)
+            ends = torch.zeros(len(lengths) + 1, dtype=torch.int64, device=lengths.device)
+            torch.cumsum(lengths, 0, out=ends[1:])
+            dense_off = ends[torch.from_numpy(self.offsets).to(lengths.device)].cpu().numpy()
+        else:
+            flat = np.repeat(self.values, self.lengths)
+            ends = np.zeros(len(self.lengths) + 1, dtype=np.int64)
+            np.cumsum(self.lengths, out=ends[1:])
+            dense_off = ends[self.offsets]
+        return CountSignals(None, False, flat=flat, offsets=dense_off)
+
+    def __repr__(self):
+        return f"CoverageRuns object with {len(self)} regions and {int(self.offsets[-1])} runs"
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # argument helpers (R/wrappers.R:76-98)
 # ------------------------------------------------------------------------------------------------------------------
@@ -300,6 +349,14 @@ def lib():
     L.bsg_pileup_staged_device.restype = C.c_int
     L.bsg_coverage_staged_device.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 4 + [C.c_void_p, i64p, C.c_void_p]
     L.bsg_coverage_staged_device.restype = C.c_int
+    L.bsg_coverage_runs.argtypes = region_args + [i32p] + [C.c_int32] * 5 + [i64p, C.POINTER(C.c_void_p), C.POINTER(BsgOpts)]
+    L.bsg_coverage_runs.restype = C.c_int
+    L.bsg_coverage_runs_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 4 + [i64p, C.POINTER(C.c_void_p)]
+    L.bsg_coverage_runs_staged.restype = C.c_int
+    L.bsg_runs_read.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.bsg_runs_read.restype = C.c_int
+    L.bsg_runs_free.argtypes = [C.c_void_p]
+    L.bsg_runs_free.restype = None
     L.bsg_stage_close.argtypes = [C.c_void_p]
     L.bsg_stage_close.restype = None
     L.bsg_debug_plan.argtypes = region_args + [C.c_int64, i64p, i64p, i64p, i32p, i32p, C.c_int64]
@@ -396,14 +453,21 @@ def device_buffer(out, total):
     return ptr, cai.get("stream") or 0
 
 
+def _cuda_device(device):
+    """`device` (a torch.device, "cuda:1" or 1) as a torch.device with an index; TypeError unless it is a CUDA device."""
+    import torch
+    dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
+    if dev.type != "cuda":
+        raise TypeError(f"device must be a CUDA device, not {dev}")
+    return dev if dev.index is not None else torch.device("cuda", torch.cuda.current_device())
+
+
 def _empty_on(device, gr, binsize, ss):
     """The flat int32 result buffer of a call, allocated by torch on `device` (a torch.device, "cuda:1" or 1)."""
     import torch
     if not isinstance(gr, GRanges):
         raise TypeError("must provide a GRanges object")             # src/bamsignals.cpp:94
-    dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
-    if dev.type != "cuda":
-        raise TypeError(f"device must be a CUDA device, not {dev}")
+    dev = _cuda_device(device)
     n = int(output_layout(gr.width, int(binsize), bool(ss))[-1])
     return torch.empty(n, dtype=torch.int32, device=dev)
 
@@ -465,6 +529,43 @@ def coverage_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1
     return split_signals(flat, off, False)
 
 
+def _take_runs(h, offsets, device):
+    """Copy a bsg_runs result into numpy arrays (device None) or torch tensors on `device`, then free it."""
+    try:
+        n = int(offsets[-1])
+        if device is None:
+            lengths, values = np.empty(n, dtype=np.int32), np.empty(n, dtype=np.int32)
+            _check(lib().bsg_runs_read(h, lengths.ctypes.data or None, values.ctypes.data or None, None))
+        else:
+            import torch
+            lengths = torch.empty(n, dtype=torch.int32, device=device)
+            values = torch.empty(n, dtype=torch.int32, device=device)
+            _check(lib().bsg_runs_read(h, lengths.data_ptr() or None, values.data_ptr() or None,
+                                       torch.cuda.current_stream(device).cuda_stream))
+    finally:
+        lib().bsg_runs_free(h)
+    return CoverageRuns(lengths, values, offsets)
+
+
+def coverage_runs_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, maxgap=16385,
+                       opts: Optional[BsgOpts] = None, device=None) -> CoverageRuns:
+    """coverage_core's arguments -> the coverage as runs (bsg_coverage_runs).  device=None: numpy arrays on the host;
+    device= a CUDA device: torch tensors there (the call runs on that device; only the offsets cross PCIe)."""
+    m = marshal_regions(gr)
+    dev = None if device is None else _cuda_device(device)
+    if dev is not None and opts is None:
+        opts = default_opts(devices=[dev.index])
+    tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+    offsets = np.zeros(m.R + 1, dtype=np.int64)
+    h = C.c_void_p()
+    _check(lib().bsg_coverage_runs(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                   _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                   None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
+                                   int(filteredF), int(bool(tspan)), int(maxgap), _p(offsets, C.c_int64), C.byref(h),
+                                   None if opts is None else C.byref(opts)))
+    return _take_runs(h, offsets, dev)
+
+
 class Stage:
     """Resident session (bsg_stage_*): the byte ranges `gr` needs (with halo `ext_hint`) are fetched, inflated and
     uploaded once; every pileup()/coverage() call then runs the device path only.  want_output=False leaves the
@@ -509,6 +610,17 @@ class Stage:
                                          int(requiredF), int(filteredF), int(bool(tspan)),
                                          None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
         return flat
+
+    def coverage_runs(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, device=None) -> CoverageRuns:
+        """coverage() as runs (bsg_coverage_runs_staged); device= must be the session's device."""
+        dev = None if device is None else _cuda_device(device)
+        tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+        offsets = np.zeros(self._m.R + 1, dtype=np.int64)
+        h = C.c_void_p()
+        _check(lib().bsg_coverage_runs_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                              int(requiredF), int(filteredF), int(bool(tspan)), _p(offsets, C.c_int64),
+                                              C.byref(h)))
+        return _take_runs(h, offsets, dev)
 
     def close(self):
         if self._h:
@@ -585,10 +697,15 @@ def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=
     return CountSignals(None, ss, flat=flat, offsets=off)
 
 
+# runs=True: the coverage as a CoverageRuns (run-length pairs per region) instead of a CountSignals; with device= its
+# arrays are torch tensors on that device.
 def bamCoverage(bampath, gr, mapqual=0, paired_end=("ignore", "extend"), tlenFilter=None, filteredFlag=-1,
-                verbose=False, opts=None, device=None):
+                verbose=False, opts=None, device=None, runs=False):
     pe = _match_arg(paired_end, ("ignore", "extend"))
     bampath = os.path.expanduser(bampath)
+    if runs:
+        return coverage_runs_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), flagMask(pe), _trunc(filteredFlag),
+                                  pe == "extend", opts=opts, device=device)
     out = None if device is None else _empty_on(device, gr, 1, False)
     flat, off = coverage_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), flagMask(pe), _trunc(filteredFlag),
                               pe == "extend", opts=opts, _lazy=True, out=out)

@@ -31,6 +31,21 @@
 #include "plan.h"
 #include "pool.h"
 
+// A run-length coverage result (bsg_coverage_runs): lengths[n] and values[n] in device memory on `dev`.
+struct bsg_runs {
+    int dev = -1;
+    int32_t* lengths = nullptr;
+    int32_t* values = nullptr;
+    int64_t n = 0;
+    bool live = false;                          // false once bsg_shutdown() has freed the arrays
+    void release() {
+        if (lengths || values) { cudaSetDevice(dev); cudaFree(lengths); cudaFree(values); cudaGetLastError(); }
+        lengths = values = nullptr;
+        live = false;
+    }
+    ~bsg_runs() { release(); }
+};
+
 namespace bsg {
 void write_sam_as_bam_and_index(const char* sampath, const char* bampath);      // bamwrite.cpp
 namespace {
@@ -98,13 +113,14 @@ struct DeviceCtx {
     PinBuf h_raw[kSlots], h_offs[kSlots];
     cudaEvent_t ev_h2d[kSlots] = {}, ev_free[kSlots] = {};
     DevBuf tab[2], c0, c1, tiles_i32, tiles_i64, out, scalars;
+    DevBuf runs_i32, runs_i64;                  // run-length coverage: per-tile and per-region scratch (RunTiles, run_off)
     uint64_t tiles_gen = 0;                     // bumped whenever a Session uploads tiles: a staged Session's cached tiles are
                                                 // only valid while no other call has replaced them on this device
     // GPU inflate: an upload ring of kUp slots (compressed bytes, descriptors, walk scratch) and two raw / offsets buffers
     DevBuf g_comp[kUp], g_blocks[kUp], g_crc[kUp], g_walkers[kUp], g_counts[kUp], g_base[kUp], g_wscr[kUp], g_spec[kUp], g_raw[2], g_offs[2], g_total;
     PinBuf h_total, h_desc[kUp];
     cudaEvent_t ev_pin[kSlots] = {}, ev_up[kUp] = {}, ev_total[kUp] = {}, ev_inflated[kUp] = {}, ev_crc[kUp] = {}, ev_gfree[2] = {};
-    PinBuf h_scalars, h_out[kOutSlots], h_tiles, h_front, h_ovf[kOutSlots], h_pack_cnt;
+    PinBuf h_scalars, h_out[kOutSlots], h_tiles, h_front, h_ovf[kOutSlots], h_pack_cnt, h_runs;
     DevBuf g_pack[kOutSlots], g_pack_cnt;       // result narrowing (opts.result_pack): packed bytes per ring slot, overflow counters
     cudaEvent_t ev_d2h[kOutSlots] = {}, ev_front[2] = {}, ev_order = nullptr;
     cudaEvent_t ev_caller = nullptr;            // device-output calls: the caller's stream at entry
@@ -169,6 +185,7 @@ struct DeviceCtx {
         }
         for (auto& b : tab) b.release();
         c0.release(); c1.release(); tiles_i32.release(); tiles_i64.release(); out.release(); scalars.release();
+        runs_i32.release(); runs_i64.release(); h_runs.release();
         h_scalars.release();
         for (int i = 0; i < kOutSlots; ++i) { h_out[i].release(); h_ovf[i].release(); g_pack[i].release(); cudaEventDestroy(ev_d2h[i]); }
         h_pack_cnt.release(); g_pack_cnt.release();
@@ -724,7 +741,7 @@ public:
         tm_.out_elems = total;
         if (dev_out_.on) {
             cnt_.dst = dev_out_.ptr;
-        } else {
+        } else if (!runs_.res) {
             c.out.ensure(size_t(total) * sizeof(int32_t) + 64);
             cnt_.dst = c.out.as<int32_t>();
         }
@@ -747,8 +764,8 @@ public:
         cnt_.rows_ready = rows;
         const uint64_t key = uint64_t(f_tid) << 32 | uint64_t(uint32_t(std::max(f_pos, 0)));
         const int64_t t_new = std::upper_bound(tile_final_key_.begin(), tile_final_key_.end(), key) - tile_final_key_.begin();
-        // worth a launch + copy only in decent portions
-        if (opts_.stream_min_ints < 0) return;
+        // worth a launch + copy only in decent portions; runs are counted at the end of the call
+        if (opts_.stream_min_ints < 0 || runs_.res) return;
         const int64_t min_ints = opts_.stream_min_ints > 0 ? opts_.stream_min_ints : (int64_t(4) << 20);
         if (t_new > cnt_.t_done && tile_dev_off_[t_new] - tile_dev_off_[cnt_.t_done] >= min_ints) count_tiles(cnt_.t_done, t_new);
     }
@@ -757,11 +774,11 @@ public:
         Nvtx r("bsg:finish_count+d2h");
         DeviceCtx& c = *ctx_;
         cnt_.rows_ready = n_rows_;
-        if (n_tiles_ > cnt_.t_done) count_tiles(cnt_.t_done, n_tiles_);
+        if (n_tiles_ > cnt_.t_done || runs_.res) count_tiles(cnt_.t_done, n_tiles_);      // runs: also without tiles
         DeviceScalars* sc = c.scalars.as<DeviceScalars>();
         BSG_CUDA(cudaGetLastError());
         double scalar_bytes = double(sizeof(DeviceScalars));
-        if (dev_out_.on) {
+        if (dev_out_.on || runs_.res) {
             // nothing of the result comes back: only the header (status, candidates) and the used kept[] slots
             DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
             const size_t head = offsetof(DeviceScalars, pad2), pitch = kKeptStride * sizeof(unsigned long long);
@@ -801,8 +818,20 @@ public:
     void use_device_output(int32_t* d_out, cudaStream_t caller) {
         BSG_CUDA(cudaEventRecord(ctx_->ev_caller, caller));
         dev_out_ = DeviceOutput{true, d_out};
+        runs_ = RunsOutput{};
     }
-    void use_host_output() { dev_out_ = DeviceOutput{}; }
+    void use_host_output() { dev_out_ = DeviceOutput{}; runs_ = RunsOutput{}; }
+    // The next call counts coverage as runs (count_runs) into `res`, and fills the caller's run_offsets[R + 1].
+    void use_runs_output(bsg_runs* res, int64_t* run_offsets) {
+        dev_out_ = DeviceOutput{};
+        runs_ = RunsOutput{res, run_offsets};
+    }
+    // bsg_output_layout() of bamCoverage for this session's regions: the tiles are cut from it
+    std::vector<int64_t> coverage_layout() const {
+        std::vector<int64_t> off(size_t(rg_.R) + 1, 0);
+        for (int64_t i = 0; i < rg_.R; ++i) off[i + 1] = off[i] + rg_.width[i];
+        return off;
+    }
     int device() const { return ctx_->dev; }
     int64_t regions() const { return rg_.R; }
 
@@ -820,6 +849,7 @@ private:
         int64_t rows_ready = 0, t_done = 0;
     };
     struct DeviceOutput { bool on = false; int32_t* ptr = nullptr; };
+    struct RunsOutput { bsg_runs* res = nullptr; int64_t* run_offsets = nullptr; };
     struct OutJob { int slot; int64_t t0, t1; cudaEvent_t computed; };
 
     cudaStream_t cnt_stream() const { return hi_prio_ ? ctx_->s_hi : ctx_->s_comp; }
@@ -843,6 +873,7 @@ private:
             BSG_CUDA(cudaEventRecord(sp.b, st));
             kt_.join.push_back(sp); kt_.launches += 1;
         }
+        if (runs_.res) { count_runs(tt, n, st); cnt_.t_done = t1; return; }
         if (dev_out_.on) BSG_CUDA(cudaStreamWaitEvent(st, c.ev_caller, 0));
         {
             Span sp{c.timing_event(), c.timing_event()};
@@ -855,6 +886,49 @@ private:
             if (cnt_.want_output) ship_tiles(t0, t1, sp.b);
         }
         cnt_.t_done = t1;
+    }
+
+    // Coverage as runs (DESIGN.md §10) over ALL tiles (t0 == 0, advance() never counts early): count pass + scans, the
+    // region spans come back (the only D2H besides the control scalars), the result is allocated at its exact size, then
+    // the write pass.  Device memory: 28 bytes per tile, 16 per region, 8 per run.
+    void count_runs(const TileTable& tt, int64_t nt, cudaStream_t st) {
+        DeviceCtx& c = *ctx_;
+        if (nt != n_tiles_) fail(BSG_EARG, "internal error: runs are counted over all tiles at once");
+        const int64_t R = rg_.R;
+        runs_tiles_.resize(size_t(nt) * 2);
+        for (int64_t t = 0; t < nt; ++t) {
+            const int64_t i = ht_.region[t];
+            runs_tiles_[t] = int32_t(i);
+            runs_tiles_[nt + t] = int32_t(ht_.out_off[t] - tiles_offsets_[i]);
+        }
+        c.runs_i32.ensure(size_t(nt) * 5 * sizeof(int32_t) + 64);
+        c.runs_i64.ensure((size_t(nt) + 3 * size_t(R) + 1) * sizeof(int64_t) + 64);
+        c.h_runs.ensure((size_t(R) + 1) * sizeof(int64_t));
+        int32_t* ri = c.runs_i32.as<int32_t>();
+        int64_t* rl = c.runs_i64.as<int64_t>();
+        const RunTiles rt{ri, ri + nt, ri + 2 * nt, ri + 3 * nt, ri + 4 * nt, rl, rl + nt, rl + nt + R};
+        int64_t* run_off = rl + nt + 2 * R;
+        Span sp{c.timing_event(), c.timing_event()};
+        BSG_CUDA(cudaEventRecord(sp.a, st));
+        if (nt) BSG_CUDA(cudaMemcpyAsync(ri, runs_tiles_.data(), size_t(nt) * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        if (R) BSG_CUDA(cudaMemsetAsync(rt.rfirst, 0, size_t(R) * 2 * sizeof(int64_t), st));
+        launch_coverage_runs(tt, nt, c.c0.as<int32_t>(), c.c1.as<int32_t>(), max_tile_ints_, rt, R, run_off, st);
+        BSG_CUDA(cudaMemcpyAsync(c.h_runs.p, run_off, (size_t(R) + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        BSG_CUDA(cudaStreamSynchronize(st));
+        BSG_CUDA(cudaGetLastError());
+        memcpy(runs_.run_offsets, c.h_runs.p, (size_t(R) + 1) * sizeof(int64_t));
+        bsg_runs& res = *runs_.res;
+        res.dev = c.dev;
+        res.n = runs_.run_offsets[R];
+        const size_t bytes = size_t(std::max<int64_t>(res.n, 1)) * sizeof(int32_t);
+        BSG_CUDA(cudaMalloc(&res.lengths, bytes));
+        BSG_CUDA(cudaMalloc(&res.values, bytes));
+        BSG_CUDA(cudaMemsetAsync(res.lengths, 0, bytes, st));
+        launch_coverage_runs_write(tt, nt, c.c0.as<int32_t>(), c.c1.as<int32_t>(), max_tile_ints_, rt, run_off, res.lengths, res.values, st);
+        BSG_CUDA(cudaEventRecord(sp.b, st));
+        kt_.count.push_back(sp); kt_.launches += nt ? 3 : 1;
+        tm_.out_elems = 2 * res.n;
+        os_bytes_ += double((R + 1) * int64_t(sizeof(int64_t)));
     }
 
     // ---- output streamer: D2H on its own stream into a pinned ring, a host thread scatters tiles to the caller ------------
@@ -1615,6 +1689,8 @@ private:
     // cached tiles
     bool tiles_valid_ = false, tiles_caller_ = false;
     DeviceOutput dev_out_;
+    RunsOutput runs_;
+    std::vector<int32_t> runs_tiles_;           // region, rel of every tile (uploaded by count_runs)
     Mode tiles_mode_ = MODE_COUNT;
     int32_t tiles_binsize_ = 0;
     int tiles_ss_ = 0;
@@ -1831,6 +1907,24 @@ namespace {
 // open staged sessions: bsg_shutdown() ends them (their device memory and streams are about to go away); the handles stay
 // valid to pass to bsg_stage_close(), every other use is refused
 std::vector<bsg_stage*> g_stages;
+
+// live run-length results: bsg_shutdown() frees their device memory, the handles stay valid for bsg_runs_free()
+std::vector<bsg_runs*> g_runs;
+
+// A bsg_runs_read destination: true for device (or managed) memory on the result's device, false for host memory.
+bool runs_destination(const int32_t* p, const bsg_runs* r, const char* what) {
+    if (!p) fail(BSG_EARG, std::string(what) + " is NULL");
+    if (reinterpret_cast<uintptr_t>(p) & 3) fail(BSG_EARG, std::string(what) + " must be 4-byte aligned");
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        fail(BSG_EARG, std::string(what) + " is not a pointer CUDA knows");
+    }
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return false;
+    if (a.device != r->dev)
+        fail(BSG_EARG, std::string(what) + " is on CUDA device " + std::to_string(a.device) + ", the result on device " + std::to_string(r->dev));
+    return true;
+}
 
 // the device that owns d_out must be the session's (-1: empty layout, nothing is written)
 void check_staged_output(const bsg_stage* st, const int32_t* d_out, const int64_t* out_offsets) {
@@ -2059,6 +2153,90 @@ int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_
     });
 }
 
+int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                      const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                      int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t /*maxgap*/,
+                      int64_t* run_offsets, bsg_runs** runs, const bsg_opts* opts) {
+    if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
+    *runs = nullptr;
+    return guarded([&] {
+        const double t0 = now_ms();
+        const bsg_opts o = effective_opts(opts);
+        validate_devices(o);
+        if (o.n_devices > 1) fail(BSG_EARG, "run-length coverage runs on one device: n_devices must be 0 or 1");
+        if (!run_offsets) fail(BSG_EARG, "run_offsets is required");
+        KeepCurrentDevice keep;
+        Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts);
+        const int64_t ext = ext_coverage(tlen_filter, tspan);
+        const std::vector<int64_t> dense = s.coverage_layout();
+        s.start_plan(ext);
+        auto res = std::make_unique<bsg_runs>();
+        s.use_runs_output(res.get(), run_offsets);
+        const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
+        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, 0, ext, nullptr, dense.data(), nullptr, false, s.setup_stream()); });
+        s.stage(ext, false);
+        s.finish_count();
+        s.finish_timings(t0);
+        s.kick_page_locking();
+        res->live = true;
+        g_runs.push_back(res.get());
+        *runs = res.release();
+    });
+}
+
+int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF,
+                             int32_t tspan, int64_t* run_offsets, bsg_runs** runs) {
+    if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
+    *runs = nullptr;
+    if (!st) { g_err = "null stage"; return BSG_EARG; }
+    return guarded([&] {
+        if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
+        if (!run_offsets) fail(BSG_EARG, "run_offsets is required");
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        BSG_CUDA(cudaSetDevice(st->s->device()));
+        st->s->reset_counters();
+        st->s->require_ext(ext_coverage(tlen_filter, tspan));
+        auto res = std::make_unique<bsg_runs>();
+        st->s->use_runs_output(res.get(), run_offsets);
+        const std::vector<int64_t> dense = st->s->coverage_layout();
+        st->s->prepare_tiles(MODE_COVERAGE, 1, 0, dense.data());
+        const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
+        st->s->decode_resident(MODE_COVERAGE, fp);
+        st->s->count(MODE_COVERAGE, fp, 1, 0, nullptr, dense.data(), nullptr, false);
+        st->s->finish_timings(t0);
+        st->s->use_host_output();
+        res->live = true;
+        g_runs.push_back(res.get());
+        *runs = res.release();
+    });
+}
+
+int bsg_runs_read(const bsg_runs* runs, int32_t* lengths, int32_t* values, void* stream) {
+    if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
+    return guarded([&] {
+        if (!runs->live) fail(BSG_EARG, "this result was freed by bsg_shutdown()");
+        if (runs->n == 0) return;
+        KeepCurrentDevice keep;
+        const bool dev_l = runs_destination(lengths, runs, "lengths"), dev_v = runs_destination(values, runs, "values");
+        BSG_CUDA(cudaSetDevice(runs->dev));
+        // on the caller's stream: ordered after what it has queued; synchronous like every call
+        cudaStream_t s = static_cast<cudaStream_t>(stream);
+        const size_t bytes = size_t(runs->n) * sizeof(int32_t);
+        BSG_CUDA(cudaMemcpyAsync(lengths, runs->lengths, bytes, dev_l ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
+        BSG_CUDA(cudaMemcpyAsync(values, runs->values, bytes, dev_v ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
+        BSG_CUDA(cudaStreamSynchronize(s));
+    });
+}
+
+void bsg_runs_free(bsg_runs* runs) {
+    if (!runs) return;
+    std::lock_guard<std::mutex> g(g_mu);
+    g_runs.erase(std::remove(g_runs.begin(), g_runs.end(), runs), g_runs.end());
+    KeepCurrentDevice keep;
+    delete runs;
+}
+
 void bsg_stage_close(bsg_stage* st) {
     if (!st) return;
     std::lock_guard<std::mutex> g(g_mu);
@@ -2084,6 +2262,10 @@ void bsg_shutdown(void) {
     std::lock_guard<std::mutex> g(g_mu);
     stop_pin_thread();
     for (bsg_stage* st : g_stages) st->s.reset();
+    {
+        KeepCurrentDevice keep;
+        for (bsg_runs* r : g_runs) r->release();
+    }
     for (auto& c : g_ctx) c.release();
     g_pool.reset();
     g_bams.clear();

@@ -463,25 +463,11 @@ __global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const
 // across the whole CTA with three barriers per chunk: ncu showed the kernel issue-bound - 66 % of the issue slots, 2.5 TB/s
 // of DRAM traffic - on ~6 k warp instructions per tile, half of them the scan.)
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const int32_t* __restrict__ c0,
-                                                       const int32_t* __restrict__ c1, int32_t* __restrict__ out) {
-    extern __shared__ __align__(16) int32_t smem[];
-    __shared__ int32_t s_warp[kThreads / 32];
-    const int64_t tix = blockIdx.x;
-    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
-    const bool neg_region = tiles.strand[tix] < 0;
-    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
-    const int64_t off = tiles.out_off[tix];
+// The tile's difference array d[0, len): +1 where a read's interval begins (a start before the tile is clamped into
+// d[0]), -1 behind where it ends (an end past the tile is dropped).  Shared by k_coverage and the run-length kernels.
+__device__ __forceinline__ void scatter_coverage(int32_t* d, int32_t loc, int32_t len, bool neg_region, int64_t lo, int64_t hi,
+                                                 const int32_t* __restrict__ c0, const int32_t* __restrict__ c1) {
     const int32_t rend = loc + len;                          // region end, exclusive
-    // d[j] <-> out[off + j]; d sits `ph` ints into the 16-byte aligned buffer so that shared and global addresses
-    // have the same phase; the ph leading ints are zeros and simply take part in the scan.
-    const int ph = out_phase(out + off);
-    int32_t* d = smem + ph;
-    const int total = ph + len;
-    const int nquads = (total + 3) >> 2;
-    int4* s4 = reinterpret_cast<int4*>(smem);
-    for (int k = threadIdx.x; k < nquads; k += kThreads) s4[k] = make_int4(0, 0, 0, 0);
-    __syncthreads();
     for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
         const int32_t s = __ldg(c0 + i), e = __ldg(c1 + i);
         if (s >= rend || e < loc) continue;                  // src/bamsignals.cpp:420 (dropped reads: s = INT_MAX)
@@ -491,6 +477,27 @@ __global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const in
         atomicAdd(&d[up > 0 ? up : 0], 1);
         if (down < len) atomicAdd(&d[down], -1);
     }
+}
+
+__global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const int32_t* __restrict__ c0,
+                                                       const int32_t* __restrict__ c1, int32_t* __restrict__ out) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_warp[kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const bool neg_region = tiles.strand[tix] < 0;
+    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
+    const int64_t off = tiles.out_off[tix];
+    // d[j] <-> out[off + j]; d sits `ph` ints into the 16-byte aligned buffer so that shared and global addresses
+    // have the same phase; the ph leading ints are zeros and simply take part in the scan.
+    const int ph = out_phase(out + off);
+    int32_t* d = smem + ph;
+    const int total = ph + len;
+    const int nquads = (total + 3) >> 2;
+    int4* s4 = reinterpret_cast<int4*>(smem);
+    for (int k = threadIdx.x; k < nquads; k += kThreads) s4[k] = make_int4(0, 0, 0, 0);
+    __syncthreads();
+    scatter_coverage(d, loc, len, neg_region, lo, hi, c0, c1);
     __syncthreads();
     // pass 1: every warp scans its own contiguous part in place (cumsum, src/bamsignals.cpp:464-470)
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -533,6 +540,178 @@ __global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const in
             if (j + 3 >= ph && j + 3 < total) __stcs(dst + j + 3, v.w);
         }
     }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// K5r bamCoverage as runs (DESIGN.md §10).  Inside a tile the coverage v[j] changes exactly where d[j] != 0 (j >= 1), its
+// first value is d[0] and its last value the sum of d: a tile's runs follow from the difference array without a scan.
+//   k_runs_count  per tile: nnz = #{j in [1, len): d[j] != 0}, first = d[0], last = sum(d)
+//   k_runs_scan   tile t holds runs(t) = nnz(t) + (t opens its region || first(t) != last(t-1)) run starts; one CTA
+//                 scans them over the tiles, then over the regions (caller order) -> run_off[R + 1]
+//   k_runs_write  scatter + scan again, write every run start's value at its index; lengths are end - start, added up
+//                 with atomics from the two places that know them (the run's own start, and the next run's start or
+//                 the region's end), into a zeroed buffer
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(kThreads) k_runs_count(TileTable tiles, const int32_t* __restrict__ c0,
+                                                         const int32_t* __restrict__ c1, RunTiles rt) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_nz[kThreads / 32], s_sum[kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    for (int k = threadIdx.x; k < len; k += kThreads) smem[k] = 0;
+    __syncthreads();
+    scatter_coverage(smem, loc, len, tiles.strand[tix] < 0, tiles.cand_lo[tix], tiles.cand_hi[tix], c0, c1);
+    __syncthreads();
+    int nz = 0, sum = 0;
+    for (int j = threadIdx.x; j < len; j += kThreads) {
+        const int32_t v = smem[j];
+        sum += v;
+        nz += int(j > 0 && v != 0);
+    }
+    nz = __reduce_add_sync(FULL, nz);
+    sum = __reduce_add_sync(FULL, sum);
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    if (lane == 0) { s_nz[wid] = nz; s_sum[wid] = sum; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int tn = 0, ts = 0;
+        for (int k = 0; k < kThreads / 32; ++k) { tn += s_nz[k]; ts += s_sum[k]; }
+        rt.nnz[tix] = tn;
+        rt.first[tix] = smem[0];
+        rt.last[tix] = ts;
+    }
+}
+
+// Exclusive prefix of v over the CTA (1024 threads, blockDim.x == kScanThreads); *total receives the sum.
+constexpr int kScanThreads = 1024;
+__device__ __forceinline__ long long block_exclusive_scan(long long v, long long* total) {
+    __shared__ long long s_w[kScanThreads / 32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    long long incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long up = __shfl_up_sync(FULL, incl, o);
+        if (lane >= o) incl += up;
+    }
+    if (lane == 31) s_w[wid] = incl;
+    __syncthreads();
+    long long before = 0, all = 0;
+    for (int k = 0; k < kScanThreads / 32; ++k) {
+        const long long w = s_w[k];
+        if (k < wid) before += w;
+        all += w;
+    }
+    __syncthreads();                                        // s_w may be reused by the next call
+    *total = all;
+    return before + incl - v;
+}
+
+__device__ __forceinline__ int64_t tile_runs(const RunTiles& rt, int64_t t) {
+    const bool head = t == 0 || rt.region[t - 1] != rt.region[t];
+    return int64_t(rt.nnz[t]) + int64_t(head || rt.first[t] != rt.last[t - 1]);
+}
+
+// One CTA.  Every thread walks a contiguous chunk of tiles, then of regions (a few hundred thousand of either take
+// tens of microseconds: not worth a multi-CTA scan).
+__global__ void __launch_bounds__(kScanThreads) k_runs_scan(RunTiles rt, int64_t n_tiles, int64_t R, int64_t* __restrict__ run_off) {
+    long long total = 0;
+    {
+        const int64_t per = (n_tiles + kScanThreads - 1) / kScanThreads;
+        const int64_t t0 = min(n_tiles, per * int64_t(threadIdx.x)), t1 = min(n_tiles, t0 + per);
+        long long mine = 0;
+        for (int64_t t = t0; t < t1; ++t) mine += tile_runs(rt, t);
+        long long run = block_exclusive_scan(mine, &total);
+        for (int64_t t = t0; t < t1; ++t) {
+            const int32_t reg = rt.region[t];
+            if (t == 0 || rt.region[t - 1] != reg) rt.rfirst[reg] = run;
+            rt.toff[t] = run;
+            run += tile_runs(rt, t);
+            if (t + 1 == n_tiles || rt.region[t + 1] != reg) rt.rlast[reg] = run;
+        }
+    }
+    __syncthreads();                                        // rfirst / rlast of every region are written
+    const int64_t per = (R + kScanThreads - 1) / kScanThreads;
+    const int64_t i0 = min(R, per * int64_t(threadIdx.x)), i1 = min(R, i0 + per);
+    long long mine = 0;
+    for (int64_t i = i0; i < i1; ++i) mine += rt.rlast[i] - rt.rfirst[i];
+    long long run = block_exclusive_scan(mine, &total);
+    for (int64_t i = i0; i < i1; ++i) { run_off[i] = run; run += rt.rlast[i] - rt.rfirst[i]; }
+    if (threadIdx.x == 0) run_off[R] = total;
+}
+
+__global__ void __launch_bounds__(kThreads) k_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* __restrict__ c0,
+                                                         const int32_t* __restrict__ c1, RunTiles rt,
+                                                         const int64_t* __restrict__ run_off, int32_t* __restrict__ lengths,
+                                                         int32_t* __restrict__ values) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_sum[kThreads / 32], s_cnt[kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const int32_t reg = rt.region[tix], rel = rt.rel[tix];
+    const bool head = tix == 0 || rt.region[tix - 1] != reg;
+    const bool tail = tix + 1 == n_tiles || rt.region[tix + 1] != reg;
+    const bool start0 = head || rt.first[tix] != rt.last[tix - 1];      // a run starts at the tile's first base
+    const int64_t kbeg = run_off[reg], kend = run_off[reg + 1];
+    const int64_t k0 = kbeg + (rt.toff[tix] - rt.rfirst[reg]);        // index of the tile's first run start
+    const int nquads = (len + 3) >> 2;
+    int4* s4 = reinterpret_cast<int4*>(smem);
+    for (int k = threadIdx.x; k < nquads; k += kThreads) s4[k] = make_int4(0, 0, 0, 0);
+    __syncthreads();
+    scatter_coverage(smem, loc, len, tiles.strand[tix] < 0, tiles.cand_lo[tix], tiles.cand_hi[tix], c0, c1);
+    __syncthreads();
+    // every warp owns a contiguous part of the tile (as in k_coverage): pass 1 sums its d and counts its run starts,
+    // pass 2 adds what the warps in front of it have and writes the runs
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    constexpr int kWarps = kThreads / 32;
+    const int qpw = ((nquads + kWarps - 1) / kWarps + 31) & ~31;
+    const int q_lo = wid * qpw, q_hi = min(nquads, q_lo + qpw);
+    auto flags = [&](int q, const int4& v) {                // bit e: a run starts at 4q + e
+        const int j = 4 * q;
+        return (j < len && (j == 0 ? start0 : v.x != 0) ? 1u : 0u) | (j + 1 < len && v.y != 0 ? 2u : 0u) |
+               (j + 2 < len && v.z != 0 ? 4u : 0u) | (j + 3 < len && v.w != 0 ? 8u : 0u);
+    };
+    int wsum = 0, wcnt = 0;
+    for (int q0 = q_lo; q0 < q_hi; q0 += 32) {
+        const int q = q0 + lane;
+        int4 v = make_int4(0, 0, 0, 0);
+        if (q < q_hi) v = s4[q];
+        wsum += __reduce_add_sync(FULL, v.x + v.y + v.z + v.w);
+        wcnt += __reduce_add_sync(FULL, q < q_hi ? __popc(flags(q, v)) : 0);
+    }
+    if (lane == 0) { s_sum[wid] = wsum; s_cnt[wid] = wcnt; }
+    __syncthreads();
+    int val = 0, cnt = 0;
+    for (int k = 0; k < wid; ++k) { val += s_sum[k]; cnt += s_cnt[k]; }
+    for (int q0 = q_lo; q0 < q_hi; q0 += 32) {
+        const int q = q0 + lane;
+        int4 v = make_int4(0, 0, 0, 0);
+        if (q < q_hi) v = s4[q];
+        const unsigned f = q < q_hi ? flags(q, v) : 0u;
+        int isum = v.x + v.y + v.z + v.w, icnt = __popc(f);
+        const int qs = isum, qc = icnt;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int us = __shfl_up_sync(FULL, isum, o), uc = __shfl_up_sync(FULL, icnt, o);
+            if (lane >= o) { isum += us; icnt += uc; }
+        }
+        int x = val + isum - qs;                            // coverage just before 4q
+        int64_t k = k0 + cnt + icnt - qc;                   // index of the next run start
+        const int e4[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            x += e4[e];
+            if (f >> e & 1u) {
+                const int32_t p = rel + 4 * q + e;          // run start, relative to the region in its orientation
+                values[k] = x;
+                atomicAdd(&lengths[k], -p);
+                if (k > kbeg) atomicAdd(&lengths[k - 1], p);
+                ++k;
+            }
+        }
+        val += __shfl_sync(FULL, isum, 31);
+        cnt += __shfl_sync(FULL, icnt, 31);
+    }
+    if (tail && threadIdx.x == 0 && kend > kbeg) atomicAdd(&lengths[kend - 1], rel + len);     // the region's last run ends at its width
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -631,6 +810,19 @@ void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const 
     if (n_tiles <= 0) return;
     const size_t smem = size_t(max_tile_ints + 8) * sizeof(int32_t);
     k_coverage<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, c0, c1, out);
+}
+
+void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints, RunTiles rt,
+                          int64_t R, int64_t* run_off, cudaStream_t s) {
+    if (n_tiles > 0) k_runs_count<<<unsigned(n_tiles), kThreads, size_t(max_tile_ints) * sizeof(int32_t), s>>>(tiles, c0, c1, rt);
+    k_runs_scan<<<1, kScanThreads, 0, s>>>(rt, n_tiles, R, run_off);
+}
+
+void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
+                                RunTiles rt, const int64_t* run_off, int32_t* lengths, int32_t* values, cudaStream_t s) {
+    if (n_tiles <= 0) return;
+    const size_t smem = size_t(max_tile_ints + 4) * sizeof(int32_t);
+    k_runs_write<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, run_off, lengths, values);
 }
 
 void launch_pack_u8(const int32_t* d_src, int64_t n, uint8_t* d_dst, uint2* ovf, uint32_t cap, uint32_t* d_cnt, cudaStream_t s) {

@@ -132,4 +132,24 @@ void launch_profile(TileTable tiles, int64_t n_tiles, const int32_t* c0, const i
 void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
                      int32_t* out, DeviceScalars* sc, cudaStream_t s);
 
+// K5r: bamCoverage as runs (DESIGN.md §10).  Per-tile arrays in tile order; region / rel come from the host, the rest is
+// written by the kernels.  rfirst / rlast ([R], zeroed before the launch): tile-order run index of a region's first run
+// and one past its last.
+struct RunTiles {
+    const int32_t* region;   // the caller's index of the tile's region
+    const int32_t* rel;      // the tile's first output element, relative to its region (region orientation)
+    int32_t* nnz;            // d[j] != 0 for j in [1, len)
+    int32_t* first;          // coverage at the tile's first element
+    int32_t* last;           // coverage at its last element
+    int64_t* toff;           // tile-order index of the tile's first run start
+    int64_t* rfirst;
+    int64_t* rlast;
+};
+// count pass + scans: run_off[0..R] (device) = every region's span of runs in the caller's region order
+void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints, RunTiles rt,
+                          int64_t R, int64_t* run_off, cudaStream_t s);
+// write pass: values[k] and lengths[k] for k in [0, run_off[R]); lengths must be zero before the launch
+void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
+                                RunTiles rt, const int64_t* run_off, int32_t* lengths, int32_t* values, cudaStream_t s);
+
 }  // namespace bsg

@@ -189,6 +189,38 @@ int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_
                                int32_t filteredF, int32_t tspan, int32_t* d_out, const int64_t* out_offsets, void* stream);
 void bsg_stage_close(bsg_stage* st);
 
+/* ---- bamCoverage as runs: run-length (length, value) pairs counted on the GPU ------------------------------------------
+ * Coverage is piecewise constant; these calls return it as runs instead of one int32 per base, without ever holding the
+ * dense result.  Region i's coverage, in region orientation (a '-' region's runs describe the reversed vector), is
+ * runs [run_offsets[i], run_offsets[i+1]): expanding them gives exactly what bsg_coverage writes for that region.
+ * Adjacent runs of a region have different values, every length is >= 1, a region's lengths sum to its width, a
+ * zero-width region has no runs, and runs never merge across regions (even regions that touch).
+ *   bsg_coverage_runs          the arguments of bsg_coverage up to maxgap; run_offsets is host memory of R + 1 int64
+ *                              (the total may pass 2^31).  *runs receives the result, which stays in device memory on
+ *                              the device the call ran on until bsg_runs_free.
+ *   bsg_coverage_runs_staged   the same on a staged session (its device).
+ *   bsg_runs_read              copies all run_offsets[R] lengths and values into the caller's arrays, any number of
+ *                              times.  Each destination is host memory, or 4-byte aligned device / managed memory on the
+ *                              result's device; device copies follow the contract of bsg_pileup_device: ordered after
+ *                              what `stream` (0 = the legacy default stream) has queued, complete on return.
+ *                              NULL destinations are accepted only for an empty result.
+ *   bsg_runs_free              releases a result (NULL is a no-op).  bsg_shutdown() frees every live result's device
+ *                              memory: bsg_runs_read on it is then BSG_EARG, bsg_runs_free on it stays valid.
+ * BSG_EARG before any work: runs == NULL, opts->n_devices > 1 (no multi-device variant), a bsg_runs_read destination
+ * that is misaligned or on another device.  Without a device: BSG_ECUDA.
+ * Timings (bsg_get_timings): out_elems is 2 x runs; bytes_d2h counts only what crosses PCIe - the control scalars and
+ * run_offsets - nothing of the runs themselves.  bsg_runs_read does not change the timings.
+ * The runs are counted when every batch has been decoded: opts->stream_min_ints does not apply. */
+typedef struct bsg_runs bsg_runs;      /* a finished run-length coverage result, held in device memory */
+int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                      const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                      const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
+                      int32_t maxgap, int64_t* run_offsets, bsg_runs** runs, const bsg_opts* opts);
+int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                             int32_t filteredF, int32_t tspan, int64_t* run_offsets, bsg_runs** runs);
+int bsg_runs_read(const bsg_runs* runs, int32_t* lengths, int32_t* values, void* stream);
+void bsg_runs_free(bsg_runs* runs);
+
 /*
  * writeSamAsBamAndIndex (src/bamsignals.cpp:496-534, .Call symbol bamsignals_writeSamAsBamAndIndex,
  * src/bamsignals_init.c:17): SAM text -> <bampath> (BGZF/BAM) + <bampath>.bai.  Host-only (no device needed).  The
@@ -215,7 +247,8 @@ int64_t bsg_debug_plan(const char* bampath, int64_t R, const char* const* seq_le
 const char* bsg_last_error(void);          /* valid until the next call on this thread */
 int  bsg_get_timings(bsg_timings* t);      /* of the last call on this thread */
 int  bsg_device_count(void);               /* CUDA devices visible (0 if none) */
-void bsg_shutdown(void);                   /* release cached device / pinned memory, worker threads, cached BAM handles
+void bsg_shutdown(void);                   /* release cached device / pinned memory, worker threads, cached BAM handles,
+                                              open staged sessions and run-length results
                                               (the mmap of up to four recently used BAM files + their parsed indexes are
                                               kept between calls while size and mtime are unchanged: do not truncate or
                                               rewrite a BAM in place while a call on it is running) */

@@ -17,7 +17,9 @@ through the bsg_*_device entry points; nothing of the result crosses PCIe.  torc
 
 Coverage as runs (beyond the R interface): `bamCoverage(..., runs=True)`, `coverage_runs_core` and
 `Stage.coverage_runs` return a CoverageRuns - run-length (length, value) pairs per region, counted on the GPU through
-bsg_coverage_runs, on the host or (device=) in torch tensors.
+bsg_coverage_runs, on the host or (device=) in torch tensors.  Profiles likewise: `bamProfile(..., runs=True)`,
+`profile_runs_core` and `Stage.profile_runs` return a ProfileRuns (bsg_profile_runs), runs over bins per region and
+strand row.
 """
 from __future__ import annotations
 
@@ -184,11 +186,25 @@ class CountSignals:
         return f"CountSignals object with {len(self)} {kind} signals"
 
 
-class CoverageRuns:
-    """bamCoverage as runs: region i's coverage (in region orientation) is lengths[offsets[i]:offsets[i+1]] bases of
-    values[offsets[i]:offsets[i+1]].  `lengths` / `values` are flat int32 numpy arrays or torch tensors on one device;
-    `offsets` is numpy int64 (R + 1).  Adjacent runs of a region differ in value, every length is >= 1, a zero-width
-    region has no runs.  The same thing as an RleList of GenomicAlignments::coverage, one Rle per region."""
+def _expand_runs(lengths, values, offsets):
+    """The dense vector that runs describe (every list's expansion, one after another, on the runs' device) and the
+    dense offset of every list (numpy int64, len(offsets))."""
+    if _is_tensor(lengths):
+        torch = sys.modules["torch"]
+        lengths = lengths.long()
+        flat = torch.repeat_interleave(values, lengths)
+        ends = torch.zeros(len(lengths) + 1, dtype=torch.int64, device=lengths.device)
+        torch.cumsum(lengths, 0, out=ends[1:])
+        return flat, ends[torch.from_numpy(offsets).to(lengths.device)].cpu().numpy()
+    flat = np.repeat(values, lengths)
+    ends = np.zeros(len(lengths) + 1, dtype=np.int64)
+    np.cumsum(lengths, out=ends[1:])
+    return flat, ends[offsets]
+
+
+class _RunLists:
+    """Flat int32 `lengths` / `values` (numpy arrays or torch tensors on one device) and numpy int64 `offsets`: list k
+    is lengths[offsets[k]:offsets[k+1]] elements of values[offsets[k]:offsets[k+1]]."""
 
     def __init__(self, lengths, values, offsets):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -198,35 +214,90 @@ class CoverageRuns:
             raise ValueError(f"lengths and values must have offsets[-1] = {int(offsets[-1])} elements")
         self.lengths, self.values, self.offsets = lengths, values, offsets
 
+    def _list(self, k):
+        a, b = int(self.offsets[k]), int(self.offsets[k + 1])
+        return self.lengths[a:b], self.values[a:b]
+
+    def _index(self, i):
+        if not isinstance(i, (int, np.integer)):
+            raise TypeError(f"{type(self).__name__} indices must be integers")
+        if i < 0 or i >= len(self):
+            raise IndexError("subscript out of bounds")
+        return int(i)
+
+
+class CoverageRuns(_RunLists):
+    """bamCoverage as runs: region i's coverage (in region orientation) is lengths[offsets[i]:offsets[i+1]] bases of
+    values[offsets[i]:offsets[i+1]].  `lengths` / `values` are flat int32 numpy arrays or torch tensors on one device;
+    `offsets` is numpy int64 (R + 1).  Adjacent runs of a region differ in value, every length is >= 1, a zero-width
+    region has no runs.  The same thing as an RleList of GenomicAlignments::coverage, one Rle per region."""
+
     def __len__(self):
         return len(self.offsets) - 1
 
     def __getitem__(self, i):
-        if not isinstance(i, (int, np.integer)):
-            raise TypeError("CoverageRuns indices must be integers")
-        if i < 0 or i >= len(self):
-            raise IndexError("subscript out of bounds")
-        a, b = int(self.offsets[i]), int(self.offsets[i + 1])
-        return self.lengths[a:b], self.values[a:b]
+        return self._list(self._index(i))
 
     def to_dense(self) -> CountSignals:
         """The bamCoverage result these runs describe (a CountSignals over one flat buffer on the runs' device)."""
-        if _is_tensor(self.lengths):
-            torch = sys.modules["torch"]
-            lengths = self.lengths.long()
-            flat = torch.repeat_interleave(self.values, lengths)
-            ends = torch.zeros(len(lengths) + 1, dtype=torch.int64, device=lengths.device)
-            torch.cumsum(lengths, 0, out=ends[1:])
-            dense_off = ends[torch.from_numpy(self.offsets).to(lengths.device)].cpu().numpy()
-        else:
-            flat = np.repeat(self.values, self.lengths)
-            ends = np.zeros(len(self.lengths) + 1, dtype=np.int64)
-            np.cumsum(self.lengths, out=ends[1:])
-            dense_off = ends[self.offsets]
+        flat, dense_off = _expand_runs(self.lengths, self.values, self.offsets)
         return CountSignals(None, False, flat=flat, offsets=dense_off)
 
     def __repr__(self):
         return f"CoverageRuns object with {len(self)} regions and {int(self.offsets[-1])} runs"
+
+
+class ProfileRuns(_RunLists):
+    """bamProfile as runs over bins (in region orientation, a partial last bin is one element).  Without `ss` list i is
+    region i's profile; with `ss` list 2i is region i's sense row and list 2i+1 its antisense row, so `offsets` has
+    (ss ? 2R : R) + 1 entries.  Adjacent runs of a list differ in value, every length is >= 1, a list's lengths sum to
+    its bin count, a zero-width region has no runs.  len() is R; [i] is (lengths, values), or with ss a
+    (sense, antisense) pair of them."""
+
+    def __init__(self, lengths, values, offsets, ss):
+        super().__init__(lengths, values, offsets)
+        self.ss = bool(ss)
+        if self.ss and (len(self.offsets) - 1) % 2:
+            raise ValueError("a strand-specific result has two lists per region: offsets must have 2R + 1 entries")
+
+    def __len__(self):
+        return (len(self.offsets) - 1) // (2 if self.ss else 1)
+
+    def __getitem__(self, i):
+        i = self._index(i)
+        return (self._list(2 * i), self._list(2 * i + 1)) if self.ss else self._list(i)
+
+    def to_dense(self) -> CountSignals:
+        """The bamProfile result these runs describe (a CountSignals over one flat buffer on the runs' device, with the
+        (2, w) [sense; antisense] views when ss)."""
+        if not self.ss:
+            flat, dense_off = _expand_runs(self.lengths, self.values, self.offsets)
+            return CountSignals(None, False, flat=flat, offsets=dense_off)
+        # Every region's dense slice [s_0, a_0, s_1, ...] starts at an even offset, so the even elements of the whole
+        # result are all sense rows one after another and the odd ones all antisense rows.
+        sizes = np.diff(self.offsets)
+        row_of_run = np.repeat(np.arange(len(sizes)) % 2, sizes)
+        rows = []
+        for a in (0, 1):
+            sel = row_of_run == a
+            if _is_tensor(self.lengths):
+                sel = sys.modules["torch"].from_numpy(sel).to(self.lengths.device)
+            off = np.zeros(len(self) + 1, dtype=np.int64)
+            np.cumsum(sizes[a::2], out=off[1:])
+            rows.append(_expand_runs(self.lengths[sel], self.values[sel], off))
+        (sense, bins), (anti, bins_anti) = rows
+        if not np.array_equal(bins, bins_anti):
+            raise ValueError("the sense and antisense rows of a region must have the same number of bins")
+        if _is_tensor(sense):
+            flat = sys.modules["torch"].stack((sense, anti), dim=1).reshape(-1)
+        else:
+            flat = np.empty(2 * len(sense), dtype=sense.dtype)
+            flat[0::2], flat[1::2] = sense, anti
+        return CountSignals(None, True, flat=flat, offsets=2 * bins)
+
+    def __repr__(self):
+        kind = "strand-specific" if self.ss else "strand-unspecific"
+        return f"ProfileRuns object with {len(self)} {kind} regions and {int(self.offsets[-1])} runs"
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -353,6 +424,10 @@ def lib():
     L.bsg_coverage_runs.restype = C.c_int
     L.bsg_coverage_runs_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 4 + [i64p, C.POINTER(C.c_void_p)]
     L.bsg_coverage_runs_staged.restype = C.c_int
+    L.bsg_profile_runs.argtypes = region_args + [i32p] + [C.c_int32] * 8 + [i64p, C.POINTER(C.c_void_p), C.POINTER(BsgOpts)]
+    L.bsg_profile_runs.restype = C.c_int
+    L.bsg_profile_runs_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 7 + [i64p, C.POINTER(C.c_void_p)]
+    L.bsg_profile_runs_staged.restype = C.c_int
     L.bsg_runs_read.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.bsg_runs_read.restype = C.c_int
     L.bsg_runs_free.argtypes = [C.c_void_p]
@@ -530,7 +605,8 @@ def coverage_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1
 
 
 def _take_runs(h, offsets, device):
-    """Copy a bsg_runs result into numpy arrays (device None) or torch tensors on `device`, then free it."""
+    """Copy a bsg_runs result into numpy arrays (device None) or torch tensors on `device`, then free it: (lengths,
+    values)."""
     try:
         n = int(offsets[-1])
         if device is None:
@@ -544,7 +620,7 @@ def _take_runs(h, offsets, device):
                                        torch.cuda.current_stream(device).cuda_stream))
     finally:
         lib().bsg_runs_free(h)
-    return CoverageRuns(lengths, values, offsets)
+    return lengths, values
 
 
 def coverage_runs_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, maxgap=16385,
@@ -563,7 +639,26 @@ def coverage_runs_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filtere
                                    None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
                                    int(filteredF), int(bool(tspan)), int(maxgap), _p(offsets, C.c_int64), C.byref(h),
                                    None if opts is None else C.byref(opts)))
-    return _take_runs(h, offsets, dev)
+    return CoverageRuns(*_take_runs(h, offsets, dev), offsets)
+
+
+def profile_runs_core(bampath, gr, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1,
+                      pe_mid=False, maxgap=16385, opts: Optional[BsgOpts] = None, device=None) -> ProfileRuns:
+    """pileup_core's arguments (binsize >= 1) -> the profile as runs (bsg_profile_runs).  device=None: numpy arrays on
+    the host; device= a CUDA device: torch tensors there (the call runs on that device; only the offsets cross PCIe)."""
+    m = marshal_regions(gr)
+    dev = None if device is None else _cuda_device(device)
+    if dev is not None and opts is None:
+        opts = default_opts(devices=[dev.index])
+    tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+    offsets = np.zeros((2 if ss else 1) * m.R + 1, dtype=np.int64)
+    h = C.c_void_p()
+    _check(lib().bsg_profile_runs(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                  _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                  None if tl is None else _p(tl, C.c_int32), int(mapqual), int(binsize), int(shift),
+                                  int(bool(ss)), int(requiredF), int(filteredF), int(bool(pe_mid)), int(maxgap),
+                                  _p(offsets, C.c_int64), C.byref(h), None if opts is None else C.byref(opts)))
+    return ProfileRuns(*_take_runs(h, offsets, dev), offsets, ss)
 
 
 class Stage:
@@ -620,7 +715,19 @@ class Stage:
         _check(lib().bsg_coverage_runs_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
                                               int(requiredF), int(filteredF), int(bool(tspan)), _p(offsets, C.c_int64),
                                               C.byref(h)))
-        return _take_runs(h, offsets, dev)
+        return CoverageRuns(*_take_runs(h, offsets, dev), offsets)
+
+    def profile_runs(self, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1, pe_mid=False,
+                     device=None) -> ProfileRuns:
+        """pileup() (binsize >= 1) as runs (bsg_profile_runs_staged); device= must be the session's device."""
+        dev = None if device is None else _cuda_device(device)
+        tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
+        offsets = np.zeros((2 if ss else 1) * self._m.R + 1, dtype=np.int64)
+        h = C.c_void_p()
+        _check(lib().bsg_profile_runs_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual), int(binsize),
+                                             int(shift), int(bool(ss)), int(requiredF), int(filteredF), int(bool(pe_mid)),
+                                             _p(offsets, C.c_int64), C.byref(h)))
+        return ProfileRuns(*_take_runs(h, offsets, dev), offsets, ss)
 
     def close(self):
         if self._h:
@@ -682,8 +789,10 @@ def _tlen(tf, pe):
     return (int(tf[0]), int(tf[1]))
 
 
+# runs=True: the profile as a ProfileRuns (run-length pairs per region and strand row) instead of a CountSignals; with
+# device= its arrays are torch tensors on that device.
 def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=("ignore", "filter", "midpoint"),
-               tlenFilter=None, filteredFlag=-1, verbose=False, opts=None, device=None):
+               tlenFilter=None, filteredFlag=-1, verbose=False, opts=None, device=None, runs=False):
     if binsize < 1:
         raise ValueError("provide a binsize greater or equal to 1")                  # R/wrappers.R:136-137
     if binsize > 1 and isinstance(gr, GRanges) and (gr.width % int(binsize) != 0).any():
@@ -691,6 +800,9 @@ def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=
                       "some bins will correspond to less than binsize basepairs")     # R/wrappers.R:138-141
     pe = _match_arg(paired_end, ("ignore", "filter", "midpoint"))
     bampath = os.path.expanduser(bampath)
+    if runs:
+        return profile_runs_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), _trunc(binsize), _trunc(shift), ss,
+                                 flagMask(pe), _trunc(filteredFlag), pe == "midpoint", opts=opts, device=device)
     out = None if device is None else _empty_on(device, gr, _trunc(binsize), ss)
     flat, off = pileup_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), _trunc(binsize), _trunc(shift), ss,
                             flagMask(pe), _trunc(filteredFlag), pe == "midpoint", opts=opts, _lazy=True, out=out)

@@ -31,7 +31,7 @@
 #include "plan.h"
 #include "pool.h"
 
-// A run-length coverage result (bsg_coverage_runs): lengths[n] and values[n] in device memory on `dev`.
+// A run-length result (bsg_coverage_runs, bsg_profile_runs): lengths[n] and values[n] in device memory on `dev`.
 struct bsg_runs {
     int dev = -1;
     int32_t* lengths = nullptr;
@@ -113,7 +113,7 @@ struct DeviceCtx {
     PinBuf h_raw[kSlots], h_offs[kSlots];
     cudaEvent_t ev_h2d[kSlots] = {}, ev_free[kSlots] = {};
     DevBuf tab[2], c0, c1, tiles_i32, tiles_i64, out, scalars;
-    DevBuf runs_i32, runs_i64;                  // run-length coverage: per-tile and per-region scratch (RunTiles, run_off)
+    DevBuf runs_i32, runs_i64;                  // run-length results: per-tile and per-list scratch (RunTiles, run_off)
     uint64_t tiles_gen = 0;                     // bumped whenever a Session uploads tiles: a staged Session's cached tiles are
                                                 // only valid while no other call has replaced them on this device
     // GPU inflate: an upload ring of kUp slots (compressed bytes, descriptors, walk scratch) and two raw / offsets buffers
@@ -821,7 +821,8 @@ public:
         runs_ = RunsOutput{};
     }
     void use_host_output() { dev_out_ = DeviceOutput{}; runs_ = RunsOutput{}; }
-    // The next call counts coverage as runs (count_runs) into `res`, and fills the caller's run_offsets[R + 1].
+    // The next call counts coverage or a profile as runs (count_runs) into `res`, and fills the caller's run_offsets
+    // (R + 1 entries, or 2R + 1 for a strand-specific profile).
     void use_runs_output(bsg_runs* res, int64_t* run_offsets) {
         dev_out_ = DeviceOutput{};
         runs_ = RunsOutput{res, run_offsets};
@@ -830,6 +831,13 @@ public:
     std::vector<int64_t> coverage_layout() const {
         std::vector<int64_t> off(size_t(rg_.R) + 1, 0);
         for (int64_t i = 0; i < rg_.R; ++i) off[i + 1] = off[i] + rg_.width[i];
+        return off;
+    }
+    // bsg_output_layout() of bamProfile (binsize >= 1) for this session's regions
+    std::vector<int64_t> profile_layout(int32_t binsize, int ss) const {
+        const int64_t mult = ss ? 2 : 1;
+        std::vector<int64_t> off(size_t(rg_.R) + 1, 0);
+        for (int64_t i = 0; i < rg_.R; ++i) off[i + 1] = off[i] + mult * ((int64_t(rg_.width[i]) + binsize - 1) / binsize);
         return off;
     }
     int device() const { return ctx_->dev; }
@@ -888,47 +896,67 @@ private:
         cnt_.t_done = t1;
     }
 
-    // Coverage as runs (DESIGN.md §10) over ALL tiles (t0 == 0, advance() never counts early): count pass + scans, the
-    // region spans come back (the only D2H besides the control scalars), the result is allocated at its exact size, then
-    // the write pass.  Device memory: 28 bytes per tile, 16 per region, 8 per run.
+    // Coverage (DESIGN.md §10) or a profile (§11) as runs over ALL tiles (t0 == 0, advance() never counts early): count
+    // pass + scans, the list spans come back (the only D2H besides the control scalars), the result is allocated at its
+    // exact size, then the write pass.  A list is a region, or with a strand-specific profile one strand row of a region
+    // (list mult * i + a); every tile holds one virtual tile per row: row a of the j-th of region i's n_i tiles, T_i
+    // its first, is v = mult * T_i + a * n_i + j, so that a list's pieces are consecutive (identity when mult is 1).
+    // Device memory: 28 bytes per virtual tile (+4 with ss), 24 per list, 8 per run.
     void count_runs(const TileTable& tt, int64_t nt, cudaStream_t st) {
         DeviceCtx& c = *ctx_;
         if (nt != n_tiles_) fail(BSG_EARG, "internal error: runs are counted over all tiles at once");
-        const int64_t R = rg_.R;
-        runs_tiles_.resize(size_t(nt) * 2);
-        for (int64_t t = 0; t < nt; ++t) {
-            const int64_t i = ht_.region[t];
-            runs_tiles_[t] = int32_t(i);
-            runs_tiles_[nt + t] = int32_t(ht_.out_off[t] - tiles_offsets_[i]);
+        const bool profile = cnt_.mode == MODE_PROFILE;
+        const int64_t mult = profile && cnt_.ss ? 2 : 1;
+        const int64_t R = rg_.R, L = mult * R, nv = mult * nt;
+        const int64_t up = mult == 2 ? 3 : 2;                  // uploaded per virtual tile: list, rel (and vt with ss)
+        runs_tiles_.resize(size_t(nv * up));
+        for (int64_t t0 = 0; t0 < nt;) {
+            const int64_t i = ht_.region[t0];
+            int64_t t1 = t0 + 1;
+            while (t1 < nt && ht_.region[t1] == i) ++t1;
+            for (int64_t t = t0; t < t1; ++t)
+                for (int64_t a = 0; a < mult; ++a) {
+                    const int64_t v = mult * t0 + a * (t1 - t0) + (t - t0);
+                    runs_tiles_[v] = int32_t(mult * i + a);
+                    runs_tiles_[nv + v] = int32_t((ht_.out_off[t] - tiles_offsets_[i]) / mult);
+                    if (mult == 2) runs_tiles_[2 * nv + a * nt + t] = int32_t(v);
+                }
+            t0 = t1;
         }
-        c.runs_i32.ensure(size_t(nt) * 5 * sizeof(int32_t) + 64);
-        c.runs_i64.ensure((size_t(nt) + 3 * size_t(R) + 1) * sizeof(int64_t) + 64);
-        c.h_runs.ensure((size_t(R) + 1) * sizeof(int64_t));
+        c.runs_i32.ensure(size_t(nv) * (up + 3) * sizeof(int32_t) + 64);
+        c.runs_i64.ensure((size_t(nv) + 3 * size_t(L) + 1) * sizeof(int64_t) + 64);
+        c.h_runs.ensure((size_t(L) + 1) * sizeof(int64_t));
         int32_t* ri = c.runs_i32.as<int32_t>();
         int64_t* rl = c.runs_i64.as<int64_t>();
-        const RunTiles rt{ri, ri + nt, ri + 2 * nt, ri + 3 * nt, ri + 4 * nt, rl, rl + nt, rl + nt + R};
-        int64_t* run_off = rl + nt + 2 * R;
+        int32_t* rw = ri + up * nv;
+        const RunTiles rt{ri, ri + nv, rw, rw + nv, rw + 2 * nv, rl, rl + nv, rl + nv + L};
+        const int32_t* vt = mult == 2 ? ri + 2 * nv : nullptr;
+        int64_t* run_off = rl + nv + 2 * L;
+        int32_t* c0 = c.c0.as<int32_t>();
+        int32_t* c1 = c.c1.as<int32_t>();
         Span sp{c.timing_event(), c.timing_event()};
         BSG_CUDA(cudaEventRecord(sp.a, st));
-        if (nt) BSG_CUDA(cudaMemcpyAsync(ri, runs_tiles_.data(), size_t(nt) * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        if (R) BSG_CUDA(cudaMemsetAsync(rt.rfirst, 0, size_t(R) * 2 * sizeof(int64_t), st));
-        launch_coverage_runs(tt, nt, c.c0.as<int32_t>(), c.c1.as<int32_t>(), max_tile_ints_, rt, R, run_off, st);
-        BSG_CUDA(cudaMemcpyAsync(c.h_runs.p, run_off, (size_t(R) + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        if (nv) BSG_CUDA(cudaMemcpyAsync(ri, runs_tiles_.data(), size_t(nv * up) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        if (L) BSG_CUDA(cudaMemsetAsync(rt.rfirst, 0, size_t(L) * 2 * sizeof(int64_t), st));
+        if (profile) launch_profile_runs(tt, nt, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, rt, vt, L, run_off, st);
+        else launch_coverage_runs(tt, nt, c0, c1, max_tile_ints_, rt, R, run_off, st);
+        BSG_CUDA(cudaMemcpyAsync(c.h_runs.p, run_off, (size_t(L) + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         BSG_CUDA(cudaStreamSynchronize(st));
         BSG_CUDA(cudaGetLastError());
-        memcpy(runs_.run_offsets, c.h_runs.p, (size_t(R) + 1) * sizeof(int64_t));
+        memcpy(runs_.run_offsets, c.h_runs.p, (size_t(L) + 1) * sizeof(int64_t));
         bsg_runs& res = *runs_.res;
         res.dev = c.dev;
-        res.n = runs_.run_offsets[R];
+        res.n = runs_.run_offsets[L];
         const size_t bytes = size_t(std::max<int64_t>(res.n, 1)) * sizeof(int32_t);
         BSG_CUDA(cudaMalloc(&res.lengths, bytes));
         BSG_CUDA(cudaMalloc(&res.values, bytes));
         BSG_CUDA(cudaMemsetAsync(res.lengths, 0, bytes, st));
-        launch_coverage_runs_write(tt, nt, c.c0.as<int32_t>(), c.c1.as<int32_t>(), max_tile_ints_, rt, run_off, res.lengths, res.values, st);
+        if (profile) launch_profile_runs_write(tt, nt, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, rt, vt, run_off, res.lengths, res.values, st);
+        else launch_coverage_runs_write(tt, nt, c0, c1, max_tile_ints_, rt, run_off, res.lengths, res.values, st);
         BSG_CUDA(cudaEventRecord(sp.b, st));
         kt_.count.push_back(sp); kt_.launches += nt ? 3 : 1;
         tm_.out_elems = 2 * res.n;
-        os_bytes_ += double((R + 1) * int64_t(sizeof(int64_t)));
+        os_bytes_ += double((L + 1) * int64_t(sizeof(int64_t)));
     }
 
     // ---- output streamer: D2H on its own stream into a pinned ring, a host thread scatters tiles to the caller ------------
@@ -1690,7 +1718,7 @@ private:
     bool tiles_valid_ = false, tiles_caller_ = false;
     DeviceOutput dev_out_;
     RunsOutput runs_;
-    std::vector<int32_t> runs_tiles_;           // region, rel of every tile (uploaded by count_runs)
+    std::vector<int32_t> runs_tiles_;           // list, rel (and vt) of every virtual tile (uploaded by count_runs)
     Mode tiles_mode_ = MODE_COUNT;
     int32_t tiles_binsize_ = 0;
     int tiles_ss_ = 0;
@@ -2204,6 +2232,68 @@ int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t 
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
         st->s->decode_resident(MODE_COVERAGE, fp);
         st->s->count(MODE_COVERAGE, fp, 1, 0, nullptr, dense.data(), nullptr, false);
+        st->s->finish_timings(t0);
+        st->s->use_host_output();
+        res->live = true;
+        g_runs.push_back(res.get());
+        *runs = res.release();
+    });
+}
+
+int bsg_profile_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                     const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                     int32_t mapqual, int32_t binsize, int32_t shift, int32_t ss, int32_t requiredF, int32_t filteredF,
+                     int32_t pe_mid, int32_t /*maxgap*/, int64_t* run_offsets, bsg_runs** runs, const bsg_opts* opts) {
+    if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
+    *runs = nullptr;
+    return guarded([&] {
+        const double t0 = now_ms();
+        const bsg_opts o = effective_opts(opts);
+        validate_devices(o);
+        if (o.n_devices > 1) fail(BSG_EARG, "run-length profiles run on one device: n_devices must be 0 or 1");
+        if (!run_offsets) fail(BSG_EARG, "run_offsets is required");
+        if (binsize < 1) fail(BSG_EARG, "run-length profiles need binsize >= 1 (bamCount has no runs form)");
+        const int64_t ext = ext_pileup(tlen_filter, shift, pe_mid);
+        KeepCurrentDevice keep;
+        Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts);
+        const std::vector<int64_t> dense = s.profile_layout(binsize, ss != 0);
+        s.start_plan(ext);
+        auto res = std::make_unique<bsg_runs>();
+        s.use_runs_output(res.get(), run_offsets);
+        const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
+        s.defer_setup([&] { s.begin_count(MODE_PROFILE, fp, binsize, ss != 0, ext, nullptr, dense.data(), nullptr, false, s.setup_stream()); });
+        s.stage(ext, false);
+        s.finish_count();
+        s.finish_timings(t0);
+        s.kick_page_locking();
+        res->live = true;
+        g_runs.push_back(res.get());
+        *runs = res.release();
+    });
+}
+
+int bsg_profile_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift,
+                            int32_t ss, int32_t requiredF, int32_t filteredF, int32_t pe_mid, int64_t* run_offsets,
+                            bsg_runs** runs) {
+    if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
+    *runs = nullptr;
+    if (!st) { g_err = "null stage"; return BSG_EARG; }
+    return guarded([&] {
+        if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
+        if (!run_offsets) fail(BSG_EARG, "run_offsets is required");
+        if (binsize < 1) fail(BSG_EARG, "run-length profiles need binsize >= 1 (bamCount has no runs form)");
+        const double t0 = now_ms();
+        KeepCurrentDevice keep;
+        BSG_CUDA(cudaSetDevice(st->s->device()));
+        st->s->reset_counters();
+        st->s->require_ext(ext_pileup(tlen_filter, shift, pe_mid));
+        auto res = std::make_unique<bsg_runs>();
+        st->s->use_runs_output(res.get(), run_offsets);
+        const std::vector<int64_t> dense = st->s->profile_layout(binsize, ss != 0);
+        st->s->prepare_tiles(MODE_PROFILE, binsize, ss != 0, dense.data());
+        const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
+        st->s->decode_resident(MODE_PROFILE, fp);
+        st->s->count(MODE_PROFILE, fp, binsize, ss != 0, nullptr, dense.data(), nullptr, false);
         st->s->finish_timings(t0);
         st->s->use_host_output();
         res->live = true;

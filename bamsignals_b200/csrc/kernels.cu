@@ -4,6 +4,7 @@
 #include "kernels.cuh"
 
 #include <climits>
+#include <type_traits>
 
 namespace bsg {
 namespace {
@@ -353,7 +354,24 @@ __device__ __forceinline__ uint32_t fast_div(uint32_t n, uint64_t magic, uint32_
 // K4 bamProfile: one CTA per tile (<= kTileInts output ints), shared-memory histogram.
 // k_profile: one read per lane and one shared atomic per counted read (binsize 1..3: neighbouring reads fall into
 // different bins anyway).
+// The histograms are built by __device__ helpers shared with the run-length kernels (K4r), so that both count every
+// tile through the same code: hist[0, nout) zeroed before, the caller's barrier after.
 // ---------------------------------------------------------------------------------------------------------------
+template <bool SS, bool BIN1>
+__device__ __forceinline__ void scatter_profile(int32_t* hist, int32_t loc, int32_t len, int flip, int64_t lo, int64_t hi,
+                                                const int32_t* __restrict__ c0, const int32_t* __restrict__ c1,
+                                                uint64_t magic, uint32_t mshift) {
+    for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
+        const int32_t p5 = __ldg(c0 + i), ng = __ldg(c1 + i);
+        int32_t rel = p5 - loc;
+        if (ng < 0 || uint32_t(rel) >= uint32_t(len)) continue;                    // src/bamsignals.cpp:351-353
+        const int a = (ng ^ flip) & 1;
+        if (flip) rel = len - 1 - rel;                                             // :356-359
+        const int32_t bin = BIN1 ? rel : int32_t(fast_div(uint32_t(rel), magic, mshift));
+        atomicAdd(&hist[SS ? 2 * bin + a : bin], 1);                               // :361-362
+    }
+}
+
 template <bool SS, bool BIN1>
 __global__ void __launch_bounds__(kThreads) k_profile(TileTable tiles, const int32_t* __restrict__ c0,
                                                       const int32_t* __restrict__ c1, int32_t binsize, uint64_t magic,
@@ -369,15 +387,7 @@ __global__ void __launch_bounds__(kThreads) k_profile(TileTable tiles, const int
     int32_t* hist = smem + out_phase(out + off);           // same 16-byte phase as the destination
     for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
     __syncthreads();
-    for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
-        const int32_t p5 = __ldg(c0 + i), ng = __ldg(c1 + i);
-        int32_t rel = p5 - loc;
-        if (ng < 0 || uint32_t(rel) >= uint32_t(len)) continue;                    // src/bamsignals.cpp:351-353
-        const int a = (ng ^ flip) & 1;
-        if (flip) rel = len - 1 - rel;                                             // :356-359
-        const int32_t bin = BIN1 ? rel : int32_t(fast_div(uint32_t(rel), magic, mshift));
-        atomicAdd(&hist[SS ? 2 * bin + a : bin], 1);                               // :361-362
-    }
+    scatter_profile<SS, BIN1>(hist, loc, len, flip, lo, hi, c0, c1, magic, mshift);
     __syncthreads();
     copy_out(out + off, hist, nout);
 }
@@ -390,20 +400,9 @@ __global__ void __launch_bounds__(kThreads) k_profile(TileTable tiles, const int
 // Division by binsize: exact for 0 <= n < 2^31 with a 32-bit multiplier m = ceil(2^(31+L) / d), L = ceil(log2 d):
 // n / d = umulhi(n, m) >> (L - 1).
 template <bool SS>
-__global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const int32_t* __restrict__ c0,
-                                                          const int32_t* __restrict__ c1, int32_t binsize, uint32_t magic,
-                                                          uint32_t mshift, int32_t* __restrict__ out) {
-    extern __shared__ __align__(16) int32_t smem[];
-    const int64_t tix = blockIdx.x;
-    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
-    const bool flip = tiles.strand[tix] < 0;
-    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
-    const int64_t off = tiles.out_off[tix];
-    const int nbins = int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize));
-    const int nout = SS ? 2 * nbins : nbins;
-    int32_t* hist = smem + out_phase(out + off);
-    for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
-    __syncthreads();
+__device__ __forceinline__ void scatter_profile_agg(int32_t* hist, int32_t loc, int32_t len, bool flip, int64_t lo, int64_t hi,
+                                                    const int32_t* __restrict__ c0, const int32_t* __restrict__ c1,
+                                                    uint32_t magic, uint32_t mshift) {
     const int lane = threadIdx.x & 31;
     const int4* c0q = reinterpret_cast<const int4*>(c0);
     const int4* c1q = reinterpret_cast<const int4*>(c1);
@@ -449,6 +448,24 @@ __global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const
         }
         if (key != INT_MAX) atomicAdd(&hist[key], cnt);
     }
+}
+
+template <bool SS>
+__global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const int32_t* __restrict__ c0,
+                                                          const int32_t* __restrict__ c1, int32_t binsize, uint32_t magic,
+                                                          uint32_t mshift, int32_t* __restrict__ out) {
+    extern __shared__ __align__(16) int32_t smem[];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const bool flip = tiles.strand[tix] < 0;
+    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
+    const int64_t off = tiles.out_off[tix];
+    const int nbins = int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize));
+    const int nout = SS ? 2 * nbins : nbins;
+    int32_t* hist = smem + out_phase(out + off);
+    for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
+    __syncthreads();
+    scatter_profile_agg<SS>(hist, loc, len, flip, lo, hi, c0, c1, magic, mshift);
     __syncthreads();
     copy_out(out + off, hist, nout);
 }
@@ -715,6 +732,128 @@ __global__ void __launch_bounds__(kThreads) k_runs_write(TileTable tiles, int64_
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// K4r bamProfile as runs (DESIGN.md §11).  A profile has no running sum: inside a tile, strand row a's histogram
+// h[j] = hist[mult * j + a] changes exactly where h[j] != h[j-1].  Row a of the j-th of region i's n_i tiles (T_i its
+// first) is the virtual tile v = mult * T_i + a * n_i + j, in list mult * i + a; vt[a * n_tiles + t] holds v for tile t.
+// A list's pieces are consecutive virtual tiles, so k_runs_scan runs unchanged over the virtual tiles.
+//   k_profile_runs_count  per tile and row: nnz = #{j in [1, nbins): h[j] != h[j-1]}, first = h[0], last = h[nbins-1]
+//   k_profile_runs_write  the histogram again; every run start writes h[j] at its index, and the lengths are added up
+//                         with atomics as in k_runs_write
+// KIND: 0 = k_profile<SS, true>'s histogram (binsize 1), 1 = k_profile<SS, false>'s, 2 = k_profile_agg<SS>'s
+// (binsize >= 4): the same helpers give the same histogram as the dense call.  The histogram sits at smem[0].
+// ---------------------------------------------------------------------------------------------------------------
+template <bool SS, int KIND>
+__device__ __forceinline__ int profile_runs_hist(int32_t* hist, const TileTable& tiles, int64_t tix, const int32_t* __restrict__ c0,
+                                                 const int32_t* __restrict__ c1, int32_t binsize, uint64_t magic, uint32_t mshift) {
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const bool flip = tiles.strand[tix] < 0;
+    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
+    const int nbins = KIND == 0 ? len : int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize));
+    const int nout = SS ? 2 * nbins : nbins;
+    for (int k = threadIdx.x; k < nout; k += kThreads) hist[k] = 0;
+    __syncthreads();
+    if constexpr (KIND == 2) scatter_profile_agg<SS>(hist, loc, len, flip, lo, hi, c0, c1, uint32_t(magic), mshift);
+    else scatter_profile<SS, KIND == 0>(hist, loc, len, flip ? 1 : 0, lo, hi, c0, c1, magic, mshift);
+    __syncthreads();
+    return nbins;
+}
+
+template <bool SS, int KIND>
+__global__ void __launch_bounds__(kThreads) k_profile_runs_count(TileTable tiles, int64_t n_tiles, const int32_t* __restrict__ c0,
+                                                                 const int32_t* __restrict__ c1, int32_t binsize, uint64_t magic,
+                                                                 uint32_t mshift, RunTiles rt, const int32_t* __restrict__ vt) {
+    constexpr int M = SS ? 2 : 1;
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_nz[M][kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int nbins = profile_runs_hist<SS, KIND>(smem, tiles, tix, c0, c1, binsize, magic, mshift);
+    // element k = M j + a compares with k - M; kThreads is even, so a thread only ever sees one row (a = k & 1)
+    int nz = 0;
+    for (int k = threadIdx.x + M; k < M * nbins; k += kThreads) nz += int(smem[k] != smem[k - M]);
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+    for (int a = 0; a < M; ++a) {
+        const int n = __reduce_add_sync(FULL, (threadIdx.x & (M - 1)) == a ? nz : 0);
+        if (lane == 0) s_nz[a][wid] = n;
+    }
+    __syncthreads();
+    if (threadIdx.x < M) {
+        const int a = threadIdx.x;
+        int tn = 0;
+        for (int k = 0; k < kThreads / 32; ++k) tn += s_nz[a][k];
+        const int32_t v = vt ? vt[a * n_tiles + tix] : int32_t(tix);
+        rt.nnz[v] = tn;
+        rt.first[v] = smem[a];
+        rt.last[v] = smem[M * (nbins - 1) + a];
+    }
+}
+
+template <bool SS, int KIND>
+__global__ void __launch_bounds__(kThreads) k_profile_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* __restrict__ c0,
+                                                                 const int32_t* __restrict__ c1, int32_t binsize, uint64_t magic,
+                                                                 uint32_t mshift, RunTiles rt, const int32_t* __restrict__ vt,
+                                                                 const int64_t* __restrict__ run_off, int32_t* __restrict__ lengths,
+                                                                 int32_t* __restrict__ values) {
+    constexpr int M = SS ? 2 : 1;
+    constexpr int kWarps = kThreads / 32;
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_cnt[M][kWarps];
+    const int64_t tix = blockIdx.x;
+    const int nbins = profile_runs_hist<SS, KIND>(smem, tiles, tix, c0, c1, binsize, magic, mshift);
+    const int64_t n_virtual = M * n_tiles;
+    // every warp owns a contiguous part of the tile's bins (as in k_runs_write): pass 1 counts its run starts per row,
+    // pass 2 adds what the warps in front of it have and writes the runs
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int bpw = ((nbins + kWarps - 1) / kWarps + 31) & ~31;
+    const int j_lo = wid * bpw, j_hi = min(nbins, j_lo + bpw);
+    bool start0[M];
+    int cnt[M];
+#pragma unroll
+    for (int a = 0; a < M; ++a) {
+        const int64_t v = vt ? vt[a * n_tiles + tix] : tix;
+        const int32_t list = rt.region[v];
+        start0[a] = v == 0 || rt.region[v - 1] != list || rt.first[v] != rt.last[v - 1];     // a run starts at bin 0
+        cnt[a] = 0;
+    }
+    auto flag = [&](int j, int a) {
+        return j < j_hi && (j == 0 ? start0[a] : smem[M * j + a] != smem[M * (j - 1) + a]);
+    };
+    for (int j0 = j_lo; j0 < j_hi; j0 += 32) {                                      // warp-uniform
+#pragma unroll
+        for (int a = 0; a < M; ++a) cnt[a] += __popc(__ballot_sync(FULL, flag(j0 + lane, a)));
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int a = 0; a < M; ++a) s_cnt[a][wid] = cnt[a];
+    }
+    __syncthreads();
+    const unsigned below = (1u << lane) - 1u;
+#pragma unroll
+    for (int a = 0; a < M; ++a) {
+        const int64_t v = vt ? vt[a * n_tiles + tix] : tix;
+        const int32_t list = rt.region[v], rel = rt.rel[v];
+        const int64_t kbeg = run_off[list], kend = run_off[list + 1];
+        int64_t k0 = kbeg + (rt.toff[v] - rt.rfirst[list]);                      // index of the tile's first run start
+        for (int w = 0; w < wid; ++w) k0 += s_cnt[a][w];
+        for (int j0 = j_lo; j0 < j_hi; j0 += 32) {
+            const int j = j0 + lane;
+            const bool f = flag(j, a);
+            const unsigned b = __ballot_sync(FULL, f);
+            if (f) {
+                const int64_t k = k0 + __popc(b & below);
+                const int32_t p = rel + j;                                         // run start, relative to the list
+                values[k] = smem[M * j + a];
+                atomicAdd(&lengths[k], -p);
+                if (k > kbeg) atomicAdd(&lengths[k - 1], p);
+            }
+            k0 += __popc(b);
+        }
+        const bool tail = v + 1 == n_virtual || rt.region[v + 1] != list;
+        if (tail && threadIdx.x == 0 && kend > kbeg) atomicAdd(&lengths[kend - 1], rel + nbins);    // the list's last run ends at its bin count
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // Result narrowing (see kernels.cuh): four elements per thread, one 32-bit store; src is only 4-byte aligned.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_pack_u8(const int32_t* __restrict__ src, int64_t n, uint8_t* __restrict__ dst, uint2* ovf,
@@ -751,6 +890,32 @@ void magic_for(int32_t d, uint64_t* magic, uint32_t* shift) {
     *shift = 32 + L;
     const unsigned __int128 num = (unsigned __int128)1 << (32 + L);
     *magic = uint64_t((num + uint64_t(d) - 1) / uint64_t(d));
+}
+// k_profile_agg's 32-bit multiplier and shift (see there)
+void agg_magic_for(int32_t d, uint32_t* magic, uint32_t* shift) {
+    uint32_t L = 0;
+    while ((1ull << L) < uint64_t(d)) ++L;
+    *magic = uint32_t(((1ull << (31 + L)) + uint64_t(d) - 1) / uint64_t(d));
+    *shift = L - 1;
+}
+
+// The runs kernels' instantiation for (ss, binsize), with the divisor of the dense kernel that binsize selects:
+// f(std::bool_constant<SS>, std::integral_constant<int, KIND>, magic, mshift).
+template <class F>
+void with_profile_kind(int ss, int32_t binsize, F&& f) {
+    using K0 = std::integral_constant<int, 0>;
+    using K1 = std::integral_constant<int, 1>;
+    using K2 = std::integral_constant<int, 2>;
+    if (binsize >= 4) {
+        uint32_t magic, mshift;
+        agg_magic_for(binsize, &magic, &mshift);
+        if (ss) f(std::true_type{}, K2{}, uint64_t(magic), mshift); else f(std::false_type{}, K2{}, uint64_t(magic), mshift);
+        return;
+    }
+    uint64_t magic; uint32_t mshift;
+    magic_for(binsize, &magic, &mshift);
+    if (binsize == 1) { if (ss) f(std::true_type{}, K0{}, magic, mshift); else f(std::false_type{}, K0{}, magic, mshift); }
+    else              { if (ss) f(std::true_type{}, K1{}, magic, mshift); else f(std::false_type{}, K1{}, magic, mshift); }
 }
 
 }  // namespace
@@ -790,11 +955,10 @@ void launch_profile(TileTable tiles, int64_t n_tiles, const int32_t* c0, const i
     const size_t smem = size_t(max_tile_ints + 4) * sizeof(int32_t);
     const unsigned grid = unsigned(n_tiles);
     if (binsize >= 4) {
-        uint32_t L = 0;
-        while ((1ull << L) < uint64_t(binsize)) ++L;
-        const uint32_t magic = uint32_t(((1ull << (31 + L)) + uint64_t(binsize) - 1) / uint64_t(binsize));
-        if (ss) k_profile_agg<true><<<grid, kThreads, smem, s>>>(tiles, c0, c1, binsize, magic, L - 1, out);
-        else k_profile_agg<false><<<grid, kThreads, smem, s>>>(tiles, c0, c1, binsize, magic, L - 1, out);
+        uint32_t magic, mshift;
+        agg_magic_for(binsize, &magic, &mshift);
+        if (ss) k_profile_agg<true><<<grid, kThreads, smem, s>>>(tiles, c0, c1, binsize, magic, mshift, out);
+        else k_profile_agg<false><<<grid, kThreads, smem, s>>>(tiles, c0, c1, binsize, magic, mshift, out);
         return;
     }
     uint64_t magic; uint32_t mshift;
@@ -823,6 +987,26 @@ void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t*
     if (n_tiles <= 0) return;
     const size_t smem = size_t(max_tile_ints + 4) * sizeof(int32_t);
     k_runs_write<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, run_off, lengths, values);
+}
+
+void launch_profile_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,
+                         int max_tile_ints, RunTiles rt, const int32_t* vt, int64_t lists, int64_t* run_off, cudaStream_t s) {
+    if (n_tiles > 0)
+        with_profile_kind(ss, binsize, [&](auto SS, auto KIND, uint64_t magic, uint32_t mshift) {
+            k_profile_runs_count<SS(), KIND()><<<unsigned(n_tiles), kThreads, size_t(max_tile_ints) * sizeof(int32_t), s>>>(
+                tiles, n_tiles, c0, c1, binsize, magic, mshift, rt, vt);
+        });
+    k_runs_scan<<<1, kScanThreads, 0, s>>>(rt, (ss ? 2 : 1) * n_tiles, lists, run_off);
+}
+
+void launch_profile_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,
+                               int max_tile_ints, RunTiles rt, const int32_t* vt, const int64_t* run_off, int32_t* lengths,
+                               int32_t* values, cudaStream_t s) {
+    if (n_tiles <= 0) return;
+    with_profile_kind(ss, binsize, [&](auto SS, auto KIND, uint64_t magic, uint32_t mshift) {
+        k_profile_runs_write<SS(), KIND()><<<unsigned(n_tiles), kThreads, size_t(max_tile_ints) * sizeof(int32_t), s>>>(
+            tiles, n_tiles, c0, c1, binsize, magic, mshift, rt, vt, run_off, lengths, values);
+    });
 }
 
 void launch_pack_u8(const int32_t* d_src, int64_t n, uint8_t* d_dst, uint2* ovf, uint32_t cap, uint32_t* d_cnt, cudaStream_t s) {

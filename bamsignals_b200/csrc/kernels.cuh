@@ -152,4 +152,17 @@ void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, c
 void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
                                 RunTiles rt, const int64_t* run_off, int32_t* lengths, int32_t* values, cudaStream_t s);
 
+// K4r: bamProfile as runs (DESIGN.md §11), over VIRTUAL tiles: row a (sense / antisense with ss) of the j-th of region
+// i's n_i tiles, T_i its first tile, is virtual tile v = mult * T_i + a * n_i + j in list mult * i + a (mult = ss ? 2 : 1).
+// rt is indexed by virtual tile and list (region = the list, rel = the tile's first bin relative to the region);
+// vt[a * n_tiles + t] = v of row a of tile t, or NULL for the identity (no ss).  The same histogram as launch_profile
+// with the same binsize; rfirst / rlast ([lists], zeroed before the launch) as for coverage.
+// count pass + scans: run_off[0..lists] (device) = every list's span of runs, lists in the caller's region order
+void launch_profile_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,
+                         int max_tile_ints, RunTiles rt, const int32_t* vt, int64_t lists, int64_t* run_off, cudaStream_t s);
+// write pass: values[k] and lengths[k] for k in [0, run_off[lists]); lengths must be zero before the launch
+void launch_profile_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,
+                               int max_tile_ints, RunTiles rt, const int32_t* vt, const int64_t* run_off, int32_t* lengths,
+                               int32_t* values, cudaStream_t s);
+
 }  // namespace bsg

@@ -211,7 +211,7 @@ void bsg_stage_close(bsg_stage* st);
  * Timings (bsg_get_timings): out_elems is 2 x runs; bytes_d2h counts only what crosses PCIe - the control scalars and
  * run_offsets - nothing of the runs themselves.  bsg_runs_read does not change the timings.
  * The runs are counted when every batch has been decoded: opts->stream_min_ints does not apply. */
-typedef struct bsg_runs bsg_runs;      /* a finished run-length coverage result, held in device memory */
+typedef struct bsg_runs bsg_runs;      /* a finished run-length result (coverage or profile), held in device memory */
 int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
                       const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
                       const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
@@ -220,6 +220,33 @@ int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t 
                              int32_t filteredF, int32_t tspan, int64_t* run_offsets, bsg_runs** runs);
 int bsg_runs_read(const bsg_runs* runs, int32_t* lengths, int32_t* values, void* stream);
 void bsg_runs_free(bsg_runs* runs);
+
+/* ---- bamProfile as runs: run-length (length, value) pairs of read-end profiles counted on the GPU -----------------------
+ * The same result as bsg_pileup with binsize >= 1, as runs over output elements (bins) instead of one int32 per bin,
+ * without ever holding the dense result.  A result has L = (ss ? 2 : 1) x R lists, in the caller's region order:
+ *   without ss, list i is region i's profile;
+ *   with ss, list 2i is region i's sense row and list 2i+1 its antisense row.
+ * List k is runs [run_offsets[k], run_offsets[k+1]), in region orientation, exactly as bsg_pileup lays the bins out (a
+ * partial last bin is one element): expanding list i, or interleaving the expansions of lists 2i and 2i+1, gives
+ * exactly region i's slice of bsg_pileup's result with the same arguments.  Every length is >= 1, a list's lengths sum
+ * to its bin count, adjacent runs of a list have different values, a zero-width region has no runs, and runs never merge
+ * across lists.  bamCount (binsize <= 0) has no runs form.
+ *   bsg_profile_runs           the arguments of bsg_pileup up to maxgap; run_offsets is host memory of L + 1 int64.
+ *                              *runs receives the result, which stays in device memory on the device the call ran on.
+ *   bsg_profile_runs_staged    the same on a staged session (its device).
+ * bsg_runs_read, bsg_runs_free and the bsg_shutdown() rules of coverage runs apply unchanged.
+ * BSG_EARG before any work: runs or run_offsets NULL, binsize < 1, opts->n_devices > 1, pe_mid without tlen_filter, a
+ * staged call that needs more halo than the session was staged with.  Without a device: BSG_ECUDA.
+ * Timings, and opts->stream_min_ints: as for coverage runs (out_elems is 2 x runs; bytes_d2h counts only the control
+ * scalars and run_offsets). */
+int bsg_profile_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                     const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                     const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift, int32_t ss,
+                     int32_t requiredF, int32_t filteredF, int32_t pe_mid, int32_t maxgap,
+                     int64_t* run_offsets /* (ss ? 2R : R) + 1 */, bsg_runs** runs, const bsg_opts* opts);
+int bsg_profile_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t binsize, int32_t shift,
+                            int32_t ss, int32_t requiredF, int32_t filteredF, int32_t pe_mid,
+                            int64_t* run_offsets, bsg_runs** runs);
 
 /*
  * writeSamAsBamAndIndex (src/bamsignals.cpp:496-534, .Call symbol bamsignals_writeSamAsBamAndIndex,

@@ -12,7 +12,8 @@ wall time of the whole Python call (for runs_host this includes reading the runs
 bytes to bytes_d2h).  device_mb_peak: the largest rise of the device's used memory (cudaMemGetInfo, polled every
 millisecond from a second thread during the timed calls) over what the process held before its first call - on a
 shared GPU, other processes' allocations would show up in it too.  Every arm digests its last result in dense
-bsg_output_layout() order (runs are expanded in chunks); the parent checks that all digests agree."""
+bsg_output_layout() order (runs are expanded in chunks); the parent checks that all digests agree.
+tools/profile_runs_bench.py drives its arms with the same code (measure_arm, run_arms)."""
 import argparse
 import hashlib
 import json
@@ -49,13 +50,32 @@ def workload(preset, gscale, density):
 
 
 def digest(res):
-    """blake2b of the coverage in bsg_output_layout() order, and its sum; runs are expanded CHUNK runs at a time."""
+    """blake2b of the result in bsg_output_layout() order, and its sum; runs are expanded CHUNK runs at a time.  A
+    strand-specific ProfileRuns is walked region by region, CHUNK bins at a time, its two rows interleaved
+    [s_0, a_0, s_1, ...] as in the dense layout."""
     import numpy as np
     h, total = hashlib.blake2b(), 0
 
     def host(x):
         return x if isinstance(x, np.ndarray) else x.cpu().numpy()
-    if hasattr(res, "lengths"):
+    if getattr(res, "ss", False) and hasattr(res, "lengths"):
+        lengths, values, off = host(res.lengths).astype(np.int64), host(res.values), res.offsets
+        ends = np.cumsum(lengths)
+        for i in range(len(res)):
+            rows = [(int(off[k]), int(off[k + 1])) for k in (2 * i, 2 * i + 1)]
+            base = [int(ends[a] - lengths[a]) if b > a else 0 for a, b in rows]    # the list's first bin, flat
+            nb = int(lengths[rows[0][0]:rows[0][1]].sum())
+            for b0 in range(0, nb, CHUNK):
+                b1 = min(nb, b0 + CHUNK)
+                part = np.empty(2 * (b1 - b0), np.int32)
+                for a, ((k0, k1), z) in enumerate(zip(rows, base)):
+                    e = ends[k0:k1] - z                                             # run ends, relative to the list
+                    lo, hi = np.searchsorted(e, b0, "right"), np.searchsorted(e, b1 - 1, "right") + 1
+                    seg = np.minimum(e[lo:hi], b1) - np.maximum(e[lo:hi] - lengths[k0 + lo:k0 + hi], b0)
+                    part[a::2] = np.repeat(values[k0 + lo:k0 + hi], seg)
+                h.update(memoryview(part))
+                total += int(part.sum(dtype=np.int64))
+    elif hasattr(res, "lengths"):
         n = int(res.offsets[-1])
         for a in range(0, n, CHUNK):
             dense = np.repeat(host(res.values[a:a + CHUNK]), host(res.lengths[a:a + CHUNK])).astype(np.int32)
@@ -83,14 +103,13 @@ class MemPoll:
             time.sleep(0.001)
 
 
-def run_arm(args):
+def measure_arm(args, call, n_elems, elem, head):
+    """Run `call(device, runs)` --warmup + --calls times for args.arm and print its JSON line: `head` first, then the
+    medians, the runs per output element (`elem`: "base", "bin") over n_elems, the peak device memory, the digest."""
     import torch
     import bamsignals_b200 as B
-    if B.lib().bsg_device_count() < 1:
-        raise SystemExit("coverage_runs_bench needs a CUDA device")
-    bam, info, gr, kw = workload(args.preset, args.gscale, args.density)
-    opts = B.default_opts(gpu_inflate=args.gpu_inflate)
     device = "cuda:0" if args.arm.endswith("device") else None
+    is_runs = args.arm.startswith("runs")
     torch.empty(1, device="cuda:0")                          # CUDA context + allocator set-up outside the timed calls
     poll = MemPoll(torch)
     th = None
@@ -101,32 +120,69 @@ def run_arm(args):
             th.start()
         res = None                                           # a fresh result per call, as a user's call has
         t0 = time.perf_counter()
-        res = B.bamCoverage(bam, gr, opts=opts, device=device, runs=args.arm.startswith("runs"), **kw)
+        res = call(device, is_runs)
         if device:
             torch.cuda.synchronize()
         wall = (time.perf_counter() - t0) * 1e3
         t = B.timings()
         if i >= args.warmup:
-            runs = int(res.offsets[-1]) if args.arm.startswith("runs") else None
+            runs = int(res.offsets[-1]) if is_runs else None
             read = 8 * runs if args.arm == "runs_host" else 0
             rows.append(dict(wall_ms=wall, ms_total=t["ms_total"], ms_d2h=t["ms_d2h"], bytes_d2h=t["bytes_d2h"],
                              bytes_pcie=t["bytes_d2h"] + read, ms_fetch=t["ms_fetch"], ms_kernels=t["ms_kernels"],
                              out_elems=t["out_elems"]))
     poll.stop = True
     th.join()
-    bases = int(sum(int(w) for w in gr.width))
-    runs = int(res.offsets[-1]) if args.arm.startswith("runs") else None
+    runs = int(res.offsets[-1]) if is_runs else None
     dig, total = digest(res)
     med = {k: statistics.median(r[k] for r in rows) for k in ("wall_ms", "ms_total", "ms_d2h", "bytes_d2h", "bytes_pcie",
                                                                 "ms_fetch", "ms_kernels")}
-    line = dict(preset=args.preset, gscale=args.gscale, density=args.density if args.preset == "genome_low" else 1.0,
-                arm=args.arm, call=f"bamCoverage {kw}", regions=len(gr), bases=bases, reads_in_bam=info["records"],
-                warmup=args.warmup, calls=args.calls, gpu_inflate=args.gpu_inflate, median=med,
-                ms_total_all=[round(r["ms_total"], 2) for r in rows], wall_ms_all=[round(r["wall_ms"], 2) for r in rows],
-                out_elems=int(rows[-1]["out_elems"]), runs=runs, runs_per_base=None if runs is None else runs / bases,
-                device_mb_peak=round(poll.peak / 2 ** 20, 1), result_sum=total, result_blake2b=dig)
+    line = dict(head)
+    line.update({"arm": args.arm, elem + "s": n_elems, "warmup": args.warmup, "calls": args.calls,
+                 "gpu_inflate": args.gpu_inflate, "median": med,
+                 "ms_total_all": [round(r["ms_total"], 2) for r in rows], "wall_ms_all": [round(r["wall_ms"], 2) for r in rows],
+                 "out_elems": int(rows[-1]["out_elems"]), "runs": runs,
+                 f"runs_per_{elem}": None if runs is None else runs / n_elems,
+                 "device_mb_peak": round(poll.peak / 2 ** 20, 1), "result_sum": total, "result_blake2b": dig})
     line.update(gpu_info())
     print(json.dumps(line), flush=True)
+
+
+def run_arm(args):
+    import bamsignals_b200 as B
+    if B.lib().bsg_device_count() < 1:
+        raise SystemExit("coverage_runs_bench needs a CUDA device")
+    bam, info, gr, kw = workload(args.preset, args.gscale, args.density)
+    opts = B.default_opts(gpu_inflate=args.gpu_inflate)
+    head = dict(preset=args.preset, gscale=args.gscale, density=args.density if args.preset == "genome_low" else 1.0,
+                arm=args.arm, call=f"bamCoverage {kw}", regions=len(gr))
+    bases = int(sum(int(w) for w in gr.width))
+    head.update(bases=bases, reads_in_bam=info["records"])
+    measure_arm(args, lambda device, runs: B.bamCoverage(bam, gr, opts=opts, device=device, runs=runs, **kw), bases, "base", head)
+
+
+def run_arms(args, script, child_args, skip=None):
+    """Every arm of args.arms in a fresh process (`script --arm <arm> child_args`); skip(arm) may return a reason to
+    leave an arm out, which becomes that arm's line.  Prints the lines (appended to args.out) with digests_equal over
+    the arms that ran; exits non-zero if they differ."""
+    lines = []
+    for arm in args.arms.split(","):
+        why = skip(arm) if skip else None
+        if why:
+            lines.append(dict(preset=args.preset, gscale=args.gscale, arm=arm, skipped=why, **gpu_info()))
+            continue
+        cmd = [sys.executable, os.path.abspath(script), "--arm", arm] + child_args
+        out = subprocess.run(cmd, check=True, stdout=subprocess.PIPE, text=True, cwd=ROOT).stdout
+        lines.append(json.loads(out.strip().splitlines()[-1]))
+    same = len({(ln["result_blake2b"], ln["result_sum"]) for ln in lines if "skipped" not in ln}) == 1
+    for ln in lines:
+        ln["digests_equal"] = same
+        print(json.dumps(ln), flush=True)
+        if args.out:
+            with open(args.out, "a") as f:
+                f.write(json.dumps(ln) + "\n")
+    if not same:
+        raise SystemExit("the arms' results differ")
 
 
 def main():
@@ -146,22 +202,8 @@ def main():
     if args.arm:
         return run_arm(args)
     workload(args.preset, args.gscale, args.density)       # generate once, outside the arms
-    lines = []
-    for arm in args.arms.split(","):
-        cmd = [sys.executable, os.path.abspath(__file__), "--arm", arm, "--preset", args.preset, "--gscale", repr(args.gscale),
-               "--density", repr(args.density), "--warmup", str(args.warmup), "--calls", str(args.calls),
-               "--gpu-inflate", str(args.gpu_inflate)]
-        out = subprocess.run(cmd, check=True, stdout=subprocess.PIPE, text=True, cwd=ROOT).stdout
-        lines.append(json.loads(out.strip().splitlines()[-1]))
-    same = len({(ln["result_blake2b"], ln["result_sum"]) for ln in lines}) == 1
-    for ln in lines:
-        ln["digests_equal"] = same
-        print(json.dumps(ln), flush=True)
-        if args.out:
-            with open(args.out, "a") as f:
-                f.write(json.dumps(ln) + "\n")
-    if not same:
-        raise SystemExit("the arms' results differ")
+    run_arms(args, __file__, ["--preset", args.preset, "--gscale", repr(args.gscale), "--density", repr(args.density),
+                              "--warmup", str(args.warmup), "--calls", str(args.calls), "--gpu-inflate", str(args.gpu_inflate)])
 
 
 if __name__ == "__main__":

@@ -4,7 +4,8 @@
     compute-sanitizer --tool racecheck python tools/sanitize_smoke.py
 Covers K0a inflate, K0b CRC32, K0c walk (speculate / link / scan / write), K1 decode (pileup and coverage
 instantiations), K3 join, K4 count, K4 profile (binsize 1 and the aggregated binsize >= 4 kernel, ss and not), K5
-coverage, the result-narrowing kernels and the one-thread publishers, and (where torch is installed) the tile kernels writing
+coverage, the result-narrowing kernels and the one-thread publishers, K5r coverage runs and K4r profile runs (every
+instantiation: binsize 1, 2..3 and >= 4, ss and not), and (where torch is installed) the tile kernels writing
 into a caller's device buffer at every 16-byte phase (bsg_*_device); results are checked against the oracle so that a
 sanitizer-clean run is also a correct one.  (The device-inflate path is forced: a job this small would otherwise be
 inflated by the host pool.)"""
@@ -46,6 +47,19 @@ big = B.GRanges(["chr1", "chr2", "chr3"] * 8, [1] * 24, [10000] * 24, ["+", "-",
 for rp in (0, 2):
     o2 = B.default_opts(gpu_inflate=1, result_pack=rp)
     a, b = B.bamCoverage(bam, big, paired_end="extend", opts=o2).as_list(), O.bamCoverage(bam, big, paired_end="extend").as_list()
+    assert all(np.array_equal(x, y) for x, y in zip(a, b))
+    launches += B.timings()["n_launches"]
+# run-length results (bsg_coverage_runs, bsg_profile_runs), expanded and compared with the oracle
+for kw in (dict(), dict(paired_end="extend")):
+    a, b = B.bamCoverage(bam, gr, opts=opts, runs=True, **kw).to_dense().as_list(), O.bamCoverage(bam, gr, **kw).as_list()
+    assert all(np.array_equal(x, y) for x, y in zip(a, b))
+    launches += B.timings()["n_launches"]
+for kw in (dict(binsize=1, ss=True, shift=75), dict(binsize=1), dict(binsize=3, ss=True), dict(binsize=2),
+           dict(binsize=5, ss=True, paired_end="midpoint"), dict(binsize=50)):
+    import warnings
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        a, b = B.bamProfile(bam, gr, opts=opts, runs=True, **kw).to_dense().as_list(), O.bamProfile(bam, gr, **kw).as_list()
     assert all(np.array_equal(x, y) for x, y in zip(a, b))
     launches += B.timings()["n_launches"]
 # device output (bsg_*_device) into slices of every 16-byte phase of one allocation: the tile kernels place their shared

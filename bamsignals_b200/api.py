@@ -20,6 +20,9 @@ Coverage as runs (beyond the R interface): `bamCoverage(..., runs=True)`, `cover
 bsg_coverage_runs, on the host or (device=) in torch tensors.  Profiles likewise: `bamProfile(..., runs=True)`,
 `profile_runs_core` and `Stage.profile_runs` return a ProfileRuns (bsg_profile_runs), runs over bins per region and
 strand row.
+
+Strand-specific coverage (beyond the R interface): `ss=True` on bamCoverage, coverage_core, coverage_runs_core,
+Stage.coverage and Stage.coverage_runs counts sense and antisense coverage in one pass (bsg_coverage_ss*).
 """
 from __future__ import annotations
 
@@ -204,15 +207,27 @@ def _expand_runs(lengths, values, offsets):
 
 class _RunLists:
     """Flat int32 `lengths` / `values` (numpy arrays or torch tensors on one device) and numpy int64 `offsets`: list k
-    is lengths[offsets[k]:offsets[k+1]] elements of values[offsets[k]:offsets[k+1]]."""
+    is lengths[offsets[k]:offsets[k+1]] elements of values[offsets[k]:offsets[k+1]].  Without `ss` list i is region i;
+    with `ss` list 2i is region i's sense row and list 2i+1 its antisense row.  len() is R; [i] is (lengths, values), or
+    with ss a (sense, antisense) pair of them."""
 
-    def __init__(self, lengths, values, offsets):
+    def __init__(self, lengths, values, offsets, ss=False):
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         if offsets.ndim != 1 or len(offsets) < 1 or offsets[0] != 0 or (np.diff(offsets) < 0).any():
             raise ValueError("offsets must be a non-decreasing int64 vector that starts at 0")
         if len(lengths) != offsets[-1] or len(values) != offsets[-1]:
             raise ValueError(f"lengths and values must have offsets[-1] = {int(offsets[-1])} elements")
         self.lengths, self.values, self.offsets = lengths, values, offsets
+        self.ss = bool(ss)
+        if self.ss and (len(self.offsets) - 1) % 2:
+            raise ValueError("a strand-specific result has two lists per region: offsets must have 2R + 1 entries")
+
+    def __len__(self):
+        return (len(self.offsets) - 1) // (2 if self.ss else 1)
+
+    def __getitem__(self, i):
+        i = self._index(i)
+        return (self._list(2 * i), self._list(2 * i + 1)) if self.ss else self._list(i)
 
     def _list(self, k):
         a, b = int(self.offsets[k]), int(self.offsets[k + 1])
@@ -225,50 +240,8 @@ class _RunLists:
             raise IndexError("subscript out of bounds")
         return int(i)
 
-
-class CoverageRuns(_RunLists):
-    """bamCoverage as runs: region i's coverage (in region orientation) is lengths[offsets[i]:offsets[i+1]] bases of
-    values[offsets[i]:offsets[i+1]].  `lengths` / `values` are flat int32 numpy arrays or torch tensors on one device;
-    `offsets` is numpy int64 (R + 1).  Adjacent runs of a region differ in value, every length is >= 1, a zero-width
-    region has no runs.  The same thing as an RleList of GenomicAlignments::coverage, one Rle per region."""
-
-    def __len__(self):
-        return len(self.offsets) - 1
-
-    def __getitem__(self, i):
-        return self._list(self._index(i))
-
     def to_dense(self) -> CountSignals:
-        """The bamCoverage result these runs describe (a CountSignals over one flat buffer on the runs' device)."""
-        flat, dense_off = _expand_runs(self.lengths, self.values, self.offsets)
-        return CountSignals(None, False, flat=flat, offsets=dense_off)
-
-    def __repr__(self):
-        return f"CoverageRuns object with {len(self)} regions and {int(self.offsets[-1])} runs"
-
-
-class ProfileRuns(_RunLists):
-    """bamProfile as runs over bins (in region orientation, a partial last bin is one element).  Without `ss` list i is
-    region i's profile; with `ss` list 2i is region i's sense row and list 2i+1 its antisense row, so `offsets` has
-    (ss ? 2R : R) + 1 entries.  Adjacent runs of a list differ in value, every length is >= 1, a list's lengths sum to
-    its bin count, a zero-width region has no runs.  len() is R; [i] is (lengths, values), or with ss a
-    (sense, antisense) pair of them."""
-
-    def __init__(self, lengths, values, offsets, ss):
-        super().__init__(lengths, values, offsets)
-        self.ss = bool(ss)
-        if self.ss and (len(self.offsets) - 1) % 2:
-            raise ValueError("a strand-specific result has two lists per region: offsets must have 2R + 1 entries")
-
-    def __len__(self):
-        return (len(self.offsets) - 1) // (2 if self.ss else 1)
-
-    def __getitem__(self, i):
-        i = self._index(i)
-        return (self._list(2 * i), self._list(2 * i + 1)) if self.ss else self._list(i)
-
-    def to_dense(self) -> CountSignals:
-        """The bamProfile result these runs describe (a CountSignals over one flat buffer on the runs' device, with the
+        """The dense result these runs describe (a CountSignals over one flat buffer on the runs' device, with the
         (2, w) [sense; antisense] views when ss)."""
         if not self.ss:
             flat, dense_off = _expand_runs(self.lengths, self.values, self.offsets)
@@ -294,6 +267,35 @@ class ProfileRuns(_RunLists):
             flat = np.empty(2 * len(sense), dtype=sense.dtype)
             flat[0::2], flat[1::2] = sense, anti
         return CountSignals(None, True, flat=flat, offsets=2 * bins)
+
+
+class CoverageRuns(_RunLists):
+    """bamCoverage as runs: region i's coverage (in region orientation) is lengths[offsets[i]:offsets[i+1]] bases of
+    values[offsets[i]:offsets[i+1]].  `lengths` / `values` are flat int32 numpy arrays or torch tensors on one device;
+    `offsets` is numpy int64 (R + 1).  Adjacent runs of a region differ in value, every length is >= 1, a zero-width
+    region has no runs.  The same thing as an RleList of GenomicAlignments::coverage, one Rle per region.
+    With `ss` (strand-specific coverage) the lists are those of a strand-specific ProfileRuns: list 2i is region i's
+    sense row, list 2i+1 its antisense row, `offsets` has 2R + 1 entries, [i] is the (sense, antisense) pair and
+    to_dense() gives bamCoverage(..., ss=True)'s CountSignals."""
+
+    def __init__(self, lengths, values, offsets, ss=False):
+        super().__init__(lengths, values, offsets, ss)
+
+    def __repr__(self):
+        if self.ss:
+            return f"CoverageRuns object with {len(self)} strand-specific regions and {int(self.offsets[-1])} runs"
+        return f"CoverageRuns object with {len(self)} regions and {int(self.offsets[-1])} runs"
+
+
+class ProfileRuns(_RunLists):
+    """bamProfile as runs over bins (in region orientation, a partial last bin is one element).  Without `ss` list i is
+    region i's profile; with `ss` list 2i is region i's sense row and list 2i+1 its antisense row, so `offsets` has
+    (ss ? 2R : R) + 1 entries.  Adjacent runs of a list differ in value, every length is >= 1, a list's lengths sum to
+    its bin count, a zero-width region has no runs.  len() is R; [i] is (lengths, values), or with ss a
+    (sense, antisense) pair of them."""
+
+    def __init__(self, lengths, values, offsets, ss):
+        super().__init__(lengths, values, offsets, ss)
 
     def __repr__(self):
         kind = "strand-specific" if self.ss else "strand-unspecific"
@@ -428,6 +430,19 @@ def lib():
     L.bsg_profile_runs.restype = C.c_int
     L.bsg_profile_runs_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 7 + [i64p, C.POINTER(C.c_void_p)]
     L.bsg_profile_runs_staged.restype = C.c_int
+    L.bsg_coverage_ss.argtypes = region_args + [i32p] + [C.c_int32] * 6 + [i32p, i64p, C.POINTER(C.POINTER(C.c_int32)),
+                                                                       C.POINTER(BsgOpts)]
+    L.bsg_coverage_ss.restype = C.c_int
+    L.bsg_coverage_ss_device.argtypes = region_args + [i32p] + [C.c_int32] * 6 + [C.c_void_p, i64p, C.c_void_p, C.POINTER(BsgOpts)]
+    L.bsg_coverage_ss_device.restype = C.c_int
+    L.bsg_coverage_ss_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 5 + [i32p, i64p]
+    L.bsg_coverage_ss_staged.restype = C.c_int
+    L.bsg_coverage_ss_staged_device.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 5 + [C.c_void_p, i64p, C.c_void_p]
+    L.bsg_coverage_ss_staged_device.restype = C.c_int
+    L.bsg_coverage_runs_ss.argtypes = region_args + [i32p] + [C.c_int32] * 6 + [i64p, C.POINTER(C.c_void_p), C.POINTER(BsgOpts)]
+    L.bsg_coverage_runs_ss.restype = C.c_int
+    L.bsg_coverage_runs_ss_staged.argtypes = [C.c_void_p, i32p] + [C.c_int32] * 5 + [i64p, C.POINTER(C.c_void_p)]
+    L.bsg_coverage_runs_ss_staged.restype = C.c_int
     L.bsg_runs_read.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.bsg_runs_read.restype = C.c_int
     L.bsg_runs_free.argtypes = [C.c_void_p]
@@ -579,29 +594,32 @@ def pileup_core(bampath, gr, tlen_filter, mapqual=0, binsize=1, shift=0, ss=Fals
 
 
 def coverage_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, maxgap=16385,
-                  opts: Optional[BsgOpts] = None, _lazy=False, out=None):
-    """The .Call('bamsignals_coverage_core') entry point (src/bamsignals.cpp:474-494).  `out`: as for pileup_core."""
+                  opts: Optional[BsgOpts] = None, _lazy=False, out=None, ss=False):
+    """The .Call('bamsignals_coverage_core') entry point (src/bamsignals.cpp:474-494).  `out`: as for pileup_core.
+    ss=True (beyond the reference): strand-specific coverage (bsg_coverage_ss), one (2, w) [sense; antisense] matrix per
+    region, the layout of a binsize-1 strand-specific profile."""
     m = marshal_regions(gr)
-    off = output_layout(m.width, 1, False)
+    ss = bool(ss)
+    off = output_layout(m.width, 1, ss)
     tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
     if out is not None:
         ptr, stream = device_buffer(out, int(off[-1]))
-        _check(lib().bsg_coverage_device(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
-                                         _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
-                                         None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
-                                         int(filteredF), int(bool(tspan)), int(maxgap), ptr, _p(off, C.c_int64), stream,
-                                         None if opts is None else C.byref(opts)))
+        _check(lib().bsg_coverage_ss_device(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                            _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                            None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
+                                            int(filteredF), int(bool(tspan)), int(ss), int(maxgap), ptr, _p(off, C.c_int64),
+                                            stream, None if opts is None else C.byref(opts)))
         return (out, off) if _lazy else out
     flat = np.empty(int(off[-1]), dtype=np.int32)
-    rc = lib().bsg_coverage(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
-                            _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
-                            None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF), int(filteredF),
-                            int(bool(tspan)), int(maxgap), _p(flat, C.c_int32), _p(off, C.c_int64), None,
-                            None if opts is None else C.byref(opts))
+    rc = lib().bsg_coverage_ss(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                               _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                               None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF), int(filteredF),
+                               int(bool(tspan)), int(ss), int(maxgap), _p(flat, C.c_int32), _p(off, C.c_int64), None,
+                               None if opts is None else C.byref(opts))
     _check(rc)
     if _lazy:
         return flat, off
-    return split_signals(flat, off, False)
+    return split_signals(flat, off, ss)
 
 
 def _take_runs(h, offsets, device):
@@ -624,22 +642,22 @@ def _take_runs(h, offsets, device):
 
 
 def coverage_runs_core(bampath, gr, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, maxgap=16385,
-                       opts: Optional[BsgOpts] = None, device=None) -> CoverageRuns:
-    """coverage_core's arguments -> the coverage as runs (bsg_coverage_runs).  device=None: numpy arrays on the host;
+                       opts: Optional[BsgOpts] = None, device=None, ss=False) -> CoverageRuns:
+    """coverage_core's arguments -> the coverage as runs (bsg_coverage_runs_ss).  device=None: numpy arrays on the host;
     device= a CUDA device: torch tensors there (the call runs on that device; only the offsets cross PCIe)."""
     m = marshal_regions(gr)
     dev = None if device is None else _cuda_device(device)
     if dev is not None and opts is None:
         opts = default_opts(devices=[dev.index])
     tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
-    offsets = np.zeros(m.R + 1, dtype=np.int64)
+    offsets = np.zeros((2 if ss else 1) * m.R + 1, dtype=np.int64)
     h = C.c_void_p()
-    _check(lib().bsg_coverage_runs(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
-                                   _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
-                                   None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
-                                   int(filteredF), int(bool(tspan)), int(maxgap), _p(offsets, C.c_int64), C.byref(h),
-                                   None if opts is None else C.byref(opts)))
-    return CoverageRuns(*_take_runs(h, offsets, dev), offsets)
+    _check(lib().bsg_coverage_runs_ss(os.fsencode(bampath), m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                      _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8),
+                                      None if tl is None else _p(tl, C.c_int32), int(mapqual), int(requiredF),
+                                      int(filteredF), int(bool(tspan)), int(bool(ss)), int(maxgap), _p(offsets, C.c_int64),
+                                      C.byref(h), None if opts is None else C.byref(opts)))
+    return CoverageRuns(*_take_runs(h, offsets, dev), offsets, ss)
 
 
 def profile_runs_core(bampath, gr, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1,
@@ -691,31 +709,33 @@ class Stage:
                                        None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
         return flat
 
-    def coverage(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, want_output=True, out=None):
-        off = output_layout(self._m.width, 1, False)
+    def coverage(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, want_output=True, out=None, ss=False):
+        """ss=True: strand-specific coverage, the flat interleaved layout of a binsize-1 strand-specific profile."""
+        off = output_layout(self._m.width, 1, bool(ss))
         tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
         if out is not None:
             ptr, stream = device_buffer(out, int(off[-1]))
-            _check(lib().bsg_coverage_staged_device(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
-                                                    int(requiredF), int(filteredF), int(bool(tspan)), ptr,
-                                                    _p(off, C.c_int64), stream))
+            _check(lib().bsg_coverage_ss_staged_device(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                                       int(requiredF), int(filteredF), int(bool(tspan)), int(bool(ss)), ptr,
+                                                       _p(off, C.c_int64), stream))
             return out
         flat = np.empty(int(off[-1]), dtype=np.int32) if want_output else None
-        _check(lib().bsg_coverage_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
-                                         int(requiredF), int(filteredF), int(bool(tspan)),
-                                         None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
+        _check(lib().bsg_coverage_ss_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                            int(requiredF), int(filteredF), int(bool(tspan)), int(bool(ss)),
+                                            None if flat is None else _p(flat, C.c_int32), _p(off, C.c_int64)))
         return flat
 
-    def coverage_runs(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, device=None) -> CoverageRuns:
-        """coverage() as runs (bsg_coverage_runs_staged); device= must be the session's device."""
+    def coverage_runs(self, tlen_filter, mapqual=0, requiredF=0, filteredF=-1, tspan=False, device=None,
+                      ss=False) -> CoverageRuns:
+        """coverage() as runs (bsg_coverage_runs_ss_staged); device= must be the session's device."""
         dev = None if device is None else _cuda_device(device)
         tl = None if tlen_filter is None else np.asarray(tlen_filter, dtype=np.int32)
-        offsets = np.zeros(self._m.R + 1, dtype=np.int64)
+        offsets = np.zeros((2 if ss else 1) * self._m.R + 1, dtype=np.int64)
         h = C.c_void_p()
-        _check(lib().bsg_coverage_runs_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
-                                              int(requiredF), int(filteredF), int(bool(tspan)), _p(offsets, C.c_int64),
-                                              C.byref(h)))
-        return CoverageRuns(*_take_runs(h, offsets, dev), offsets)
+        _check(lib().bsg_coverage_runs_ss_staged(self._h, None if tl is None else _p(tl, C.c_int32), int(mapqual),
+                                                 int(requiredF), int(filteredF), int(bool(tspan)), int(bool(ss)),
+                                                 _p(offsets, C.c_int64), C.byref(h)))
+        return CoverageRuns(*_take_runs(h, offsets, dev), offsets, ss)
 
     def profile_runs(self, tlen_filter, mapqual=0, binsize=1, shift=0, ss=False, requiredF=0, filteredF=-1, pe_mid=False,
                      device=None) -> ProfileRuns:
@@ -811,14 +831,18 @@ def bamProfile(bampath, gr, binsize=1, mapqual=0, shift=0, ss=False, paired_end=
 
 # runs=True: the coverage as a CoverageRuns (run-length pairs per region) instead of a CountSignals; with device= its
 # arrays are torch tensors on that device.
+# ss=True (beyond the R interface): strand-specific coverage, a (2, w) [sense; antisense] matrix per region.  A read's
+# strand is its flag bit 0x10, relative to the region as in bamProfile; with paired_end="extend" only first mates count
+# and a fragment goes to its first mate's strand.
 def bamCoverage(bampath, gr, mapqual=0, paired_end=("ignore", "extend"), tlenFilter=None, filteredFlag=-1,
-                verbose=False, opts=None, device=None, runs=False):
+                verbose=False, opts=None, device=None, runs=False, ss=False):
     pe = _match_arg(paired_end, ("ignore", "extend"))
     bampath = os.path.expanduser(bampath)
+    ss = bool(ss)
     if runs:
         return coverage_runs_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), flagMask(pe), _trunc(filteredFlag),
-                                  pe == "extend", opts=opts, device=device)
-    out = None if device is None else _empty_on(device, gr, 1, False)
+                                  pe == "extend", opts=opts, device=device, ss=ss)
+    out = None if device is None else _empty_on(device, gr, 1, ss)
     flat, off = coverage_core(bampath, gr, _tlen(tlenFilter, pe), _trunc(mapqual), flagMask(pe), _trunc(filteredFlag),
-                              pe == "extend", opts=opts, _lazy=True, out=out)
-    return CountSignals(None, False, flat=flat, offsets=off)
+                              pe == "extend", opts=opts, _lazy=True, out=out, ss=ss)
+    return CountSignals(None, ss, flat=flat, offsets=off)

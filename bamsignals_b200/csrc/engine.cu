@@ -596,14 +596,14 @@ public:
     }
 
     // Staged sessions: decode + filter every resident raw batch again (K1) in ONE launch, timed.
-    void decode_resident(Mode mode, const FilterParams& fp) {
+    void decode_resident(Mode mode, const FilterParams& fp, int ss = 0) {
         DeviceCtx& c = *ctx_;
         BSG_CUDA(cudaMemsetAsync(c.scalars.p, 0, sizeof(DeviceScalars), c.s_comp));
         if (resident_.empty()) return;
         Span sp{c.timing_event(), c.timing_event()};
         BSG_CUDA(cudaEventRecord(sp.a, c.s_comp));
         launch_decode_table(batch_table_.as<DecodeBatch>(), int(resident_.size()), resident_chunks_, table(),
-                            mode == MODE_COVERAGE, fp, c.scalars.as<DeviceScalars>(), c.s_comp);
+                            mode == MODE_COVERAGE, ss != 0, fp, c.scalars.as<DeviceScalars>(), c.s_comp);
         BSG_CUDA(cudaEventRecord(sp.b, c.s_comp));
         kt_.decode.push_back(sp); kt_.launches += 1;
     }
@@ -663,12 +663,17 @@ public:
             if (R > 0 && out_offsets[0] < 0) fail(BSG_EARG, "out_offsets must not be negative");
             for (int64_t i = 0; i < R; ++i) {
                 const int64_t want = mode == MODE_COUNT ? mult
-                                   : (mode == MODE_COVERAGE ? int64_t(rg_.width[i])
+                                   : (mode == MODE_COVERAGE ? mult * int64_t(rg_.width[i])
                                                             : mult * ((int64_t(rg_.width[i]) + binsize - 1) / binsize));
                 if (out_offsets[i + 1] - out_offsets[i] != want)
                     fail(BSG_EARG, "out_offsets[" + std::to_string(i + 1) + "] - out_offsets[" + std::to_string(i) + "] is " +
                                    std::to_string(out_offsets[i + 1] - out_offsets[i]) + ", the layout of this call needs " + std::to_string(want) +
                                    " (see bsg_output_layout)");
+                // the stranded read table tells the strands apart by the sign of a read's end (kernels.cuh), so a read that
+                // ends before position 0 is not counted: no region may reach there
+                if (mode == MODE_COVERAGE && ss && rg_.loc[i] < 0)
+                    fail(BSG_EARG, "strand-specific coverage needs regions that start at position 1 or later (region " +
+                                   std::to_string(i + 1) + ")");
             }
         }
     }
@@ -822,15 +827,16 @@ public:
     }
     void use_host_output() { dev_out_ = DeviceOutput{}; runs_ = RunsOutput{}; }
     // The next call counts coverage or a profile as runs (count_runs) into `res`, and fills the caller's run_offsets
-    // (R + 1 entries, or 2R + 1 for a strand-specific profile).
+    // (R + 1 entries, or 2R + 1 when strand-specific).
     void use_runs_output(bsg_runs* res, int64_t* run_offsets) {
         dev_out_ = DeviceOutput{};
         runs_ = RunsOutput{res, run_offsets};
     }
-    // bsg_output_layout() of bamCoverage for this session's regions: the tiles are cut from it
-    std::vector<int64_t> coverage_layout() const {
+    // bsg_output_layout() of bamCoverage (strand-specific with ss) for this session's regions: the tiles are cut from it
+    std::vector<int64_t> coverage_layout(int ss) const {
+        const int64_t mult = ss ? 2 : 1;
         std::vector<int64_t> off(size_t(rg_.R) + 1, 0);
-        for (int64_t i = 0; i < rg_.R; ++i) off[i + 1] = off[i] + rg_.width[i];
+        for (int64_t i = 0; i < rg_.R; ++i) off[i + 1] = off[i] + mult * rg_.width[i];
         return off;
     }
     // bsg_output_layout() of bamProfile (binsize >= 1) for this session's regions
@@ -888,7 +894,7 @@ private:
             BSG_CUDA(cudaEventRecord(sp.a, st));
             if (cnt_.mode == MODE_COUNT) launch_count(tt, n, c0, c1, cnt_.ss, cnt_.dst, sc, st);
             else if (cnt_.mode == MODE_PROFILE) launch_profile(tt, n, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, cnt_.dst, sc, st);
-            else launch_coverage(tt, n, c0, c1, max_tile_ints_, cnt_.dst, sc, st);
+            else launch_coverage(tt, n, c0, c1, cnt_.ss, max_tile_ints_, cnt_.dst, sc, st);
             BSG_CUDA(cudaEventRecord(sp.b, st));
             kt_.count.push_back(sp); kt_.launches += 1;
             if (cnt_.want_output) ship_tiles(t0, t1, sp.b);
@@ -896,17 +902,17 @@ private:
         cnt_.t_done = t1;
     }
 
-    // Coverage (DESIGN.md §10) or a profile (§11) as runs over ALL tiles (t0 == 0, advance() never counts early): count
-    // pass + scans, the list spans come back (the only D2H besides the control scalars), the result is allocated at its
-    // exact size, then the write pass.  A list is a region, or with a strand-specific profile one strand row of a region
-    // (list mult * i + a); every tile holds one virtual tile per row: row a of the j-th of region i's n_i tiles, T_i
-    // its first, is v = mult * T_i + a * n_i + j, so that a list's pieces are consecutive (identity when mult is 1).
+    // Coverage (DESIGN.md §10, §12) or a profile (§11) as runs over ALL tiles (t0 == 0, advance() never counts early):
+    // count pass + scans, the list spans come back (the only D2H besides the control scalars), the result is allocated at
+    // its exact size, then the write pass.  A list is a region, or with ss one strand row of a region (list mult * i + a);
+    // every tile holds one virtual tile per row: row a of the j-th of region i's n_i tiles, T_i its first, is
+    // v = mult * T_i + a * n_i + j, so that a list's pieces are consecutive (identity when mult is 1).
     // Device memory: 28 bytes per virtual tile (+4 with ss), 24 per list, 8 per run.
     void count_runs(const TileTable& tt, int64_t nt, cudaStream_t st) {
         DeviceCtx& c = *ctx_;
         if (nt != n_tiles_) fail(BSG_EARG, "internal error: runs are counted over all tiles at once");
         const bool profile = cnt_.mode == MODE_PROFILE;
-        const int64_t mult = profile && cnt_.ss ? 2 : 1;
+        const int64_t mult = cnt_.ss ? 2 : 1;
         const int64_t R = rg_.R, L = mult * R, nv = mult * nt;
         const int64_t up = mult == 2 ? 3 : 2;                  // uploaded per virtual tile: list, rel (and vt with ss)
         runs_tiles_.resize(size_t(nv * up));
@@ -939,7 +945,7 @@ private:
         if (nv) BSG_CUDA(cudaMemcpyAsync(ri, runs_tiles_.data(), size_t(nv * up) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         if (L) BSG_CUDA(cudaMemsetAsync(rt.rfirst, 0, size_t(L) * 2 * sizeof(int64_t), st));
         if (profile) launch_profile_runs(tt, nt, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, rt, vt, L, run_off, st);
-        else launch_coverage_runs(tt, nt, c0, c1, max_tile_ints_, rt, R, run_off, st);
+        else launch_coverage_runs(tt, nt, c0, c1, cnt_.ss, max_tile_ints_, rt, vt, L, run_off, st);
         BSG_CUDA(cudaMemcpyAsync(c.h_runs.p, run_off, (size_t(L) + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         BSG_CUDA(cudaStreamSynchronize(st));
         BSG_CUDA(cudaGetLastError());
@@ -952,7 +958,7 @@ private:
         BSG_CUDA(cudaMalloc(&res.values, bytes));
         BSG_CUDA(cudaMemsetAsync(res.lengths, 0, bytes, st));
         if (profile) launch_profile_runs_write(tt, nt, c0, c1, cnt_.ss, cnt_.binsize, max_tile_ints_, rt, vt, run_off, res.lengths, res.values, st);
-        else launch_coverage_runs_write(tt, nt, c0, c1, max_tile_ints_, rt, run_off, res.lengths, res.values, st);
+        else launch_coverage_runs_write(tt, nt, c0, c1, cnt_.ss, max_tile_ints_, rt, vt, run_off, res.lengths, res.values, st);
         BSG_CUDA(cudaEventRecord(sp.b, st));
         kt_.count.push_back(sp); kt_.launches += nt ? 3 : 1;
         tm_.out_elems = 2 * res.n;
@@ -1286,7 +1292,7 @@ private:
                 Span sp{c.timing_event(), c.timing_event()};
                 BSG_CUDA(cudaEventRecord(sp.a, c.s_comp));
                 if (!cnt_.active) fail(BSG_EARG, "internal error: streaming decode without a counting call");
-                launch_decode(DecodeBatch{d_raw, d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.fp,
+                launch_decode(DecodeBatch{d_raw, d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
                               c.scalars.as<DeviceScalars>(), c.s_comp);
                 BSG_CUDA(cudaEventRecord(sp.b, c.s_comp));
                 BSG_CUDA(cudaEventRecord(c.ev_free[slot], c.s_comp));
@@ -1574,7 +1580,7 @@ private:
                 Span sp{c.timing_event(), c.timing_event()};
                 BSG_CUDA(cudaEventRecord(sp.a, c.s_hi));
                 if (!cnt_.active) fail(BSG_EARG, "internal error: streaming decode without a counting call");
-                launch_decode(DecodeBatch{up.d_raw, up.d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.fp,
+                launch_decode(DecodeBatch{up.d_raw, up.d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
                               c.scalars.as<DeviceScalars>(), c.s_hi);
                 BSG_CUDA(cudaEventRecord(sp.b, c.s_hi));
                 kt_.decode.push_back(sp); kt_.launches += n > 0;
@@ -1883,6 +1889,19 @@ int output_device(const int32_t* d_out, int64_t R, const int64_t* out_offsets) {
     return a.device;
 }
 
+// With ss, bsg_coverage_ss / bsg_coverage_ss_device refuse a layout that is not the stranded one before any device work,
+// so that a caller who passes bamCoverage's unstranded offsets learns it even without a GPU (validate_layout checks the
+// layout again once the regions are resolved).
+void check_stranded_layout(int64_t R, const int32_t* width, const int64_t* out_offsets) {
+    if (!out_offsets) fail(BSG_EARG, "out_offsets is required");
+    if (R < 0 || (R > 0 && !width)) fail(BSG_EARG, "invalid region arrays");
+    for (int64_t i = 0; i < R; ++i)
+        if (out_offsets[i + 1] - out_offsets[i] != 2 * int64_t(width[i]))
+            fail(BSG_EARG, "out_offsets[" + std::to_string(i + 1) + "] - out_offsets[" + std::to_string(i) + "] is " +
+                           std::to_string(out_offsets[i + 1] - out_offsets[i]) + ", strand-specific coverage needs 2 x width = " +
+                           std::to_string(2 * int64_t(width[i])) + " (see bsg_output_layout with binsize 1 and ss)");
+}
+
 // The device a bsg_*_device call runs on: the one that owns d_out; opts may name it, but only that one.
 int device_for_output(const int32_t* d_out, int64_t R, const int64_t* out_offsets, const bsg_opts* opts) {
     const int dev = output_device(d_out, R, out_offsets);
@@ -2004,25 +2023,34 @@ int bsg_pileup(const char* bampath, int64_t R, const char* const* seq_levels, in
 
 int bsg_coverage(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
                  const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
-                 int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t /*maxgap*/, int32_t* out,
+                 int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t maxgap, int32_t* out,
                  const int64_t* out_offsets, int32_t* const* out_ptrs, const bsg_opts* opts) {
+    return bsg_coverage_ss(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, tlen_filter, mapqual, requiredF,
+                           filteredF, tspan, 0, maxgap, out, out_offsets, out_ptrs, opts);
+}
+
+int bsg_coverage_ss(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                    const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                    int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t ss, int32_t /*maxgap*/,
+                    int32_t* out, const int64_t* out_offsets, int32_t* const* out_ptrs, const bsg_opts* opts) {
     return guarded([&] {
         const double t0 = now_ms();
+        if (ss) check_stranded_layout(R, width, out_offsets);
         const bsg_opts o = effective_opts(opts);
         validate_devices(o);
         if (o.n_devices > 1) {
             run_multi_device(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, o, MODE_COVERAGE,
-                             make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan), 1, 0,
+                             make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan), 1, ss != 0,
                              ext_coverage(tlen_filter, tspan), out, out_offsets, out_ptrs, t0);
             return;
         }
         Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts);
         const int64_t ext = ext_coverage(tlen_filter, tspan);
         s.start_plan(ext);
-        s.validate_layout(MODE_COVERAGE, 1, 0, out_offsets);
+        s.validate_layout(MODE_COVERAGE, 1, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
         if (out && out_offsets) s.request_prefault(out, out_offsets[R]);
-        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, 0, ext, out, out_offsets, out_ptrs, true, s.setup_stream()); });
+        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, ss != 0, ext, out, out_offsets, out_ptrs, true, s.setup_stream()); });
         s.stage(ext, false);
         s.finish_count();
         s.finish_timings(t0);
@@ -2056,19 +2084,28 @@ int bsg_pileup_device(const char* bampath, int64_t R, const char* const* seq_lev
 
 int bsg_coverage_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
                         const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
-                        int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t /*maxgap*/,
+                        int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t maxgap,
                         int32_t* d_out, const int64_t* out_offsets, void* stream, const bsg_opts* opts) {
+    return bsg_coverage_ss_device(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, tlen_filter, mapqual, requiredF,
+                                  filteredF, tspan, 0, maxgap, d_out, out_offsets, stream, opts);
+}
+
+int bsg_coverage_ss_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                           const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                           int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t ss, int32_t /*maxgap*/,
+                           int32_t* d_out, const int64_t* out_offsets, void* stream, const bsg_opts* opts) {
     return guarded([&] {
         const double t0 = now_ms();
+        if (ss) check_stranded_layout(R, width, out_offsets);
         KeepCurrentDevice keep;
         const int dev = device_for_output(d_out, R, out_offsets, opts);
         Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts, dev);
         const int64_t ext = ext_coverage(tlen_filter, tspan);
         s.start_plan(ext);
-        s.validate_layout(MODE_COVERAGE, 1, 0, out_offsets);
+        s.validate_layout(MODE_COVERAGE, 1, ss != 0, out_offsets);
         s.use_device_output(d_out, static_cast<cudaStream_t>(stream));
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
-        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, 0, ext, nullptr, out_offsets, nullptr, false, s.setup_stream()); });
+        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, ss != 0, ext, nullptr, out_offsets, nullptr, false, s.setup_stream()); });
         s.stage(ext, false);
         s.finish_count();
         s.finish_timings(t0);
@@ -2124,6 +2161,11 @@ int bsg_pileup_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual
 
 int bsg_coverage_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
                         int32_t filteredF, int32_t tspan, int32_t* out, const int64_t* out_offsets) {
+    return bsg_coverage_ss_staged(st, tlen_filter, mapqual, requiredF, filteredF, tspan, 0, out, out_offsets);
+}
+
+int bsg_coverage_ss_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                           int32_t filteredF, int32_t tspan, int32_t ss, int32_t* out, const int64_t* out_offsets) {
     if (!st) { g_err = "null stage"; return BSG_EARG; }
     return guarded([&] {
         if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
@@ -2131,10 +2173,10 @@ int bsg_coverage_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqu
         st->s->reset_counters();
         st->s->require_ext(ext_coverage(tlen_filter, tspan));
         st->s->use_host_output();
-        st->s->prepare_tiles(MODE_COVERAGE, 1, 0, out_offsets);
+        st->s->prepare_tiles(MODE_COVERAGE, 1, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
-        st->s->decode_resident(MODE_COVERAGE, fp);
-        st->s->count(MODE_COVERAGE, fp, 1, 0, out, out_offsets, nullptr, out != nullptr);
+        st->s->decode_resident(MODE_COVERAGE, fp, ss != 0);
+        st->s->count(MODE_COVERAGE, fp, 1, ss != 0, out, out_offsets, nullptr, out != nullptr);
         st->s->finish_timings(t0);
     });
 }
@@ -2163,6 +2205,12 @@ int bsg_pileup_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t 
 
 int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
                                int32_t filteredF, int32_t tspan, int32_t* d_out, const int64_t* out_offsets, void* stream) {
+    return bsg_coverage_ss_staged_device(st, tlen_filter, mapqual, requiredF, filteredF, tspan, 0, d_out, out_offsets, stream);
+}
+
+int bsg_coverage_ss_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                                  int32_t filteredF, int32_t tspan, int32_t ss, int32_t* d_out, const int64_t* out_offsets,
+                                  void* stream) {
     if (!st) { g_err = "null stage"; return BSG_EARG; }
     return guarded([&] {
         if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
@@ -2173,18 +2221,26 @@ int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_
         st->s->reset_counters();
         st->s->require_ext(ext_coverage(tlen_filter, tspan));
         st->s->use_device_output(d_out, static_cast<cudaStream_t>(stream));
-        st->s->prepare_tiles(MODE_COVERAGE, 1, 0, out_offsets);
+        st->s->prepare_tiles(MODE_COVERAGE, 1, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
-        st->s->decode_resident(MODE_COVERAGE, fp);
-        st->s->count(MODE_COVERAGE, fp, 1, 0, nullptr, out_offsets, nullptr, false);
+        st->s->decode_resident(MODE_COVERAGE, fp, ss != 0);
+        st->s->count(MODE_COVERAGE, fp, 1, ss != 0, nullptr, out_offsets, nullptr, false);
         st->s->finish_timings(t0);
     });
 }
 
 int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
                       const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
-                      int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t /*maxgap*/,
+                      int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t maxgap,
                       int64_t* run_offsets, bsg_runs** runs, const bsg_opts* opts) {
+    return bsg_coverage_runs_ss(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, tlen_filter, mapqual, requiredF,
+                                filteredF, tspan, 0, maxgap, run_offsets, runs, opts);
+}
+
+int bsg_coverage_runs_ss(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels, const int32_t* seq_idx,
+                         const int32_t* loc, const int32_t* width, const int8_t* strand, const int32_t* tlen_filter,
+                         int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan, int32_t ss, int32_t /*maxgap*/,
+                         int64_t* run_offsets, bsg_runs** runs, const bsg_opts* opts) {
     if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
     *runs = nullptr;
     return guarded([&] {
@@ -2196,12 +2252,12 @@ int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_lev
         KeepCurrentDevice keep;
         Session s(bampath, R, seq_levels, n_levels, seq_idx, loc, width, strand, opts);
         const int64_t ext = ext_coverage(tlen_filter, tspan);
-        const std::vector<int64_t> dense = s.coverage_layout();
+        const std::vector<int64_t> dense = s.coverage_layout(ss != 0);
         s.start_plan(ext);
         auto res = std::make_unique<bsg_runs>();
         s.use_runs_output(res.get(), run_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
-        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, 0, ext, nullptr, dense.data(), nullptr, false, s.setup_stream()); });
+        s.defer_setup([&] { s.begin_count(MODE_COVERAGE, fp, 1, ss != 0, ext, nullptr, dense.data(), nullptr, false, s.setup_stream()); });
         s.stage(ext, false);
         s.finish_count();
         s.finish_timings(t0);
@@ -2214,6 +2270,11 @@ int bsg_coverage_runs(const char* bampath, int64_t R, const char* const* seq_lev
 
 int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF,
                              int32_t tspan, int64_t* run_offsets, bsg_runs** runs) {
+    return bsg_coverage_runs_ss_staged(st, tlen_filter, mapqual, requiredF, filteredF, tspan, 0, run_offsets, runs);
+}
+
+int bsg_coverage_runs_ss_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF,
+                                int32_t tspan, int32_t ss, int64_t* run_offsets, bsg_runs** runs) {
     if (!runs) { g_err = "runs must not be NULL"; return BSG_EARG; }
     *runs = nullptr;
     if (!st) { g_err = "null stage"; return BSG_EARG; }
@@ -2227,11 +2288,11 @@ int bsg_coverage_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t 
         st->s->require_ext(ext_coverage(tlen_filter, tspan));
         auto res = std::make_unique<bsg_runs>();
         st->s->use_runs_output(res.get(), run_offsets);
-        const std::vector<int64_t> dense = st->s->coverage_layout();
-        st->s->prepare_tiles(MODE_COVERAGE, 1, 0, dense.data());
+        const std::vector<int64_t> dense = st->s->coverage_layout(ss != 0);
+        st->s->prepare_tiles(MODE_COVERAGE, 1, ss != 0, dense.data());
         const FilterParams fp = make_params(tlen_filter, mapqual, 0, requiredF, filteredF, 0, tspan);
-        st->s->decode_resident(MODE_COVERAGE, fp);
-        st->s->count(MODE_COVERAGE, fp, 1, 0, nullptr, dense.data(), nullptr, false);
+        st->s->decode_resident(MODE_COVERAGE, fp, ss != 0);
+        st->s->count(MODE_COVERAGE, fp, 1, ss != 0, nullptr, dense.data(), nullptr, false);
         st->s->finish_timings(t0);
         st->s->use_host_output();
         res->live = true;

@@ -111,9 +111,11 @@ __device__ __forceinline__ bool keep_read(const FilterParams& p, uint32_t fm, in
 // decoded fields while they are still in registers, so a read costs its raw bytes in and 16 bytes out
 // (tid, pos for the join; c0, c1 for the counting kernels) instead of a 20-byte table row written, read again and
 // turned into 8 more bytes by a second kernel.
-template <bool COVERAGE>
-__global__ void __launch_bounds__(kDecThreads) k_decode(DecodeBatch single, const DecodeBatch* __restrict__ table,
-                                                     int n_batches, ReadTable t, FilterParams p, DeviceScalars* sc) {
+// SS (strand-specific coverage, DESIGN.md §12): a reverse read stores ~e in c1, so c1 < 0 marks the strand (e >= pos >= 0
+// for every read that can overlap a region; a kept read with e < 0 overlaps none and is stored dropped).
+template <bool COVERAGE, bool SS>
+__device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBatch* __restrict__ table, int n_batches,
+                                             ReadTable t, const FilterParams& p, DeviceScalars* sc) {
     extern __shared__ __align__(128) uint8_t sm_raw[];
     __shared__ __align__(8) uint64_t bar;
     __shared__ uint32_t s_lo, s_bytes;
@@ -196,6 +198,10 @@ __global__ void __launch_bounds__(kDecThreads) k_decode(DecodeBatch single, cons
             o0 = keep ? s : INT_MAX;
             o1 = keep ? e : INT_MIN;
             if (keep) { hlo = e - d.pos; hhi = d.pos - s; }
+            if (SS) {
+                if (e < 0) o0 = INT_MAX;
+                if (keep && neg) o1 = ~e;
+            }
         }
         const int64_t row = B.row0 + i;
         t.tid[row] = d.tid;
@@ -252,6 +258,17 @@ __global__ void __launch_bounds__(kDecThreads) k_decode(DecodeBatch single, cons
         if (s_hhi > s_ghhi) atomicMax(&sc->halo_hi, s_hhi);
         atomicAdd(&sc->kept[(blockIdx.x & (kKeptSlots - 1)) * kKeptStride], (unsigned long long)kept_cta);
     }
+}
+
+template <bool COVERAGE>
+__global__ void __launch_bounds__(kDecThreads) k_decode(DecodeBatch single, const DecodeBatch* __restrict__ table,
+                                                     int n_batches, ReadTable t, FilterParams p, DeviceScalars* sc) {
+    decode_chunk<COVERAGE, false>(single, table, n_batches, t, p, sc);
+}
+
+__global__ void __launch_bounds__(kDecThreads) k_decode_coverage_ss(DecodeBatch single, const DecodeBatch* __restrict__ table,
+                                                                 int n_batches, ReadTable t, FilterParams p, DeviceScalars* sc) {
+    decode_chunk<true, true>(single, table, n_batches, t, p, sc);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -482,17 +499,28 @@ __global__ void __launch_bounds__(kThreads) k_profile_agg(TileTable tiles, const
 // ---------------------------------------------------------------------------------------------------------------
 // The tile's difference array d[0, len): +1 where a read's interval begins (a start before the tile is clamped into
 // d[0]), -1 behind where it ends (an end past the tile is dropped).  Shared by k_coverage and the run-length kernels.
+// SS (c1 from k_decode_coverage_ss): the tile holds two rows interleaved, d[2j + a], a = read strand XOR region strand
+// (0 sense, 1 antisense), in region orientation like the unstranded array.
+template <bool SS = false>
 __device__ __forceinline__ void scatter_coverage(int32_t* d, int32_t loc, int32_t len, bool neg_region, int64_t lo, int64_t hi,
                                                  const int32_t* __restrict__ c0, const int32_t* __restrict__ c1) {
     const int32_t rend = loc + len;                          // region end, exclusive
     for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
-        const int32_t s = __ldg(c0 + i), e = __ldg(c1 + i);
+        const int32_t s = __ldg(c0 + i);
+        int32_t e = __ldg(c1 + i);
+        int a = 0;
+        if (SS) { a = int(e < 0) ^ int(neg_region); e = e < 0 ? ~e : e; }
         if (s >= rend || e < loc) continue;                  // src/bamsignals.cpp:420 (dropped reads: s = INT_MAX)
         int32_t up, down;
         if (!neg_region) { up = s - loc; down = e + 1 - loc; }          // :423-428
         else { up = rend - 1 - e; down = rend - s; }                    // :431-436
-        atomicAdd(&d[up > 0 ? up : 0], 1);
-        if (down < len) atomicAdd(&d[down], -1);
+        if (SS) {
+            atomicAdd(&d[2 * (up > 0 ? up : 0) + a], 1);
+            if (down < len) atomicAdd(&d[2 * down + a], -1);
+        } else {
+            atomicAdd(&d[up > 0 ? up : 0], 1);
+            if (down < len) atomicAdd(&d[down], -1);
+        }
     }
 }
 
@@ -547,6 +575,68 @@ __global__ void __launch_bounds__(kThreads) k_coverage(TileTable tiles, const in
     for (int q = q_lo + lane; q < q_hi; q += 32) {
         int4 v = s4[q];
         v.x += before; v.y += before; v.z += before; v.w += before;
+        const int j = 4 * q;
+        if (j >= ph && j + 4 <= total) {
+            __stcs(reinterpret_cast<int4*>(dst + j), v);
+        } else {
+            if (j >= ph && j < total) __stcs(dst + j, v.x);
+            if (j + 1 >= ph && j + 1 < total) __stcs(dst + j + 1, v.y);
+            if (j + 2 >= ph && j + 2 < total) __stcs(dst + j + 2, v.z);
+            if (j + 3 >= ph && j + 3 < total) __stcs(dst + j + 3, v.w);
+        }
+    }
+}
+
+// K5 with SS (DESIGN.md §12): the same tile, two rows interleaved as in the output, d[2j + a].  A quad of shared memory is
+// (row r, row r^1, row r, row r^1) with r fixed by the 16-byte phase, so the per-warp scan adds within the quad x -> z and
+// y -> w and carries two running sums (an int2 shuffle scan); the write-out is k_coverage's.
+__global__ void __launch_bounds__(kThreads) k_coverage_ss(TileTable tiles, const int32_t* __restrict__ c0,
+                                                          const int32_t* __restrict__ c1, int32_t* __restrict__ out) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int2 s_warp[kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const bool neg_region = tiles.strand[tix] < 0;
+    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
+    int32_t* const tile_out = out + tiles.out_off[tix];
+    const int ph = out_phase(tile_out);                    // as in k_coverage: d[k] <-> tile_out[k], over 2 len ints
+    int32_t* d = smem + ph;
+    const int total = ph + 2 * len;
+    const int nquads = (total + 3) >> 2;
+    int4* s4 = reinterpret_cast<int4*>(smem);
+    for (int k = threadIdx.x; k < nquads; k += kThreads) s4[k] = make_int4(0, 0, 0, 0);
+    __syncthreads();
+    scatter_coverage<true>(d, loc, len, neg_region, lo, hi, c0, c1);
+    __syncthreads();
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    constexpr int kWarps = kThreads / 32;
+    const int qpw = ((nquads + kWarps - 1) / kWarps + 31) & ~31;
+    const int q_lo = wid * qpw, q_hi = min(nquads, q_lo + qpw);
+    int2 carry = make_int2(0, 0);
+    for (int q0 = q_lo; q0 < q_hi; q0 += 32) {                            // warp-uniform
+        const int q = q0 + lane;
+        int4 v = make_int4(0, 0, 0, 0);
+        if (q < q_hi) v = s4[q];
+        v.z += v.x; v.w += v.y;
+        int2 incl = make_int2(v.z, v.w);
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int ux = __shfl_up_sync(FULL, incl.x, o), uy = __shfl_up_sync(FULL, incl.y, o);
+            if (lane >= o) { incl.x += ux; incl.y += uy; }
+        }
+        const int px = carry.x + incl.x - v.z, py = carry.y + incl.y - v.w;
+        if (q < q_hi) { v.x += px; v.y += py; v.z += px; v.w += py; s4[q] = v; }
+        carry.x += __shfl_sync(FULL, incl.x, 31);
+        carry.y += __shfl_sync(FULL, incl.y, 31);
+    }
+    if (lane == 0) s_warp[wid] = carry;
+    __syncthreads();
+    int bx = 0, by = 0;
+    for (int k = 0; k < wid; ++k) { bx += s_warp[k].x; by += s_warp[k].y; }
+    int32_t* dst = tile_out - ph;
+    for (int q = q_lo + lane; q < q_hi; q += 32) {
+        int4 v = s4[q];
+        v.x += bx; v.y += by; v.z += bx; v.w += by;
         const int j = 4 * q;
         if (j >= ph && j + 4 <= total) {
             __stcs(reinterpret_cast<int4*>(dst + j), v);
@@ -729,6 +819,140 @@ __global__ void __launch_bounds__(kThreads) k_runs_write(TileTable tiles, int64_
         cnt += __shfl_sync(FULL, icnt, 31);
     }
     if (tail && threadIdx.x == 0 && kend > kbeg) atomicAdd(&lengths[kend - 1], rel + len);     // the region's last run ends at its width
+}
+
+// K5r with SS (DESIGN.md §12): the interleaved array of k_coverage_ss, at smem[0].  Row a of a tile is a virtual tile of
+// list 2i + a, vt[a * n_tiles + t] = v, as for strand-specific profile runs (K4r below); k_runs_scan runs unchanged over
+// the 2 * n_tiles virtual tiles and 2R lists.
+__global__ void __launch_bounds__(kThreads) k_runs_count_ss(TileTable tiles, int64_t n_tiles, const int32_t* __restrict__ c0,
+                                                            const int32_t* __restrict__ c1, RunTiles rt,
+                                                            const int32_t* __restrict__ vt) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int32_t s_nz[2][kThreads / 32], s_sum[2][kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    for (int k = threadIdx.x; k < 2 * len; k += kThreads) smem[k] = 0;
+    __syncthreads();
+    scatter_coverage<true>(smem, loc, len, tiles.strand[tix] < 0, tiles.cand_lo[tix], tiles.cand_hi[tix], c0, c1);
+    __syncthreads();
+    // element k = 2j + a: kThreads is even, so a thread only ever sees row a = threadIdx.x & 1
+    int nz = 0, sum = 0;
+    for (int k = threadIdx.x; k < 2 * len; k += kThreads) {
+        const int32_t v = smem[k];
+        sum += v;
+        nz += int(k >= 2 && v != 0);
+    }
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+        const bool mine = int(threadIdx.x & 1) == a;
+        const int n = __reduce_add_sync(FULL, mine ? nz : 0), t = __reduce_add_sync(FULL, mine ? sum : 0);
+        if (lane == 0) { s_nz[a][wid] = n; s_sum[a][wid] = t; }
+    }
+    __syncthreads();
+    if (threadIdx.x < 2) {
+        const int a = threadIdx.x;
+        int tn = 0, ts = 0;
+        for (int k = 0; k < kThreads / 32; ++k) { tn += s_nz[a][k]; ts += s_sum[a][k]; }
+        const int32_t v = vt[a * n_tiles + tix];
+        rt.nnz[v] = tn;
+        rt.first[v] = smem[a];
+        rt.last[v] = ts;
+    }
+}
+
+// k_runs_write per row: a quad of shared memory holds bases 2q and 2q + 1 of both rows, (s, a, s, a).
+__global__ void __launch_bounds__(kThreads) k_runs_write_ss(TileTable tiles, int64_t n_tiles, const int32_t* __restrict__ c0,
+                                                            const int32_t* __restrict__ c1, RunTiles rt,
+                                                            const int32_t* __restrict__ vt, const int64_t* __restrict__ run_off,
+                                                            int32_t* __restrict__ lengths, int32_t* __restrict__ values) {
+    extern __shared__ __align__(16) int32_t smem[];
+    __shared__ int2 s_sum[kThreads / 32], s_cnt[kThreads / 32];
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const int64_t n_virtual = 2 * n_tiles;
+    int32_t rel[2];
+    int64_t kbeg[2], k0[2];
+    bool start0[2];
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+        const int64_t v = vt[a * n_tiles + tix];
+        const int32_t list = rt.region[v];
+        rel[a] = rt.rel[v];
+        start0[a] = v == 0 || rt.region[v - 1] != list || rt.first[v] != rt.last[v - 1];    // a run starts at base 0
+        kbeg[a] = run_off[list];
+        k0[a] = kbeg[a] + (rt.toff[v] - rt.rfirst[list]);                                 // the row's first run start
+    }
+    const int nquads = (len + 1) >> 1;
+    int4* s4 = reinterpret_cast<int4*>(smem);
+    for (int k = threadIdx.x; k < nquads; k += kThreads) s4[k] = make_int4(0, 0, 0, 0);
+    __syncthreads();
+    scatter_coverage<true>(smem, loc, len, tiles.strand[tix] < 0, tiles.cand_lo[tix], tiles.cand_hi[tix], c0, c1);
+    __syncthreads();
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    constexpr int kWarps = kThreads / 32;
+    const int qpw = ((nquads + kWarps - 1) / kWarps + 31) & ~31;
+    const int q_lo = wid * qpw, q_hi = min(nquads, q_lo + qpw);
+    auto flags = [&](int q, int d0, int d1, int a) {        // bit e: row a has a run start at base 2q + e
+        const int j = 2 * q;
+        return (j < len && (j == 0 ? start0[a] : d0 != 0) ? 1u : 0u) | (j + 1 < len && d1 != 0 ? 2u : 0u);
+    };
+    int2 wsum = make_int2(0, 0), wcnt = make_int2(0, 0);
+    for (int q0 = q_lo; q0 < q_hi; q0 += 32) {
+        const int q = q0 + lane;
+        int4 v = make_int4(0, 0, 0, 0);
+        if (q < q_hi) v = s4[q];
+        wsum.x += __reduce_add_sync(FULL, v.x + v.z);
+        wsum.y += __reduce_add_sync(FULL, v.y + v.w);
+        wcnt.x += __reduce_add_sync(FULL, q < q_hi ? __popc(flags(q, v.x, v.z, 0)) : 0);
+        wcnt.y += __reduce_add_sync(FULL, q < q_hi ? __popc(flags(q, v.y, v.w, 1)) : 0);
+    }
+    if (lane == 0) { s_sum[wid] = wsum; s_cnt[wid] = wcnt; }
+    __syncthreads();
+    int val[2] = {0, 0}, cnt[2] = {0, 0};
+    for (int k = 0; k < wid; ++k) { val[0] += s_sum[k].x; val[1] += s_sum[k].y; cnt[0] += s_cnt[k].x; cnt[1] += s_cnt[k].y; }
+    for (int q0 = q_lo; q0 < q_hi; q0 += 32) {
+        const int q = q0 + lane;
+        int4 v = make_int4(0, 0, 0, 0);
+        if (q < q_hi) v = s4[q];
+        const int d[2][2] = {{v.x, v.z}, {v.y, v.w}};
+#pragma unroll
+        for (int a = 0; a < 2; ++a) {
+            const unsigned f = q < q_hi ? flags(q, d[a][0], d[a][1], a) : 0u;
+            int isum = d[a][0] + d[a][1], icnt = __popc(f);
+            const int qs = isum, qc = icnt;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int us = __shfl_up_sync(FULL, isum, o), uc = __shfl_up_sync(FULL, icnt, o);
+                if (lane >= o) { isum += us; icnt += uc; }
+            }
+            int x = val[a] + isum - qs;                     // the row's coverage just before base 2q
+            int64_t k = k0[a] + cnt[a] + icnt - qc;         // index of the row's next run start
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                x += d[a][e];
+                if (f >> e & 1u) {
+                    const int32_t p = rel[a] + 2 * q + e;   // run start, relative to the region in its orientation
+                    values[k] = x;
+                    atomicAdd(&lengths[k], -p);
+                    if (k > kbeg[a]) atomicAdd(&lengths[k - 1], p);
+                    ++k;
+                }
+            }
+            val[a] += __shfl_sync(FULL, isum, 31);
+            cnt[a] += __shfl_sync(FULL, icnt, 31);
+        }
+    }
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int a = 0; a < 2; ++a) {
+            const int64_t v = vt[a * n_tiles + tix];
+            const int32_t list = rt.region[v];
+            const int64_t kend = run_off[list + 1];
+            const bool tail = v + 1 == n_virtual || rt.region[v + 1] != list;
+            if (tail && kend > kbeg[a]) atomicAdd(&lengths[kend - 1], rel[a] + len);   // the row's last run ends at the width
+        }
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -920,20 +1144,23 @@ void with_profile_kind(int ss, int32_t binsize, F&& f) {
 
 }  // namespace
 
-void launch_decode(const DecodeBatch& one, ReadTable t, bool coverage, const FilterParams& p, DeviceScalars* sc, cudaStream_t s) {
+void launch_decode(const DecodeBatch& one, ReadTable t, bool coverage, bool ss, const FilterParams& p, DeviceScalars* sc, cudaStream_t s) {
     if (one.n <= 0) return;
     const int grid = (one.n + kDecThreads - 1) / kDecThreads;
     DecodeBatch b = one;
     b.chunk0 = 0;
-    if (coverage) k_decode<true><<<unsigned(grid), kDecThreads, kSpanCap + 32, s>>>(b, nullptr, 1, t, p, sc);
+    if (coverage && ss) k_decode_coverage_ss<<<unsigned(grid), kDecThreads, kSpanCap + 32, s>>>(b, nullptr, 1, t, p, sc);
+    else if (coverage) k_decode<true><<<unsigned(grid), kDecThreads, kSpanCap + 32, s>>>(b, nullptr, 1, t, p, sc);
     else k_decode<false><<<unsigned(grid), kDecThreads, kSpanCap + 32, s>>>(b, nullptr, 1, t, p, sc);
 }
 
-void launch_decode_table(const DecodeBatch* d_table, int n_batches, int total_chunks, ReadTable t, bool coverage,
+void launch_decode_table(const DecodeBatch* d_table, int n_batches, int total_chunks, ReadTable t, bool coverage, bool ss,
                          const FilterParams& p, DeviceScalars* sc, cudaStream_t s) {
     if (n_batches <= 0 || total_chunks <= 0) return;
-    if (coverage) k_decode<true><<<unsigned(total_chunks), kDecThreads, kSpanCap + 32, s>>>(DecodeBatch{}, d_table, n_batches, t, p, sc);
-    else k_decode<false><<<unsigned(total_chunks), kDecThreads, kSpanCap + 32, s>>>(DecodeBatch{}, d_table, n_batches, t, p, sc);
+    const unsigned grid = unsigned(total_chunks);
+    if (coverage && ss) k_decode_coverage_ss<<<grid, kDecThreads, kSpanCap + 32, s>>>(DecodeBatch{}, d_table, n_batches, t, p, sc);
+    else if (coverage) k_decode<true><<<grid, kDecThreads, kSpanCap + 32, s>>>(DecodeBatch{}, d_table, n_batches, t, p, sc);
+    else k_decode<false><<<grid, kDecThreads, kSpanCap + 32, s>>>(DecodeBatch{}, d_table, n_batches, t, p, sc);
 }
 
 void launch_join(ReadTable t, int64_t n, TileTable tiles, int64_t n_tiles, const DeviceScalars* sc, cudaStream_t s) {
@@ -969,24 +1196,31 @@ void launch_profile(TileTable tiles, int64_t n_tiles, const int32_t* c0, const i
 #undef BSG_LAUNCH_PROFILE
 }
 
-void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
+void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
                      int32_t* out, DeviceScalars*, cudaStream_t s) {
     if (n_tiles <= 0) return;
     const size_t smem = size_t(max_tile_ints + 8) * sizeof(int32_t);
-    k_coverage<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, c0, c1, out);
+    if (ss) k_coverage_ss<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, c0, c1, out);
+    else k_coverage<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, c0, c1, out);
 }
 
-void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints, RunTiles rt,
-                          int64_t R, int64_t* run_off, cudaStream_t s) {
-    if (n_tiles > 0) k_runs_count<<<unsigned(n_tiles), kThreads, size_t(max_tile_ints) * sizeof(int32_t), s>>>(tiles, c0, c1, rt);
-    k_runs_scan<<<1, kScanThreads, 0, s>>>(rt, n_tiles, R, run_off);
+void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
+                          RunTiles rt, const int32_t* vt, int64_t lists, int64_t* run_off, cudaStream_t s) {
+    const size_t smem = size_t(max_tile_ints) * sizeof(int32_t);
+    if (n_tiles > 0) {
+        if (ss) k_runs_count_ss<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, vt);
+        else k_runs_count<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, c0, c1, rt);
+    }
+    k_runs_scan<<<1, kScanThreads, 0, s>>>(rt, (ss ? 2 : 1) * n_tiles, lists, run_off);
 }
 
-void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
-                                RunTiles rt, const int64_t* run_off, int32_t* lengths, int32_t* values, cudaStream_t s) {
+void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
+                                RunTiles rt, const int32_t* vt, const int64_t* run_off, int32_t* lengths, int32_t* values,
+                                cudaStream_t s) {
     if (n_tiles <= 0) return;
     const size_t smem = size_t(max_tile_ints + 4) * sizeof(int32_t);
-    k_runs_write<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, run_off, lengths, values);
+    if (ss) k_runs_write_ss<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, vt, run_off, lengths, values);
+    else k_runs_write<<<unsigned(n_tiles), kThreads, smem, s>>>(tiles, n_tiles, c0, c1, rt, run_off, lengths, values);
 }
 
 void launch_profile_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,

@@ -5,7 +5,8 @@
 //                  uint32 offs[n+1]     byte offset of every record's block_size field; offs[n] = end of last record
 //   read table     int32  tid[N] pos[N]  (8 B / read) the join key: rows are in file order = sorted by (tid, pos)
 //                  int32  c0[N] c1[N]    (8 B / read) pileup: c0 = 5'/midpoint coordinate, c1 = 0 '+', 1 '-', -1 dropped
-//                                       coverage: [c0,c1] = inclusive interval, dropped reads get c0 > c1 sentinels
+//                                       coverage: [c0,c1] = inclusive interval, dropped reads get c0 > c1 sentinels;
+//                                       strand-specific coverage: c1 = ~end for reverse reads, dropped reads c0 = INT_MAX
 //                                       (end, tlen, flag and mapq never leave the decode kernel's registers)
 //   tiles          int32  rid loc len strand, int64 out_off, int64 cand_lo cand_hi   one row per region tile
 //   result         int32  out[]         flat, bsg_output_layout() order; every element written exactly once
@@ -73,8 +74,9 @@ constexpr int kDecodeChunk = BSG_DECODE_THREADS;     // records per K1 CTA (one 
 // extraction, bam_endpos (src/bamsignals.cpp:16-18) and setRead (:326-346 pileup, :392-415 coverage).
 // launch_decode: one batch (streaming path); launch_decode_table: every resident batch of a staged session in ONE
 // launch (d_table lives in device memory).
-void launch_decode(const DecodeBatch& one, ReadTable t, bool coverage, const FilterParams& p, DeviceScalars* sc, cudaStream_t s);
-void launch_decode_table(const DecodeBatch* d_table, int n_batches, int total_chunks, ReadTable t, bool coverage,
+// ss (coverage only): strand-specific coverage, reverse reads store ~c1 (DESIGN.md §12).
+void launch_decode(const DecodeBatch& one, ReadTable t, bool coverage, bool ss, const FilterParams& p, DeviceScalars* sc, cudaStream_t s);
+void launch_decode_table(const DecodeBatch* d_table, int n_batches, int total_chunks, ReadTable t, bool coverage, bool ss,
                          const FilterParams& p, DeviceScalars* sc, cudaStream_t s);
 
 // K0 (gpu_inflate): one BGZF block = one raw-DEFLATE stream of at most 64 KiB.
@@ -128,8 +130,9 @@ void launch_count(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int
 // K4: bamProfile (shared-memory bin histogram per tile; Pileupper::pileup, :349-363)
 void launch_profile(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int32_t binsize,
                     int max_tile_ints, int32_t* out, DeviceScalars* sc, cudaStream_t s);
-// K5: bamCoverage (shared-memory difference array + block scan; Coverager::pileup + cumsum, :418-438, :464-470)
-void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
+// K5: bamCoverage (shared-memory difference array + block scan; Coverager::pileup + cumsum, :418-438, :464-470);
+// ss: sense and antisense rows interleaved like a binsize-1 strand-specific profile (DESIGN.md §12)
+void launch_coverage(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
                      int32_t* out, DeviceScalars* sc, cudaStream_t s);
 
 // K5r: bamCoverage as runs (DESIGN.md §10).  Per-tile arrays in tile order; region / rel come from the host, the rest is
@@ -145,12 +148,14 @@ struct RunTiles {
     int64_t* rfirst;
     int64_t* rlast;
 };
-// count pass + scans: run_off[0..R] (device) = every region's span of runs in the caller's region order
-void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints, RunTiles rt,
-                          int64_t R, int64_t* run_off, cudaStream_t s);
-// write pass: values[k] and lengths[k] for k in [0, run_off[R]); lengths must be zero before the launch
-void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int max_tile_ints,
-                                RunTiles rt, const int64_t* run_off, int32_t* lengths, int32_t* values, cudaStream_t s);
+// With ss, rt, vt and the lists are those of a strand-specific profile (K4r below): row a of region i is list 2i + a.
+// count pass + scans: run_off[0..lists] (device) = every list's span of runs in the caller's region order
+void launch_coverage_runs(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
+                          RunTiles rt, const int32_t* vt, int64_t lists, int64_t* run_off, cudaStream_t s);
+// write pass: values[k] and lengths[k] for k in [0, run_off[lists]); lengths must be zero before the launch
+void launch_coverage_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* c0, const int32_t* c1, int ss, int max_tile_ints,
+                                RunTiles rt, const int32_t* vt, const int64_t* run_off, int32_t* lengths, int32_t* values,
+                                cudaStream_t s);
 
 // K4r: bamProfile as runs (DESIGN.md §11), over VIRTUAL tiles: row a (sense / antisense with ss) of the j-th of region
 // i's n_i tiles, T_i its first tile, is virtual tile v = mult * T_i + a * n_i + j in list mult * i + a (mult = ss ? 2 : 1).

@@ -89,14 +89,13 @@ void make_tiles(const Regions& rg, Mode mode, int32_t binsize, int ss, const int
         if (mode == MODE_COUNT) { push(rg.rid[i], loc, width, strand, base, mult); continue; }
         if (width == 0) continue;
         const int64_t bs = mode == MODE_COVERAGE ? 1 : binsize;
-        const int64_t m = mode == MODE_COVERAGE ? 1 : mult;
         const int64_t nb = (width + bs - 1) / bs;
-        const int64_t tb = std::max<int64_t>(1, tile_ints / m);             // bins per tile
+        const int64_t tb = std::max<int64_t>(1, tile_ints / mult);          // bins per tile
         for (int64_t k = 0; k * tb < nb; ++k) {
             const int64_t rel_lo = k * tb * bs, rel_hi = std::min(width, (k + 1) * tb * bs);
             const int64_t tloc = strand < 0 ? loc + width - rel_hi : loc + rel_lo;
             const int64_t bins = (rel_hi - rel_lo + bs - 1) / bs;
-            push(rg.rid[i], tloc, rel_hi - rel_lo, strand, base + m * k * tb, m * bins);
+            push(rg.rid[i], tloc, rel_hi - rel_lo, strand, base + mult * k * tb, mult * bins);
         }
     }
 }

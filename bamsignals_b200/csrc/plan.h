@@ -36,7 +36,8 @@ void resolve_regions(const BamFile& bam, int64_t R, const char* const* seq_level
 
 // Cut regions into tiles of at most tile_ints output ints.  A profile tile is a bin-aligned sub-interval counted from
 // the region's 5' end (loc for +/*, end for -, because of src/bamsignals.cpp:357); a coverage tile is any
-// sub-interval (the clamp at :424/:432 makes its prefix sum self-contained); bamCount regions are never cut.
+// sub-interval (the clamp at :424/:432 makes its prefix sum self-contained); bamCount regions are never cut.  With ss a
+// bin (a base for coverage) owns two output ints, sense and antisense.
 void make_tiles(const Regions& rg, Mode mode, int32_t binsize, int ss, const int64_t* out_offsets, int tile_ints,
                 HostTiles* tiles);
 

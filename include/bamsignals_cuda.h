@@ -248,6 +248,46 @@ int bsg_profile_runs_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t m
                             int32_t ss, int32_t requiredF, int32_t filteredF, int32_t pe_mid,
                             int64_t* run_offsets, bsg_runs** runs);
 
+/* ---- strand-specific bamCoverage: sense and antisense coverage in one pass ---------------------------------------------
+ * Each call takes the arguments of its counterpart without _ss, with `ss` inserted right after tspan (nonzero = on).
+ * With ss == 0 it is its counterpart, exactly.  With ss:
+ *   Strand   a read's strand is its own flag bit 0x10.  Sense and antisense are relative to the region, as for
+ *            bsg_pileup: on '+' and '*' regions forward reads are sense; on '-' regions reverse reads are sense and both
+ *            rows are mirrored, as unstranded coverage of a '-' region is.  With tspan (paired_end = "extend",
+ *            requiredF 66) only first mates count, and the whole fragment goes to the first mate's strand.
+ *   Layout   bsg_output_layout(R, width, 1, 1, offsets): region i is 2 x width[i] int32, interleaved
+ *            [sense_0, antisense_0, sense_1, ...] in region orientation (R's IntegerMatrix(2, w)); a zero-width region is
+ *            empty.  Runs: 2R lists as for bsg_profile_runs with ss, list 2i the sense and list 2i+1 the antisense row of
+ *            region i, run_offsets of 2R + 1 int64.
+ *   Identity with cov(F) = bsg_coverage with requiredF = F and every other argument the same: on '+' and '*' regions
+ *            antisense = cov(requiredF | 16) and sense = cov(requiredF) - cov(requiredF | 16); on '-' regions sense =
+ *            cov(requiredF | 16) and antisense = cov(requiredF) - cov(requiredF | 16).  So sense + antisense = cov(requiredF).
+ *   BSG_EARG before any work, besides the counterpart's refusals: an out_offsets that is not the stranded layout, and a
+ *            region that starts before position 1.  Multi-device calls (opts->n_devices > 1) exist for bsg_coverage_ss
+ *            only, as for the counterparts. */
+int bsg_coverage_ss(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                    const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                    const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
+                    int32_t ss, int32_t maxgap, int32_t* out, const int64_t* out_offsets, int32_t* const* out_ptrs,
+                    const bsg_opts* opts);
+int bsg_coverage_ss_device(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                           const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                           const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
+                           int32_t ss, int32_t maxgap, int32_t* d_out, const int64_t* out_offsets, void* stream,
+                           const bsg_opts* opts);
+int bsg_coverage_ss_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                           int32_t filteredF, int32_t tspan, int32_t ss, int32_t* out, const int64_t* out_offsets);
+int bsg_coverage_ss_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                                  int32_t filteredF, int32_t tspan, int32_t ss, int32_t* d_out, const int64_t* out_offsets,
+                                  void* stream);
+int bsg_coverage_runs_ss(const char* bampath, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                         const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand,
+                         const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF, int32_t filteredF, int32_t tspan,
+                         int32_t ss, int32_t maxgap, int64_t* run_offsets /* (ss ? 2R : R) + 1 */, bsg_runs** runs,
+                         const bsg_opts* opts);
+int bsg_coverage_runs_ss_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual, int32_t requiredF,
+                                int32_t filteredF, int32_t tspan, int32_t ss, int64_t* run_offsets, bsg_runs** runs);
+
 /*
  * writeSamAsBamAndIndex (src/bamsignals.cpp:496-534, .Call symbol bamsignals_writeSamAsBamAndIndex,
  * src/bamsignals_init.c:17): SAM text -> <bampath> (BGZF/BAM) + <bampath>.bai.  Host-only (no device needed).  The

@@ -367,7 +367,8 @@ class BsgOpts(C.Structure):
     _fields_ = [("struct_size", C.c_int32), ("n_devices", C.c_int32), ("devices", C.c_int32 * 16),
                 ("inflate_threads", C.c_int32), ("batch_bytes", C.c_int64), ("verify_crc", C.c_int32),
                 ("use_cache", C.c_int32), ("gpu_inflate", C.c_int32), ("stream_min_ints", C.c_int32),
-                ("result_pack", C.c_int32), ("walk_scheme", C.c_int32), ("reserved", C.c_int32 * 5)]
+                ("result_pack", C.c_int32), ("walk_scheme", C.c_int32),
+                ("resident_scheme", C.c_int32), ("reserved", C.c_int32 * 4)]
 
 
 class BsgTimings(C.Structure):

@@ -73,6 +73,10 @@ constexpr int64_t kD2HChunk = 32ll << 20;       // bytes per pinned result-stagi
 constexpr int64_t kPackMinInts = 1ll << 16;     // result portions from this size on cross PCIe as bytes (opts.result_pack)
 constexpr int kOutSlots = 3;                    // pinned result-staging ring
 constexpr int kUp = 4;                          // GPU-inflate path: upload ring (compressed bytes + descriptors); raw buffers: 2
+// Staged pileup calls take the fused step when its join would examine at most this share of the resident rows
+// (opts.resident_scheme 0).  Placed from tools/resident_ab.py's sweep on one B200 (profiles/resident_ab_c2_sweep.jsonl):
+// the fused step is 1.62x / 1.27x / 0.98x / 0.99x the table step at shares 0.13 / 0.23 / 0.34 / 0.43.
+constexpr double kFusedShare = 0.3;
 
 struct DevBuf {
     void* p = nullptr;
@@ -598,6 +602,7 @@ public:
     // Staged sessions: decode + filter every resident raw batch again (K1) in ONE launch, timed.
     void decode_resident(Mode mode, const FilterParams& fp, int ss = 0) {
         DeviceCtx& c = *ctx_;
+        fused_ = false;
         BSG_CUDA(cudaMemsetAsync(c.scalars.p, 0, sizeof(DeviceScalars), c.s_comp));
         if (resident_.empty()) return;
         Span sp{c.timing_event(), c.timing_event()};
@@ -645,10 +650,11 @@ public:
         if (setup_thread_.joinable()) setup_thread_.join();
         stop_streamer(true);
         wait_prefault();
-        if (raw_all_.p || offs_all_.p || batch_table_.p) {
+        if (raw_all_.p || offs_all_.p || batch_table_.p || idx_keys_.p || idx_scal_.p) {
             cudaSetDevice(ctx_->dev);
             cudaDeviceSynchronize();
             raw_all_.release(); offs_all_.release(); batch_table_.release();
+            idx_keys_.release(); idx_long_key_.release(); idx_long_row_.release(); idx_scal_.release(); fused_rng_.release();
         }
     }
 
@@ -803,10 +809,11 @@ public:
         tm_.bytes_d2h = os_bytes_ + scalar_bytes;
         cnt_.active = false;
         const DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
-        check_status(hs->status);
+        check_status(hs->status | (keep_raw_ ? idx_.status : 0u));     // staged: the resident records' bits, every call
         tm_.records = n_rows_;
         tm_.records_kept = 0;
         for (int k = 0; k < kKeptSlots; ++k) tm_.records_kept += int64_t(hs->kept[k * kKeptStride]);
+        if (fused_) tm_.records_kept = -1;                              // only the examined rows were filtered
         tm_.candidates = int64_t(hs->candidates);
     }
 
@@ -873,13 +880,12 @@ private:
         Nvtx r("bsg:join+count");
         DeviceCtx& c = *ctx_;
         cudaStream_t st = cnt_stream();
-        const int64_t nt_all = n_tiles_, n = t1 - t0;
-        int32_t* ti = c.tiles_i32.as<int32_t>();
-        int64_t* tl = c.tiles_i64.as<int64_t>();
-        TileTable tt{ti + t0, ti + nt_all + t0, ti + 2 * nt_all + t0, ti + 3 * nt_all + t0, tl + t0, tl + nt_all + t0, tl + 2 * nt_all + t0};
+        const int64_t n = t1 - t0;
+        const TileTable tt = tile_table(t0);
         DeviceScalars* sc = c.scalars.as<DeviceScalars>();
         int32_t* c0 = c.c0.as<int32_t>();
         int32_t* c1 = c.c1.as<int32_t>();
+        if (fused_) { count_tiles_fused(tt, t0, t1, st); return; }
         {
             Span sp{c.timing_event(), c.timing_event()};
             BSG_CUDA(cudaEventRecord(sp.a, st));
@@ -899,6 +905,40 @@ private:
             kt_.count.push_back(sp); kt_.launches += 1;
             if (cnt_.want_output) ship_tiles(t0, t1, sp.b);
         }
+        cnt_.t_done = t1;
+    }
+
+    // the device tile table from tile t0 on
+    TileTable tile_table(int64_t t0) const {
+        const int64_t nt = n_tiles_;
+        int32_t* ti = ctx_->tiles_i32.as<int32_t>();
+        int64_t* tl = ctx_->tiles_i64.as<int64_t>();
+        return TileTable{ti + t0, ti + nt + t0, ti + 2 * nt + t0, ti + 3 * nt + t0, tl + t0, tl + nt + t0, tl + 2 * nt + t0};
+    }
+
+    // K3f + K4f (staged pileup calls, DESIGN.md §13): the tiles' row ranges from the resident index, then the counts
+    // straight from the raw records.
+    void count_tiles_fused(const TileTable& tt, int64_t t0, int64_t t1, cudaStream_t st) {
+        DeviceCtx& c = *ctx_;
+        const int64_t n = t1 - t0;
+        fused_rng_.ensure(size_t(2 * n_tiles_) * sizeof(int64_t) + 64);
+        int64_t* llo = fused_rng_.as<int64_t>() + t0;
+        int64_t* lhi = fused_rng_.as<int64_t>() + n_tiles_ + t0;
+        const ResidentView v = resident_view();
+        {
+            Span sp{c.timing_event(), c.timing_event()};
+            BSG_CUDA(cudaEventRecord(sp.a, st));
+            launch_join_fused(v, tt, llo, lhi, n, fused_h_, c.scalars.as<DeviceScalars>(), st);
+            BSG_CUDA(cudaEventRecord(sp.b, st));
+            kt_.join.push_back(sp); kt_.launches += 1;
+        }
+        if (dev_out_.on) BSG_CUDA(cudaStreamWaitEvent(st, c.ev_caller, 0));
+        Span sp{c.timing_event(), c.timing_event()};
+        BSG_CUDA(cudaEventRecord(sp.a, st));
+        launch_pileup_fused(v, tt, llo, lhi, n, cnt_.ss, cnt_.mode == MODE_COUNT ? 0 : cnt_.binsize, max_tile_ints_, cnt_.fp, cnt_.dst, st);
+        BSG_CUDA(cudaEventRecord(sp.b, st));
+        kt_.count.push_back(sp); kt_.launches += 1;
+        if (cnt_.want_output) ship_tiles(t0, t1, sp.b);
         cnt_.t_done = t1;
     }
 
@@ -1675,7 +1715,161 @@ private:
         batch_table_.ensure(tab.size() * sizeof(DecodeBatch) + 64);
         if (!tab.empty()) BSG_CUDA(cudaMemcpy(batch_table_.p, tab.data(), tab.size() * sizeof(DecodeBatch), cudaMemcpyHostToDevice));
         BSG_CUDA(cudaStreamSynchronize(c.s_comp));
+        build_resident_index(row0);
     }
+
+    // The record index of the fused pileup step (DESIGN.md §13), built once per staged session by two passes of K0i
+    // over every resident record (the open call's ms_decode):
+    //   pass 0: a key per 32 rows, the unsorted / corrupt status bits, reach = max(pos + span) and
+    //           the span buckets;
+    //   host:   the long-span threshold T = 2^k - 1 for the smallest k >= 6 that leaves at most 1/64 of the rows with
+    //           span > T (C2: reads ~100 bp, 1 % spliced with a 100-10,000 bp N => T = 127, the spliced reads are long);
+    //   pass 1: the long list (rows with span > T), sorted by key on the host.
+    // The status bits do not fail the open: every staged call raises them, as K1 does on the table path.
+    void build_resident_index(int64_t n_rows) {
+        DeviceCtx& c = *ctx_;
+        idx_ = ResidentIndexHost();
+        const int nb = int(resident_.size());
+        if (n_rows <= 0 || nb == 0) return;
+        idx_.n = n_rows;
+        const int64_t n_keys = (n_rows + kIndexStride - 1) / kIndexStride;
+        idx_keys_.ensure(size_t(n_keys) * sizeof(uint64_t));
+        idx_scal_.ensure(sizeof(IndexScalars));
+        IndexScalars* isc = idx_scal_.as<IndexScalars>();
+        cudaStream_t st = c.s_comp;
+        Span sp0{c.timing_event(), c.timing_event()};
+        BSG_CUDA(cudaMemsetAsync(isc, 0, sizeof(IndexScalars), st));
+        BSG_CUDA(cudaEventRecord(sp0.a, st));
+        launch_resident_index(batch_table_.as<DecodeBatch>(), nb, resident_chunks_, 0, 0, idx_keys_.as<unsigned long long>(), nullptr,
+                              nullptr, isc, st);
+        BSG_CUDA(cudaEventRecord(sp0.b, st));
+        kt_.decode.push_back(sp0); kt_.launches += 1;
+        IndexScalars hs;
+        BSG_CUDA(cudaMemcpyAsync(&hs, isc, sizeof hs, cudaMemcpyDeviceToHost, st));
+        BSG_CUDA(cudaStreamSynchronize(st));
+        idx_.n_keys = n_keys;
+        idx_.status = hs.status;
+        idx_.reach = int64_t(hs.reach);
+        int k = 6;
+        for (; k < kSpanBuckets; ++k) {
+            uint64_t above = 0;
+            for (int b = k; b < kSpanBuckets; ++b) above += hs.bucket_n[b];
+            if (above * 64 <= uint64_t(n_rows)) break;
+        }
+        idx_.long_span = k < kSpanBuckets ? (1u << k) - 1u : ~0u;
+        uint64_t n_long = 0;
+        for (int b = 0; b < kSpanBuckets; ++b) {
+            if (b < k) idx_.short_max = std::max(idx_.short_max, int64_t(hs.bucket_max[b]));
+            else { idx_.long_max = std::max(idx_.long_max, int64_t(hs.bucket_max[b])); n_long += hs.bucket_n[b]; }
+        }
+        if (n_long) {
+            idx_long_key_.ensure(size_t(n_long) * sizeof(uint64_t));
+            idx_long_row_.ensure(size_t(n_long) * sizeof(int2));
+            Span sp1{c.timing_event(), c.timing_event()};
+            BSG_CUDA(cudaMemsetAsync(&isc->n_long, 0, sizeof(uint32_t), st));
+            BSG_CUDA(cudaEventRecord(sp1.a, st));
+            launch_resident_index(batch_table_.as<DecodeBatch>(), nb, resident_chunks_, 1, idx_.long_span, nullptr,
+                                  idx_long_key_.as<unsigned long long>(), idx_long_row_.as<int2>(), isc, st);
+            BSG_CUDA(cudaEventRecord(sp1.b, st));
+            kt_.decode.push_back(sp1); kt_.launches += 1;
+            std::vector<uint64_t> lk(n_long);
+            std::vector<int2> lr(n_long);
+            BSG_CUDA(cudaMemcpyAsync(lk.data(), idx_long_key_.p, n_long * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            BSG_CUDA(cudaMemcpyAsync(lr.data(), idx_long_row_.p, n_long * sizeof(int2), cudaMemcpyDeviceToHost, st));
+            BSG_CUDA(cudaStreamSynchronize(st));
+            // pass 1 appends in CTA completion order: sort into row order (key, then batch and record for equal keys)
+            std::vector<uint32_t> ord(n_long);
+            for (uint32_t j = 0; j < uint32_t(n_long); ++j) ord[j] = j;
+            std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) {
+                if (lk[a] != lk[b]) return lk[a] < lk[b];
+                return lr[a].x != lr[b].x ? lr[a].x < lr[b].x : lr[a].y < lr[b].y;
+            });
+            std::vector<uint64_t> keys(n_long);
+            std::vector<int2> rows(n_long);
+            for (size_t j = 0; j < n_long; ++j) { keys[j] = lk[ord[j]]; rows[j] = lr[ord[j]]; }
+            idx_.n_long = int64_t(n_long);
+            BSG_CUDA(cudaMemcpy(idx_long_key_.p, keys.data(), n_long * sizeof(uint64_t), cudaMemcpyHostToDevice));
+            BSG_CUDA(cudaMemcpy(idx_long_row_.p, rows.data(), n_long * sizeof(int2), cudaMemcpyHostToDevice));
+        }
+    }
+
+    ResidentView resident_view() const {
+        return ResidentView{batch_table_.as<DecodeBatch>(), int(resident_.size()), idx_.n, idx_keys_.as<unsigned long long>(),
+                            idx_.n_keys, idx_long_key_.as<unsigned long long>(), idx_long_row_.as<int2>(), idx_.n_long, idx_.long_span};
+    }
+
+    // Key ranges around a tile that hold every read the call can count there, in int64 from the session's spans and the
+    // call's shift / midpoint / tlen bound.  A read's pileup coordinate is pos + D, D = offset (forward) or
+    // span - 1 - offset (reverse), offset = shift or |tlen| / 2 + shift; a kept read has tmin <= |tlen| <= tmax, where
+    // |tlen| is >= 0 or INT_MIN (abs() leaves INT_MIN negative).  If a coordinate could wrap around int32 (K1 computes it
+    // in int32), the ranges are the whole contig.  The kernels' exact per-read test decides what counts.
+    FusedHalos fused_halos(const FilterParams& p) const {
+        int64_t omin = p.shift, omax = p.shift;
+        if (p.midpoint) {
+            int64_t amin = INT32_MIN, amax = INT32_MAX;
+            if (p.have_tlen) { amax = p.tmax; if (p.tmin > INT32_MIN) amin = std::max<int64_t>(p.tmin, 0); }
+            omin = amin / 2 + p.shift;       // truncating division, as the kernels' int32 a / 2
+            omax = amax / 2 + p.shift;
+        }
+        const int64_t big = int64_t(1) << 40;
+        if (std::max(std::abs(omin), std::abs(omax)) + idx_.reach + 2 > INT32_MAX) return FusedHalos{big, big, big, big};
+        auto halo = [&](int64_t smax, int64_t* lo, int64_t* hi) {
+            *lo = std::max(omax, std::max<int64_t>(smax, 1) - 1 - omin);
+            *hi = std::max(-omin, omax);
+        };
+        FusedHalos h;
+        halo(idx_.short_max, &h.s_lo, &h.s_hi);
+        halo(idx_.long_max, &h.l_lo, &h.l_hi);
+        return h;
+    }
+
+    // Rows the fused join examines with halos h: K3f itself, run over all tiles on the device (its candidate count comes
+    // back; ~0.1 ms, against 27-49 ms for four host binary searches per tile over the sampled keys on C2).  Cached for
+    // the last kEstCache (tile table, halos) pairs, so a session that alternates a few parameter sets pays it once per set.
+    int64_t fused_rows_estimate(const FusedHalos& h) {
+        for (const EstEntry& e : est_cache_)
+            if (e.gen == my_tiles_gen_ && memcmp(&e.h, &h, sizeof h) == 0) return e.rows;
+        DeviceCtx& c = *ctx_;
+        DeviceScalars* sc = c.scalars.as<DeviceScalars>();
+        fused_rng_.ensure(size_t(2 * n_tiles_) * sizeof(int64_t) + 64);
+        BSG_CUDA(cudaMemsetAsync(&sc->candidates, 0, sizeof(sc->candidates), c.s_comp));
+        launch_join_fused(resident_view(), tile_table(0), fused_rng_.as<int64_t>(), fused_rng_.as<int64_t>() + n_tiles_, n_tiles_, h, sc,
+                          c.s_comp);
+        DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
+        BSG_CUDA(cudaMemcpyAsync(&hs->candidates, &sc->candidates, sizeof(sc->candidates), cudaMemcpyDeviceToHost, c.s_comp));
+        BSG_CUDA(cudaStreamSynchronize(c.s_comp));
+        const int64_t rows = int64_t(hs->candidates);
+        if (est_cache_.size() >= size_t(kEstCache)) est_cache_.erase(est_cache_.begin());
+        est_cache_.push_back(EstEntry{my_tiles_gen_, h, rows});
+        return rows;
+    }
+
+public:
+    // Staged pileup calls (after prepare_tiles): the fused step when opts.resident_scheme is 2, or when it is 0 and the
+    // rows the fused join would examine are at most kFusedShare of the resident rows; else K1 over every resident record.
+    void prepare_resident_pileup(Mode mode, const FilterParams& fp) {
+        const int scheme = opts_.resident_scheme;
+        bool fused = scheme == 2;
+        FusedHalos h{};
+        if (scheme != 1) {
+            h = fused_halos(fp);
+            if (scheme != 2) fused = double(fused_rows_estimate(h)) <= kFusedShare * double(idx_.n);
+        }
+        if (!fused) { decode_resident(mode, fp); return; }
+        BSG_CUDA(cudaMemsetAsync(ctx_->scalars.p, 0, sizeof(DeviceScalars), ctx_->s_comp));
+        fused_ = true;
+        fused_h_ = h;
+    }
+
+private:
+    struct ResidentIndexHost {
+        int64_t n = 0;                          // resident rows
+        uint32_t status = 0;                    // STATUS_* bits of the resident records
+        int64_t reach = 0;                      // max(pos + span)
+        uint32_t long_span = ~0u;               // T: rows with span > T are on the long list
+        int64_t short_max = 0, long_max = 0;    // largest span at most T / above T
+        int64_t n_keys = 0, n_long = 0;         // sampled keys (device), long-list rows (device)
+    };
 
     struct ResidentBatch { uint64_t raw_base; int64_t offs_base; int64_t n; };
 
@@ -1702,6 +1896,14 @@ private:
     int64_t plan_ext_ = 0;
     double plan_ms_ = 0;
     int resident_chunks_ = 0;
+    // the fused pileup step of staged sessions (build_resident_index, prepare_resident_pileup)
+    ResidentIndexHost idx_;
+    DevBuf idx_keys_, idx_long_key_, idx_long_row_, idx_scal_, fused_rng_;
+    bool fused_ = false;                 // this call counts through K3f + K4f
+    FusedHalos fused_h_{};
+    struct EstEntry { uint64_t gen; FusedHalos h; int64_t rows; };
+    static constexpr int kEstCache = 8;
+    std::vector<EstEntry> est_cache_;    // fused_rows_estimate's cache, oldest first
     // background pre-faulting of the caller's output buffer
     std::mutex pf_m_;
     std::condition_variable pf_cv_;
@@ -2153,7 +2355,7 @@ int bsg_pileup_staged(bsg_stage* st, const int32_t* tlen_filter, int32_t mapqual
         st->s->use_host_output();
         st->s->prepare_tiles(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, binsize, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
-        st->s->decode_resident(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, fp);
+        st->s->prepare_resident_pileup(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, fp);
         st->s->count(binsize <= 0 ? MODE_COUNT : MODE_PROFILE, fp, binsize, ss != 0, out, out_offsets, nullptr, out != nullptr);
         st->s->finish_timings(t0);
     });
@@ -2197,7 +2399,7 @@ int bsg_pileup_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_t 
         st->s->use_device_output(d_out, static_cast<cudaStream_t>(stream));
         st->s->prepare_tiles(mode, binsize, ss != 0, out_offsets);
         const FilterParams fp = make_params(tlen_filter, mapqual, shift, requiredF, filteredF, pe_mid, 0);
-        st->s->decode_resident(mode, fp);
+        st->s->prepare_resident_pileup(mode, fp);
         st->s->count(mode, fp, binsize, ss != 0, nullptr, out_offsets, nullptr, false);
         st->s->finish_timings(t0);
     });

@@ -95,6 +95,50 @@ __device__ __forceinline__ Decoded decode_one(const LD& ld, uint32_t o, uint32_t
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return uint32_t(__cvta_generic_to_shared(p)); }
 
+// (tid, pos) of the record at the start of raw + o
+__device__ __forceinline__ int2 record_key(const uint8_t* raw, uint32_t o) {
+    const GlobalLd ld{raw};
+    const uint32_t a = o + 4, b = a & ~3u, sh = (a & 3u) * 8;
+    const uint32_t w0 = ld(b), w1 = ld(b + 4), w2 = ld(b + 8);
+    return make_int2(int32_t(__funnelshift_r(w0, w1, sh)), int32_t(__funnelshift_r(w1, w2, sh)));
+}
+
+// Bring raw[lo, lo + bytes) into shared memory with one bulk copy that completes on the mbarrier at bar_a (thread 0).
+__device__ __forceinline__ void bulk_to_shared(uint32_t bar_a, void* dst, const uint8_t* src, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(bar_a) : "memory");
+}
+__device__ __forceinline__ void wait_parity(uint32_t bar_a, uint32_t parity) {
+    uint32_t done = 0;
+    while (!done)
+        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                     : "=r"(done) : "r"(bar_a), "r"(parity) : "memory");
+}
+
+// K1's chunks of a multi-batch launch (and the resident index's, which are the same): the batch that chunk blk belongs to
+__device__ __forceinline__ int chunk_batch(const DecodeBatch* __restrict__ table, int n_batches, int blk) {
+    int lo = 0, hi = n_batches - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (blk >= table[mid].chunk0) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Coordinate-sortedness, K1 and the resident index: the (tid, pos) of the record before record i of resident batch bi,
+// from the raw bytes - record i - 1 of the batch, or for i == 0 the last record of batch bi - 1 (callers ensure that
+// one exists)
+__device__ __forceinline__ int2 key_before(const DecodeBatch* __restrict__ table, int bi, const DecodeBatch& B, int i) {
+    if (i > 0) return record_key(B.raw, __ldg(B.offs + i - 1));
+    const DecodeBatch& P = table[bi - 1];
+    return record_key(P.raw, __ldg(P.offs + P.n - 1));
+}
+__device__ __forceinline__ bool before_key(uint32_t tid, int32_t pos, uint32_t ptid, int32_t ppos) {
+    return tid < ptid || (tid == ptid && pos < ppos);
+}
+
+
 // setRead's filter (src/bamsignals.cpp:328-333, :394-399)
 __device__ __forceinline__ bool keep_read(const FilterParams& p, uint32_t fm, int32_t tlen, int32_t* abs_tlen) {
     const uint32_t flag = fm & 0xffffu, mapq = fm >> 16;
@@ -105,6 +149,13 @@ __device__ __forceinline__ bool keep_read(const FilterParams& p, uint32_t fm, in
     keep = keep && (p.filtered & ~flag);           // not all filtered bits present (:329); filtered == 0 drops all
     keep = keep && (!p.have_tlen || (a >= p.tmin && a <= p.tmax));
     return keep;
+}
+
+// setRead's pileup coordinate (src/bamsignals.cpp:339-344): the read's 5' end, or with `midpoint` its fragment's
+// midpoint, moved `shift` bases downstream.  Shared by K1 and the fused resident kernel.
+__device__ __forceinline__ int32_t pileup_coord(const FilterParams& p, const Decoded& d, int32_t abs_tlen, bool neg) {
+    const int32_t offset = p.midpoint ? abs_tlen / 2 + p.shift : p.shift;                 // :339
+    return neg ? d.end - offset : d.pos + offset;                                         // :340-344
 }
 
 // K1+K2 fused: the filter and the pileup / coverage coordinate (setRead, :326-346 and :392-415) are applied to the
@@ -125,13 +176,8 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
     DecodeBatch B = single;
     int bi = 0;
     if (table) {
-        int lo = 0, hi = n_batches - 1;
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (int(blockIdx.x) >= table[mid].chunk0) lo = mid; else hi = mid - 1;
-        }
-        B = table[lo];
-        bi = lo;
+        bi = chunk_batch(table, n_batches, int(blockIdx.x));
+        B = table[bi];
     }
     const int i0 = (int(blockIdx.x) - B.chunk0) * kDecThreads;
     const int i = i0 + threadIdx.x;
@@ -145,9 +191,7 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
             const uint32_t bar_a = smem_u32(&bar);
             asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(smem_u32(sm_raw)), "l"(B.raw + lo), "r"(bytes), "r"(bar_a) : "memory");
+            bulk_to_shared(bar_a, sm_raw, B.raw + lo, bytes);
             s_lo = lo; s_bytes = bytes;
         } else {
             s_lo = 0; s_bytes = 0;
@@ -164,13 +208,7 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
     const int lane = threadIdx.x & 31;
     __syncthreads();
     const bool staged = s_bytes != 0;
-    if (staged) {
-        const uint32_t bar_a = smem_u32(&bar);
-        uint32_t done = 0;
-        while (!done)
-            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0; selp.u32 %0, 1, 0, p; }"
-                         : "=r"(done) : "r"(bar_a) : "memory");
-    }
+    if (staged) wait_parity(smem_u32(&bar), 0);
     Decoded d;
     d.tid = -1; d.pos = -1; d.end = -1; d.tlen = 0; d.flagmq = 0; d.bad = 0;
     const SharedLd sld{sm_raw, s_lo};
@@ -184,8 +222,7 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
         const bool neg = (d.flagmq & 0x10u) != 0;
         int32_t o0, o1;
         if (!COVERAGE) {
-            const int32_t offset = p.midpoint ? a / 2 + p.shift : p.shift;               // :339
-            const int32_t pos5 = neg ? d.end - offset : d.pos + offset;                  // :340-344
+            const int32_t pos5 = pileup_coord(p, d, a, neg);
             o0 = pos5;
             o1 = keep ? int32_t(neg) : -1;
             if (keep) { hlo = pos5 - d.pos; hhi = d.pos - pos5; }
@@ -227,19 +264,13 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
             const int2 l = s_last[wid - 1];
             ptid = uint32_t(l.x); ppos = l.y;
         } else if (i > 0) {
-            const uint32_t a = __ldg(B.offs + i - 1) + 4, b = a & ~3u, sh = (a & 3u) * 8;
-            const uint32_t w0 = gld(b), w1 = gld(b + 4), w2 = gld(b + 8);
-            ptid = __funnelshift_r(w0, w1, sh);
-            ppos = int32_t(__funnelshift_r(w1, w2, sh));
+            const int2 k = record_key(B.raw, __ldg(B.offs + i - 1));
+            ptid = uint32_t(k.x); ppos = k.y;
         } else if (table && bi > 0) {
             // first record of a resident batch: the record before it is the last one of the batch before, which this
             // same launch decodes (its table row may not be written yet): read it from the raw bytes
-            const DecodeBatch Bp = table[bi - 1];
-            const GlobalLd pld{Bp.raw};
-            const uint32_t a = __ldg(Bp.offs + Bp.n - 1) + 4, b = a & ~3u, sh = (a & 3u) * 8;
-            const uint32_t w0 = pld(b), w1 = pld(b + 4), w2 = pld(b + 8);
-            ptid = __funnelshift_r(w0, w1, sh);
-            ppos = int32_t(__funnelshift_r(w1, w2, sh));
+            const int2 k = key_before(table, bi, B, 0);
+            ptid = uint32_t(k.x); ppos = k.y;
         } else if (B.row0 > 0) {          // streaming path: the row was written by an earlier launch on this stream
             ptid = uint32_t(t.tid[B.row0 - 1]);
             ppos = t.pos[B.row0 - 1];
@@ -248,7 +279,7 @@ __device__ __forceinline__ void decode_chunk(DecodeBatch single, const DecodeBat
         }
     }
     uint32_t bad = d.bad;
-    if (have_prev && (uint32_t(d.tid) < ptid || (uint32_t(d.tid) == ptid && d.pos < ppos))) bad |= STATUS_UNSORTED;
+    if (have_prev && before_key(uint32_t(d.tid), d.pos, ptid, ppos)) bad |= STATUS_UNSORTED;
     if (bad) atomicOr(&sc->status, bad);
     // halo maxima and the kept-read count: published once per CTA, the maxima only when they beat the value read at the
     // start, the count into one of kKeptSlots counters that sit on different 128-byte lines (atomics on one line
@@ -374,18 +405,30 @@ __device__ __forceinline__ uint32_t fast_div(uint32_t n, uint64_t magic, uint32_
 // The histograms are built by __device__ helpers shared with the run-length kernels (K4r), so that both count every
 // tile through the same code: hist[0, nout) zeroed before, the caller's barrier after.
 // ---------------------------------------------------------------------------------------------------------------
+// One read of a tile (Pileupper::pileup, :349-363): its histogram slot, or -1 when the tile does not count it.
+// p5 = pileup coordinate, ng = 0 '+', 1 '-', -1 dropped by the filter.  BIN: 0 = binsize 1, 1 = floor(rel / binsize)
+// by the 64-bit multiplier (fast_div), 2 = one bin per tile (bamCount: tiles are whole regions).
+enum : int { kBin1 = 0, kBinDiv = 1, kBinOne = 2 };
+template <bool SS, int BIN>
+__device__ __forceinline__ int32_t profile_slot(int32_t p5, int32_t ng, int32_t loc, int32_t len, int flip, uint64_t magic,
+                                                uint32_t mshift) {
+    int32_t rel = p5 - loc;
+    if (ng < 0 || uint32_t(rel) >= uint32_t(len)) return -1;                       // src/bamsignals.cpp:351-353
+    const int a = (ng ^ flip) & 1;
+    if (flip) rel = len - 1 - rel;                                                 // :356-359
+    const int32_t bin = BIN == kBin1 ? rel : (BIN == kBinOne ? 0 : int32_t(fast_div(uint32_t(rel), magic, mshift)));
+    return SS ? 2 * bin + a : bin;                                                 // :361-362
+}
+
 template <bool SS, bool BIN1>
 __device__ __forceinline__ void scatter_profile(int32_t* hist, int32_t loc, int32_t len, int flip, int64_t lo, int64_t hi,
                                                 const int32_t* __restrict__ c0, const int32_t* __restrict__ c1,
                                                 uint64_t magic, uint32_t mshift) {
     for (int64_t i = lo + threadIdx.x; i < hi; i += kThreads) {
         const int32_t p5 = __ldg(c0 + i), ng = __ldg(c1 + i);
-        int32_t rel = p5 - loc;
-        if (ng < 0 || uint32_t(rel) >= uint32_t(len)) continue;                    // src/bamsignals.cpp:351-353
-        const int a = (ng ^ flip) & 1;
-        if (flip) rel = len - 1 - rel;                                             // :356-359
-        const int32_t bin = BIN1 ? rel : int32_t(fast_div(uint32_t(rel), magic, mshift));
-        atomicAdd(&hist[SS ? 2 * bin + a : bin], 1);                               // :361-362
+        const int32_t k = profile_slot<SS, BIN1 ? kBin1 : kBinDiv>(p5, ng, loc, len, flip, magic, mshift);
+        if (k < 0) continue;
+        atomicAdd(&hist[k], 1);
     }
 }
 
@@ -1078,6 +1121,259 @@ __global__ void __launch_bounds__(kThreads) k_profile_runs_write(TileTable tiles
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// Staged sessions: the resident record index (K0i, once per session) and the fused pileup step (K3f join, K4f count).
+// K1 decodes every resident record on every call, but the fetch planner works in whole BGZF blocks and 16 kb index
+// windows, so most of them lie far from every region (C2: 57.8 M resident records, ~7 M near a region).  The fused
+// step finds each tile's rows from a sampled key index and decodes only those, inside the counting CTA.
+// ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned long long pack_key(int32_t tid, int32_t pos) {
+    return (unsigned long long)uint32_t(tid) << 32 | (uint32_t(pos) ^ 0x80000000u);
+}
+// key < (qt, qp) in lower_bound_tp's order: tid as uint32, then pos as a signed number (qp may lie outside int32)
+__device__ __forceinline__ bool key_less(unsigned long long k, uint32_t qt, int64_t qp) {
+    const uint32_t t = uint32_t(k >> 32);
+    const int64_t p = int32_t(uint32_t(k) ^ 0x80000000u);
+    return t < qt || (t == qt && p < qp);
+}
+
+// the resident batch that holds row r (the table has one entry per non-empty batch, rows contiguous)
+__device__ __forceinline__ int batch_of_row(const ResidentView& v, int64_t r) {
+    int lo = 0, hi = v.n_batches - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (r >= __ldg(&v.batches[mid].row0)) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// K0i: one pass over every resident record (K1's chunking, bulk copy and decode_one).  PASS 0: sampled keys, the
+// unsorted / corrupt status bits (K1's checks, across batch boundaries too), reach = max(pos + span) and the span
+// buckets the host picks the long-span threshold from.  PASS 1: appends every row with span > long_span to the long
+// list, in no particular order (the host sorts it).
+template <int PASS>
+__global__ void __launch_bounds__(kDecThreads) k_resident_index(const DecodeBatch* __restrict__ table, int n_batches,
+                                                                uint32_t long_span, unsigned long long* __restrict__ keys,
+                                                                unsigned long long* __restrict__ long_key, int2* __restrict__ long_row,
+                                                                IndexScalars* isc) {
+    extern __shared__ __align__(128) uint8_t sm_raw[];
+    __shared__ __align__(8) uint64_t bar;
+    __shared__ uint32_t s_lo, s_bytes, s_nl, s_base;
+    __shared__ int2 s_key[kDecThreads];
+    __shared__ uint32_t s_bn[kSpanBuckets], s_bm[kSpanBuckets];
+    __shared__ long long s_reach;
+    const int bi = chunk_batch(table, n_batches, int(blockIdx.x));
+    const DecodeBatch B = table[bi];
+    const int i0 = (int(blockIdx.x) - B.chunk0) * kDecThreads;
+    const int i = i0 + threadIdx.x;
+    const bool active = i < B.n;
+    if (threadIdx.x < kSpanBuckets) { s_bn[threadIdx.x] = 0; s_bm[threadIdx.x] = 0; }
+    if (threadIdx.x == 0) {
+        const int i1 = min(i0 + kDecThreads, B.n);
+        const uint32_t lo = B.offs[i0] & ~15u;
+        const uint32_t bytes = (B.offs[i1] - lo + 15u) & ~15u;
+        s_lo = lo; s_bytes = 0; s_nl = 0; s_reach = 0;
+        if (bytes <= uint32_t(kSpanCap)) {
+            const uint32_t bar_a = smem_u32(&bar);
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
+            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            bulk_to_shared(bar_a, sm_raw, B.raw + lo, bytes);
+            s_bytes = bytes;
+        }
+    }
+    uint32_t o = 0, rec_end = 0;
+    if (active) { o = __ldg(B.offs + i); rec_end = __ldg(B.offs + i + 1); }
+    __syncthreads();
+    const bool staged = s_bytes != 0;
+    if (staged) wait_parity(smem_u32(&bar), 0);
+    Decoded d;
+    d.tid = -1; d.pos = -1; d.end = -1; d.tlen = 0; d.flagmq = 0; d.bad = 0;
+    uint32_t span = 0;
+    if (active) {
+        d = staged ? decode_one(SharedLd{sm_raw, s_lo}, o, rec_end) : decode_one(GlobalLd{B.raw}, o, rec_end);
+        span = uint32_t(d.end) - uint32_t(d.pos) + 1u;                 // decode_one's reference length (>= 1)
+    }
+    const int64_t row = B.row0 + i;
+    if (PASS == 0) {
+        s_key[threadIdx.x] = make_int2(d.tid, d.pos);
+        if (active) {
+            const int bk = 31 - __clz(span);
+            atomicAdd(&s_bn[bk], 1u);
+            atomicMax(&s_bm[bk], span);
+            atomicMax(&s_reach, (long long)(int64_t(d.pos) + int64_t(span)));   // signed: a malformed pos < -1 cannot win
+            if ((row & (kIndexStride - 1)) == 0) keys[row / kIndexStride] = pack_key(d.tid, d.pos);
+        }
+        __syncthreads();
+        uint32_t bad = d.bad;
+        if (active) {
+            const bool have_prev = threadIdx.x > 0 || i > 0 || bi > 0;
+            const int2 prev = threadIdx.x > 0 ? s_key[threadIdx.x - 1] : (have_prev ? key_before(table, bi, B, i) : make_int2(0, 0));
+            if (have_prev && before_key(uint32_t(d.tid), d.pos, uint32_t(prev.x), prev.y)) bad |= STATUS_UNSORTED;
+        }
+        if (bad) atomicOr(&isc->status, bad);
+        if (threadIdx.x < kSpanBuckets && s_bn[threadIdx.x]) {
+            atomicAdd(&isc->bucket_n[threadIdx.x], s_bn[threadIdx.x]);
+            atomicMax(&isc->bucket_max[threadIdx.x], s_bm[threadIdx.x]);
+        }
+        if (threadIdx.x == 0) atomicMax(&isc->reach, s_reach);
+    } else {
+        const bool is_long = active && span > long_span;
+        const uint32_t slot = is_long ? atomicAdd(&s_nl, 1u) : 0u;
+        __syncthreads();
+        if (threadIdx.x == 0 && s_nl) s_base = atomicAdd(&isc->n_long, s_nl);
+        __syncthreads();
+        if (is_long) {
+            long_key[s_base + slot] = pack_key(d.tid, d.pos);
+            long_row[s_base + slot] = make_int2(bi, i);
+        }
+    }
+}
+
+// K3f: per tile, the short-span rows with key in [loc - s_lo, loc + len + s_hi) and the long-list entries with key in
+// [loc - l_lo, loc + len + l_hi).  A short range is found in the sampled keys first (every 32nd row; they stay in L2),
+// then among the <= 31 rows between two samples through offs[] and the raw bytes.
+__device__ __forceinline__ int64_t lower_bound_rows(const ResidentView& v, uint32_t qt, int64_t qp) {
+    int64_t lo = 0, hi = v.n_keys;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (key_less(__ldg(v.keys + mid), qt, qp)) lo = mid + 1; else hi = mid;
+    }
+    if (lo == 0) return 0;                                   // row 0 is not below the key
+    int64_t a = (lo - 1) * kIndexStride + 1, b = min(lo * kIndexStride, v.n);   // row a-1 is below, row b is not (or n)
+    while (a < b) {
+        const int64_t mid = (a + b) >> 1;
+        const DecodeBatch& B = v.batches[batch_of_row(v, mid)];
+        const int2 k = record_key(B.raw, __ldg(B.offs + (mid - B.row0)));
+        if (key_less(pack_key(k.x, k.y), qt, qp)) a = mid + 1; else b = mid;
+    }
+    return a;
+}
+__device__ __forceinline__ int64_t lower_bound_long(const ResidentView& v, uint32_t qt, int64_t qp) {
+    int64_t lo = 0, hi = v.n_long;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (key_less(__ldg(v.long_key + mid), qt, qp)) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(kThreads) k_join_fused(ResidentView v, TileTable tiles, int64_t* __restrict__ long_lo,
+                                                         int64_t* __restrict__ long_hi, int64_t n_tiles, FusedHalos h,
+                                                         DeviceScalars* sc) {
+    const int64_t i = int64_t(blockIdx.x) * kThreads + threadIdx.x;
+    long long cand = 0;
+    if (i < n_tiles) {
+        const uint32_t rid = uint32_t(tiles.rid[i]);
+        const int64_t loc = tiles.loc[i], len = tiles.len[i];
+        const int64_t lo = lower_bound_rows(v, rid, loc - h.s_lo);
+        const int64_t hi = max(lo, lower_bound_rows(v, rid, loc + len + h.s_hi));
+        const int64_t llo = lower_bound_long(v, rid, loc - h.l_lo);
+        const int64_t lhi = max(llo, lower_bound_long(v, rid, loc + len + h.l_hi));
+        tiles.cand_lo[i] = lo; tiles.cand_hi[i] = hi;
+        long_lo[i] = llo; long_hi[i] = lhi;
+        cand = (hi - lo) + (lhi - llo);
+    }
+    __shared__ long long s_c[kThreads / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) cand += __shfl_xor_sync(FULL, cand, o);
+    if ((threadIdx.x & 31) == 0) s_c[threadIdx.x >> 5] = cand;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        long long tot = 0;
+        for (int k = 0; k < kThreads / 32; ++k) tot += s_c[k];
+        if (tot) atomicAdd(&sc->candidates, (unsigned long long)tot);
+    }
+}
+
+// K4f: one CTA per tile.  The tile's short range goes through shared memory in chunks of <= kThreads rows that stay
+// inside one resident batch, one bulk copy per chunk (a chunk whose bytes exceed kFusedCap is halved until it fits; a
+// single record that does not fit takes the global-load path); one thread per record: decode_one, keep_read,
+// pileup_coord, profile_slot - K1's and K4's code.  Rows with span > long_span are left to the long list, which is read
+// with global loads.  Then copy_out, as k_profile.
+constexpr int kFusedCap = 12288;          // staging bytes per CTA: 256 records of <= 48 B, or fewer larger ones
+template <bool SS, int BIN>
+__global__ void __launch_bounds__(kThreads) k_pileup_fused(ResidentView v, TileTable tiles, const int64_t* __restrict__ long_lo,
+                                                           const int64_t* __restrict__ long_hi, FilterParams p, int32_t binsize,
+                                                           uint64_t magic, uint32_t mshift, int32_t* __restrict__ out) {
+    extern __shared__ __align__(128) uint8_t smem_f[];
+    __shared__ __align__(8) uint64_t bar;
+    __shared__ uint32_t s_lo, s_bytes;
+    __shared__ int s_b;
+    __shared__ long long s_r1;
+    const int64_t tix = blockIdx.x;
+    const int32_t loc = tiles.loc[tix], len = tiles.len[tix];
+    const int flip = tiles.strand[tix] < 0 ? 1 : 0;
+    const int64_t lo = tiles.cand_lo[tix], hi = tiles.cand_hi[tix];
+    const int64_t off = tiles.out_off[tix];
+    const int nbins = BIN == kBinOne ? 1 : (BIN == kBin1 ? len : int((uint32_t(len) + uint32_t(binsize) - 1u) / uint32_t(binsize)));
+    const int nout = SS ? 2 * nbins : nbins;
+    int32_t* const dst = out + off;
+    int32_t* hist = reinterpret_cast<int32_t*>(smem_f + kFusedCap) + out_phase(dst);     // same 16-byte phase as dst
+    const uint32_t bar_a = smem_u32(&bar);
+    // thread 0 stages the chunk of rows that starts at r0: <= kThreads rows inside one resident batch, halved until
+    // their bytes fit the staging buffer (s_bytes = 0: one record too large, the chunk takes the global-load path)
+    auto stage_chunk = [&](int64_t r0) {
+        const int b = batch_of_row(v, r0);
+        const DecodeBatch B = v.batches[b];
+        int64_t r1 = min(hi, min(r0 + kThreads, B.row0 + B.n));
+        const uint32_t o_lo = B.offs[r0 - B.row0] & ~15u;
+        uint32_t bytes = (B.offs[r1 - B.row0] - o_lo + 15u) & ~15u;
+        while (bytes > uint32_t(kFusedCap) && r1 - r0 > 1) {
+            r1 = r0 + (r1 - r0) / 2;
+            bytes = (B.offs[r1 - B.row0] - o_lo + 15u) & ~15u;
+        }
+        s_bytes = 0;
+        if (bytes <= uint32_t(kFusedCap)) { bulk_to_shared(bar_a, smem_f, B.raw + o_lo, bytes); s_bytes = bytes; }
+        s_lo = o_lo; s_b = b; s_r1 = r1;
+    };
+    // the first chunk's copy is in flight while the histogram is zeroed and the long-list rows are counted
+    if (threadIdx.x == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        if (lo < hi) stage_chunk(lo);
+    }
+    {
+        int4* h4 = reinterpret_cast<int4*>(smem_f + kFusedCap);
+        const int nq = (int(hist - reinterpret_cast<int32_t*>(h4)) + nout + 3) >> 2;
+        for (int k = threadIdx.x; k < nq; k += kThreads) h4[k] = make_int4(0, 0, 0, 0);
+    }
+    __syncthreads();
+    auto count = [&](const Decoded& d) {
+        int32_t a;
+        const bool keep = keep_read(p, d.flagmq, d.tlen, &a);
+        const bool neg = (d.flagmq & 0x10u) != 0;
+        const int32_t k = profile_slot<SS, BIN>(pileup_coord(p, d, a, neg), keep ? int32_t(neg) : -1, loc, len, flip, magic, mshift);
+        if (k >= 0) atomicAdd(&hist[k], 1);
+    };
+    for (int64_t e = long_lo[tix] + threadIdx.x; e < long_hi[tix]; e += kThreads) {
+        const int2 br = __ldg(v.long_row + e);
+        const DecodeBatch& B = v.batches[br.x];
+        count(decode_one(GlobalLd{B.raw}, __ldg(B.offs + br.y), __ldg(B.offs + br.y + 1)));
+    }
+    uint32_t phase = 0;
+    for (int64_t r0 = lo; r0 < hi;) {                                             // block-uniform
+        const int64_t r1 = s_r1;
+        const DecodeBatch& B = v.batches[s_b];
+        const int64_t r = r0 + threadIdx.x;
+        uint32_t o = 0, rec_end = 0;
+        if (r < r1) { o = __ldg(B.offs + (r - B.row0)); rec_end = __ldg(B.offs + (r - B.row0) + 1); }
+        const bool staged = s_bytes != 0;
+        if (staged) { wait_parity(bar_a, phase); phase ^= 1u; }
+        if (r < r1) {
+            const Decoded d = staged ? decode_one(SharedLd{smem_f, s_lo}, o, rec_end) : decode_one(GlobalLd{B.raw}, o, rec_end);
+            if (uint32_t(d.end) - uint32_t(d.pos) + 1u <= v.long_span) count(d);  // a longer read is the long list's
+        }
+        __syncthreads();                                                          // staging buffer and s_* free again
+        r0 = r1;
+        if (r0 < hi) {
+            if (threadIdx.x == 0) stage_chunk(r0);
+            __syncthreads();
+        }
+    }
+    __syncthreads();
+    copy_out(dst, hist, nout);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // Result narrowing (see kernels.cuh): four elements per thread, one 32-bit store; src is only 4-byte aligned.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_pack_u8(const int32_t* __restrict__ src, int64_t n, uint8_t* __restrict__ dst, uint2* ovf,
@@ -1241,6 +1537,33 @@ void launch_profile_runs_write(TileTable tiles, int64_t n_tiles, const int32_t* 
         k_profile_runs_write<SS(), KIND()><<<unsigned(n_tiles), kThreads, size_t(max_tile_ints) * sizeof(int32_t), s>>>(
             tiles, n_tiles, c0, c1, binsize, magic, mshift, rt, vt, run_off, lengths, values);
     });
+}
+
+void launch_resident_index(const DecodeBatch* d_table, int n_batches, int total_chunks, int pass, uint32_t long_span,
+                           unsigned long long* keys, unsigned long long* long_key, int2* long_row, IndexScalars* isc, cudaStream_t s) {
+    if (n_batches <= 0 || total_chunks <= 0) return;
+    if (pass == 0) k_resident_index<0><<<unsigned(total_chunks), kDecThreads, kSpanCap + 32, s>>>(d_table, n_batches, long_span, keys, long_key, long_row, isc);
+    else k_resident_index<1><<<unsigned(total_chunks), kDecThreads, kSpanCap + 32, s>>>(d_table, n_batches, long_span, keys, long_key, long_row, isc);
+}
+
+void launch_join_fused(const ResidentView& v, TileTable tiles, int64_t* long_lo, int64_t* long_hi, int64_t n_tiles,
+                       const FusedHalos& h, DeviceScalars* sc, cudaStream_t s) {
+    if (n_tiles <= 0) return;
+    k_join_fused<<<unsigned((n_tiles + kThreads - 1) / kThreads), kThreads, 0, s>>>(v, tiles, long_lo, long_hi, n_tiles, h, sc);
+}
+
+void launch_pileup_fused(const ResidentView& v, TileTable tiles, const int64_t* long_lo, const int64_t* long_hi, int64_t n_tiles,
+                         int ss, int32_t binsize, int max_tile_ints, const FilterParams& p, int32_t* out, cudaStream_t s) {
+    if (n_tiles <= 0) return;
+    const size_t smem = kFusedCap + size_t(max_tile_ints + 8) * sizeof(int32_t);
+    uint64_t magic = 0; uint32_t mshift = 0;
+    if (binsize > 1) magic_for(binsize, &magic, &mshift);
+    const unsigned grid = unsigned(n_tiles);
+#define BSG_LAUNCH_FUSED(SS, BIN) k_pileup_fused<SS, BIN><<<grid, kThreads, smem, s>>>(v, tiles, long_lo, long_hi, p, binsize, magic, mshift, out)
+    if (binsize <= 0)      { if (ss) BSG_LAUNCH_FUSED(true, kBinOne); else BSG_LAUNCH_FUSED(false, kBinOne); }
+    else if (binsize == 1) { if (ss) BSG_LAUNCH_FUSED(true, kBin1);   else BSG_LAUNCH_FUSED(false, kBin1); }
+    else                   { if (ss) BSG_LAUNCH_FUSED(true, kBinDiv); else BSG_LAUNCH_FUSED(false, kBinDiv); }
+#undef BSG_LAUNCH_FUSED
 }
 
 void launch_pack_u8(const int32_t* d_src, int64_t n, uint8_t* d_dst, uint2* ovf, uint32_t cap, uint32_t* d_cnt, cudaStream_t s) {

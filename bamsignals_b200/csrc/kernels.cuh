@@ -79,6 +79,41 @@ void launch_decode(const DecodeBatch& one, ReadTable t, bool coverage, bool ss, 
 void launch_decode_table(const DecodeBatch* d_table, int n_batches, int total_chunks, ReadTable t, bool coverage, bool ss,
                          const FilterParams& p, DeviceScalars* sc, cudaStream_t s);
 
+// Staged sessions (DESIGN.md §13): the resident record index, built once by launch_resident_index, and the fused pileup
+// step that decodes only the rows near each tile.  A key is uint64: tid as uint32 in the high half, pos ^ 0x80000000 in
+// the low half, so that unsigned order is lower_bound_tp's (tid as uint32, then pos as a signed number).
+constexpr int kIndexStride = 32;    // one sampled key per 32 rows
+constexpr int kSpanBuckets = 32;    // span bucket b = floor(log2(span))
+struct IndexScalars {
+    uint32_t status;                    // STATUS_UNSORTED / STATUS_CORRUPT as K1 detects them
+    uint32_t n_long;                    // pass 1: rows appended to the long list
+    long long reach;                    // max(0, max over rows of pos + span), a signed maximum
+    uint32_t bucket_n[kSpanBuckets];    // rows per span bucket
+    uint32_t bucket_max[kSpanBuckets];  // largest span per bucket
+};
+struct ResidentView {
+    const DecodeBatch* batches;         // the session's batch table (device)
+    int n_batches;
+    int64_t n;                          // resident rows
+    const unsigned long long* keys;     // keys[j] = key of row kIndexStride * j
+    int64_t n_keys;
+    const unsigned long long* long_key; // rows with span > long_span, in key order ...
+    const int2* long_row;               // ... and where they are: (batch, record of the batch)
+    int64_t n_long;
+    uint32_t long_span;
+};
+// Key ranges around a tile [loc, loc + len): short rows with pos in [loc - s_lo, loc + len + s_hi), long rows likewise.
+struct FusedHalos { int64_t s_lo, s_hi, l_lo, l_hi; };
+// pass 0: keys[], status, reach, span buckets (isc zeroed before); pass 1: the long list, unsorted (isc->n_long zeroed)
+void launch_resident_index(const DecodeBatch* d_table, int n_batches, int total_chunks, int pass, uint32_t long_span,
+                           unsigned long long* keys, unsigned long long* long_key, int2* long_row, IndexScalars* isc, cudaStream_t s);
+// K3f: tiles.cand_lo/hi = short row range, long_lo/hi = long list range; sc->candidates += rows examined
+void launch_join_fused(const ResidentView& v, TileTable tiles, int64_t* long_lo, int64_t* long_hi, int64_t n_tiles,
+                       const FusedHalos& h, DeviceScalars* sc, cudaStream_t s);
+// K4f: bamProfile (binsize >= 1) or bamCount (binsize <= 0, one tile per region) straight from the raw records
+void launch_pileup_fused(const ResidentView& v, TileTable tiles, const int64_t* long_lo, const int64_t* long_hi, int64_t n_tiles,
+                         int ss, int32_t binsize, int max_tile_ints, const FilterParams& p, int32_t* out, cudaStream_t s);
+
 // K0 (gpu_inflate): one BGZF block = one raw-DEFLATE stream of at most 64 KiB.
 struct InflateBlock {
     uint32_t in_off;    // byte offset of the DEFLATE payload in the batch's compressed buffer

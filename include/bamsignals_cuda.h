@@ -87,17 +87,22 @@ typedef struct bsg_opts {
                                  chains that the inflate kernel follows while the blocks are L2-resident, and only what
                                  those cannot cover is walked; 0 (default) = 1 when no span of the batch exceeds 96 KiB,
                                  else 2 */
-    int32_t reserved[5];
+    int32_t resident_scheme;  /* staged bamProfile / bamCount calls (bsg_pileup_staged*): 1 = decode every resident record
+                                 (K1) and join against the read table; 2 = fused: find each tile's rows in the session's
+                                 record index and decode only those, inside the counting kernel; 0 (default) = 2 when the
+                                 fused join would examine at most 0.3 of the resident records, else 1.  Same results. */
+    int32_t reserved[4];
 } bsg_opts;
 
 /* Counters and timings of the last call on this thread (milliseconds; kernel times from CUDA events on the
  * launching stream, summed over launches and max over devices). */
 typedef struct bsg_timings {
-    int64_t records;          /* alignment records decoded (inside the fetched ranges) */
-    int64_t records_kept;     /* records that passed the mapq/flag/tlen filter */
+    int64_t records;          /* records of the fetched ranges the call answers for */
+    int64_t records_kept;     /* records that passed the mapq/flag/tlen filter; -1 for a staged call on the fused path
+                                 (opts.resident_scheme), which filters only the rows it examines */
     int64_t bytes_compressed; /* BGZF bytes read */
     int64_t bytes_inflated;   /* uncompressed bytes produced */
-    int64_t candidates;       /* (read, tile) pairs examined by the counting kernels */
+    int64_t candidates;       /* (read, tile) pairs examined by the counting kernels (fused path: rows the join hands them) */
     int64_t out_elems;        /* int32 written to the result */
     int64_t n_tiles;
     int64_t n_batches;
@@ -106,7 +111,8 @@ typedef struct bsg_timings {
     int32_t upload_mode;      /* device inflate: 1 = compressed bytes DMA'd straight from the page-locked file mapping,
                                  0 = staged through pinned chunks by the worker pool (or host inflate) */
     double ms_total, ms_plan, ms_fetch, ms_h2d, ms_d2h;
-    double ms_decode, ms_filter, ms_join, ms_count, ms_inflate_gpu, ms_kernels;
+    double ms_decode, ms_filter, ms_join, ms_count, ms_inflate_gpu, ms_kernels;   /* bsg_stage_open: ms_decode is the pass
+                                 that builds the session's record index; a fused staged call has no decode span */
     double ms_device;         /* first to last device event of the call on the compute stream (kernels + gaps) */
     double bytes_d2h;         /* result bytes that crossed PCIe device -> host (packed bytes + (index, value) pairs, or int32) */
     double reserved[6];

@@ -448,6 +448,8 @@ def lib():
     L.bsg_runs_read.restype = C.c_int
     L.bsg_runs_free.argtypes = [C.c_void_p]
     L.bsg_runs_free.restype = None
+    L.bsg_stage_view.argtypes = [C.POINTER(C.c_void_p), C.c_void_p] + region_args[1:]
+    L.bsg_stage_view.restype = C.c_int
     L.bsg_stage_close.argtypes = [C.c_void_p]
     L.bsg_stage_close.restype = None
     L.bsg_debug_plan.argtypes = region_args + [C.c_int64, i64p, i64p, i64p, i32p, i32p, C.c_int64]
@@ -749,6 +751,18 @@ class Stage:
                                              int(shift), int(bool(ss)), int(requiredF), int(filteredF), int(bool(pe_mid)),
                                              _p(offsets, C.c_int64), C.byref(h)))
         return ProfileRuns(*_take_runs(h, offsets, dev), offsets, ss)
+
+    def view(self, gr) -> "Stage":
+        """The same resident records, counted over another region set (bsg_stage_view): no BAM bytes are read again.
+        The returned Stage has every method of this one, with its layouts from `gr`, and this session's options and
+        device.  A region outside what the session fetched is refused (BamsignalsError), as is a later call that needs
+        more halo around `gr` than the session's index queries cover.  Closing this session first leaves the view usable."""
+        m = marshal_regions(gr)
+        v = Stage.__new__(Stage)
+        v._m, v._h = m, C.c_void_p()
+        _check(lib().bsg_stage_view(C.byref(v._h), self._h, m.R, m.levels, m.n_levels, _p(m.seq_idx, C.c_int32),
+                                    _p(m.loc, C.c_int32), _p(m.width, C.c_int32), _p(m.strand, C.c_int8)))
+        return v
 
     def close(self):
         if self._h:

@@ -414,6 +414,46 @@ struct Batch {
     Error err{0, ""};
 };
 
+struct ResidentIndexHost {
+    int64_t n = 0;                          // resident rows
+    uint32_t status = 0;                    // STATUS_* bits of the resident records
+    int64_t reach = 0;                      // max(pos + span)
+    uint32_t long_span = ~0u;               // T: rows with span > T are on the long list
+    int64_t short_max = 0, long_max = 0;    // largest span at most T / above T
+    int64_t n_keys = 0, n_long = 0;         // sampled keys (device), long-list rows (device)
+};
+
+struct ResidentBatch { uint64_t raw_base; int64_t offs_base; int64_t n; };
+
+// The records a Session fetched.  A staged session (keep_raw) keeps their raw bytes, offsets, batch table and record
+// index resident; its views (bsg_stage_view) hold the same StagedRecords, so the device memory is released with the
+// last handle that shares it, whichever that is.
+struct StagedRecords {
+    int dev = 0;
+    bool keep_raw = false;
+    std::vector<ResidentBatch> batches;
+    DevBuf raw_all, offs_all, batch_table;
+    int64_t rows_cap = 0, n_rows = 0;
+    int64_t staged_ext = 0;
+    int chunks = 0;
+    // the fused pileup step of staged sessions (build_resident_index, prepare_resident_pileup)
+    ResidentIndexHost idx;
+    DevBuf idx_keys, idx_long_key, idx_long_row, idx_scal;
+    // the fetch plan's merged index queries, (rid, beg) order: every record overlapping one of them is resident
+    std::vector<QueryInterval> queries;
+
+    StagedRecords() = default;
+    StagedRecords(const StagedRecords&) = delete;
+    ~StagedRecords() {
+        if (raw_all.p || offs_all.p || batch_table.p || idx_keys.p || idx_scal.p) {
+            cudaSetDevice(dev);
+            cudaDeviceSynchronize();
+            raw_all.release(); offs_all.release(); batch_table.release();
+            idx_keys.release(); idx_long_key.release(); idx_long_row.release(); idx_scal.release();
+        }
+    }
+};
+
 // ---------------------------------------------------------------------------------------------------------------
 // Session: one BAM + one region set on one device.
 // ---------------------------------------------------------------------------------------------------------------
@@ -433,6 +473,7 @@ public:
         ctx_->ensure_init(dev);
         ctx_->ev_next = 0;
         pool_ = &get_pool(opts_.inflate_threads);
+        res_->dev = dev;
         memset(&tm_, 0, sizeof tm_);
         tm_.n_devices = 1;
     }
@@ -448,8 +489,50 @@ public:
         ctx_->ensure_init(dev);
         ctx_->ev_next = 0;
         pool_ = &get_pool(opts_.inflate_threads);
+        res_->dev = dev;
         memset(&tm_, 0, sizeof tm_);
         tm_.n_devices = 1;
+    }
+
+    // A view of a staged session (bsg_stage_view): the resident records, options and device of `st`, the region set `rg`.
+    // view_halo is how far around every region of rg the records are known to be resident (view_halo()).
+    Session(const Session& st, Regions rg, int64_t view_halo)
+        : bamp_(st.bamp_), bam_(*bamp_), opts_(st.opts_), rg_(std::move(rg)), ctx_(st.ctx_), res_(st.res_),
+          is_view_(true), view_halo_(view_halo) {
+        pool_ = &get_pool(opts_.inflate_threads);
+        memset(&tm_, 0, sizeof tm_);
+        tm_.n_devices = 1;
+        tm_.bytes_compressed = st.tm_.bytes_compressed;
+        tm_.bytes_inflated = st.tm_.bytes_inflated;
+        tm_.n_batches = st.tm_.n_batches;
+    }
+
+    // The largest halo `a` around the regions of `rg` for which this staged session holds every record: each region
+    // [loc, loc + width) with width > 0, widened by a on both sides and clamped at 0 as the planner clamps, must lie inside
+    // one of the index queries the open sent (after their merge; the index returns every record that overlaps a query).
+    // INT64_MAX when rg has no non-empty region.  BSG_EARG, naming the 1-based region, when some region has no such a >= 0.
+    int64_t view_halo(const Regions& rg) const {
+        const std::vector<QueryInterval>& q = res_->queries;
+        int64_t halo = INT64_MAX;
+        for (int64_t i = 0; i < rg.R; ++i) {
+            if (rg.width[i] == 0) continue;
+            const int64_t loc = rg.loc[i], end = loc + rg.width[i], p = std::max<int64_t>(0, loc);
+            // the last query on this contig that begins at or before p (the merged queries are disjoint)
+            auto it = std::upper_bound(q.begin(), q.end(), std::make_pair(rg.rid[i], p), [](const std::pair<int32_t, int64_t>& k, const QueryInterval& x) {
+                return k.first != x.rid ? k.first < x.rid : k.second < x.beg;
+            });
+            int64_t a = -1;
+            if (it != q.begin() && (it - 1)->rid == rg.rid[i]) {
+                const QueryInterval& x = *(it - 1);
+                a = x.end - end;
+                if (x.beg > 0) a = std::min(a, loc - x.beg);
+            }
+            if (a < 0)
+                fail(BSG_EARG, "region " + std::to_string(i + 1) + " of the view lies outside what the staged session fetched; "
+                               "stage a session over it (or a wider ext_hint) to count it");
+            halo = std::min(halo, a);
+        }
+        return halo;
     }
 
     // The fetch plan (index queries + BGZF header scan) depends only on the regions and `ext`: it can run on its own
@@ -495,8 +578,8 @@ public:
     void stage(int64_t ext, bool keep_raw) {
         if (ext < 0) fail(BSG_EARG, "negative 'ext' values don't make sense");           // src/bamsignals.cpp:243
         double t0 = now_ms();
-        keep_raw_ = keep_raw;
-        staged_ext_ = ext;
+        res_->keep_raw = keep_raw;
+        res_->staged_ext = ext;
         if (plan_thread_.joinable()) {
             plan_thread_.join();
             if (plan_err_.code) throw plan_err_;
@@ -504,7 +587,8 @@ public:
             t0 = now_ms() - plan_ms_;                    // ms_plan reports the plan's own duration, ms_fetch what follows it
         } else {
             segs_.clear();
-            plan_fetch(bam_, rg_, ext, kSegCBytes, *pool_, &segs_);
+            res_->queries.clear();
+            plan_fetch(bam_, rg_, ext, kSegCBytes, *pool_, &segs_, keep_raw ? &res_->queries : nullptr);
         }
         if (prefault_out_) { prefault_output(prefault_out_, prefault_total_); prefault_out_ = nullptr; }
         // 1 = device inflate, -1 = host zlib pool, 0 = default: device inflate unless the job is tiny.  A device-inflate
@@ -546,14 +630,14 @@ public:
             }
             batches_.push_back(std::move(b));
         }
-        rows_cap_ = (rows_cap + 3) & ~int64_t(3);
+        res_->rows_cap = (rows_cap + 3) & ~int64_t(3);
         tm_.bytes_compressed = int64_t(total_c);
         tm_.bytes_inflated = int64_t(total_bytes);
         tm_.n_batches = int64_t(batches_.size());
         tm_.ms_plan = now_ms() - t0;
         if (getenv("BSG_DEBUG"))
             fprintf(stderr, "[bsg] plan %.1f ms: %zu segments, %zu batches, %.1f MB compressed, %.1f MB inflated, rows_cap %lld\n",
-                    tm_.ms_plan, segs_.size(), batches_.size(), total_c / 1e6, total_bytes / 1e6, (long long)rows_cap_);
+                    tm_.ms_plan, segs_.size(), batches_.size(), total_c / 1e6, total_bytes / 1e6, (long long)res_->rows_cap);
 
         // device + pinned buffers
         DeviceCtx& c = *ctx_;
@@ -563,12 +647,12 @@ public:
         if (keep_raw) {
             size_t tot = 0;
             for (auto& b : batches_) tot += (b->bytes + 64 + 255) & ~255ull;
-            raw_all_.ensure(tot + 64);
-            size_t offs_tot = size_t(rows_cap_) + batches_.size() + 8;
+            res_->raw_all.ensure(tot + 64);
+            size_t offs_tot = size_t(res_->rows_cap) + batches_.size() + 8;
             if (gpu) { offs_tot = 8; for (auto& b : batches_) offs_tot += size_t(b->bytes / kMinRecord) + 2; }
-            offs_all_.ensure(offs_tot * sizeof(uint32_t));
+            res_->offs_all.ensure(offs_tot * sizeof(uint32_t));
         }
-        ensure_table(rows_cap_);
+        ensure_table(res_->rows_cap);
         c.scalars.ensure(sizeof(DeviceScalars));
         BSG_CUDA(cudaMemsetAsync(c.scalars.p, 0, sizeof(DeviceScalars), c.s_comp));
         if (gpu) {
@@ -593,10 +677,17 @@ public:
     // A staged call may only look as far around its regions as the session fetched: the reference widens every index
     // query by `ext` (src/bamsignals.cpp:255-256,457,487); with a smaller halo, reads near the region borders would
     // silently be missing.
+    // A view may look as far as its regions' resident halo (view_halo()).
     void require_ext(int64_t ext) const {
-        if (ext > staged_ext_)
+        if (is_view_) {
+            if (ext > view_halo_)
+                fail(BSG_EARG, "this call needs a halo of " + std::to_string(ext) + " bp around the regions, the staged records reach " +
+                               std::to_string(view_halo_) + " bp around every region of this view");
+            return;
+        }
+        if (ext > res_->staged_ext)
             fail(BSG_EARG, "this call needs a halo of " + std::to_string(ext) + " bp around the regions, the session was staged with ext_hint = " +
-                           std::to_string(staged_ext_));
+                           std::to_string(res_->staged_ext));
     }
 
     // Staged sessions: decode + filter every resident raw batch again (K1) in ONE launch, timed.
@@ -604,10 +695,11 @@ public:
         DeviceCtx& c = *ctx_;
         fused_ = false;
         BSG_CUDA(cudaMemsetAsync(c.scalars.p, 0, sizeof(DeviceScalars), c.s_comp));
-        if (resident_.empty()) return;
+        if (res_->batches.empty()) return;
+        ensure_table(res_->rows_cap);            // (a view's first table-path call on this device)
         Span sp{c.timing_event(), c.timing_event()};
         BSG_CUDA(cudaEventRecord(sp.a, c.s_comp));
-        launch_decode_table(batch_table_.as<DecodeBatch>(), int(resident_.size()), resident_chunks_, table(),
+        launch_decode_table(res_->batch_table.as<DecodeBatch>(), int(res_->batches.size()), res_->chunks, table(),
                             mode == MODE_COVERAGE, ss != 0, fp, c.scalars.as<DeviceScalars>(), c.s_comp);
         BSG_CUDA(cudaEventRecord(sp.b, c.s_comp));
         kt_.decode.push_back(sp); kt_.launches += 1;
@@ -650,13 +742,12 @@ public:
         if (setup_thread_.joinable()) setup_thread_.join();
         stop_streamer(true);
         wait_prefault();
-        if (raw_all_.p || offs_all_.p || batch_table_.p || idx_keys_.p || idx_scal_.p) {
+        if (fused_rng_.p) {
             cudaSetDevice(ctx_->dev);
             cudaDeviceSynchronize();
-            raw_all_.release(); offs_all_.release(); batch_table_.release();
-            idx_keys_.release(); idx_long_key_.release(); idx_long_row_.release(); idx_scal_.release(); fused_rng_.release();
+            fused_rng_.release();
         }
-    }
+    }                                            // res_: the resident records go with the last handle that shares them
 
     // Tiles depend only on the regions and on (mode, binsize, ss, layout): build + upload them before any device
     // work of the call is queued, and keep them for the next call of a staged session.
@@ -784,7 +875,7 @@ public:
     void finish_count() {
         Nvtx r("bsg:finish_count+d2h");
         DeviceCtx& c = *ctx_;
-        cnt_.rows_ready = n_rows_;
+        cnt_.rows_ready = res_->n_rows;
         if (n_tiles_ > cnt_.t_done || runs_.res) count_tiles(cnt_.t_done, n_tiles_);      // runs: also without tiles
         DeviceScalars* sc = c.scalars.as<DeviceScalars>();
         BSG_CUDA(cudaGetLastError());
@@ -809,8 +900,8 @@ public:
         tm_.bytes_d2h = os_bytes_ + scalar_bytes;
         cnt_.active = false;
         const DeviceScalars* hs = c.h_scalars.as<DeviceScalars>();
-        check_status(hs->status | (keep_raw_ ? idx_.status : 0u));     // staged: the resident records' bits, every call
-        tm_.records = n_rows_;
+        check_status(hs->status | (res_->keep_raw ? res_->idx.status : 0u));     // staged: the resident records' bits, every call
+        tm_.records = res_->n_rows;
         tm_.records_kept = 0;
         for (int k = 0; k < kKeptSlots; ++k) tm_.records_kept += int64_t(hs->kept[k * kKeptStride]);
         if (fused_) tm_.records_kept = -1;                              // only the examined rows were filtered
@@ -854,6 +945,7 @@ public:
         return off;
     }
     int device() const { return ctx_->dev; }
+    const BamFile& bam() const { return bam_; }
     int64_t regions() const { return rg_.R; }
 
 private:
@@ -1288,8 +1380,8 @@ private:
     void run_pipeline() {
         DeviceCtx& c = *ctx_;
         const size_t nb = batches_.size();
-        resident_.clear();
-        n_rows_ = 0;
+        res_->batches.clear();
+        res_->n_rows = 0;
         size_t next_submit = 0;
         uint64_t raw_base = 0; int64_t offs_base = 0;
         double h2d_ms = 0;
@@ -1309,13 +1401,13 @@ private:
             if (b->err.code) throw b->err;
             const int slot = int(commit % kSlots);
             const int64_t n = b->n_records;
-            if (n_rows_ + n > rows_cap_) fail(BSG_EFORMAT, "record count exceeds the planned table capacity");
+            if (res_->n_rows + n > res_->rows_cap) fail(BSG_EFORMAT, "record count exceeds the planned table capacity");
             const double t0 = now_ms();
             uint8_t* d_raw; uint32_t* d_offs;
-            if (keep_raw_) {
-                d_raw = raw_all_.as<uint8_t>() + raw_base;
-                d_offs = offs_all_.as<uint32_t>() + offs_base;
-                resident_.push_back(ResidentBatch{raw_base, offs_base, n});
+            if (res_->keep_raw) {
+                d_raw = res_->raw_all.as<uint8_t>() + raw_base;
+                d_offs = res_->offs_all.as<uint32_t>() + offs_base;
+                res_->batches.push_back(ResidentBatch{raw_base, offs_base, n});
                 raw_base += (b->bytes + 64 + 255) & ~255ull;
                 offs_base += n + 1;
             } else {
@@ -1325,21 +1417,21 @@ private:
             BSG_CUDA(cudaMemcpyAsync(d_raw, c.h_raw[slot].p, b->bytes + 16, cudaMemcpyHostToDevice, c.s_copy));
             BSG_CUDA(cudaMemcpyAsync(d_offs, c.h_offs[slot].p, size_t(n + 1) * 4, cudaMemcpyHostToDevice, c.s_copy));
             BSG_CUDA(cudaEventRecord(c.ev_h2d[slot], c.s_copy));
-            if (keep_raw_) {
+            if (res_->keep_raw) {
                 BSG_CUDA(cudaEventRecord(c.ev_free[slot], c.s_copy));
             } else {
                 BSG_CUDA(cudaStreamWaitEvent(c.s_comp, c.ev_h2d[slot], 0));
                 Span sp{c.timing_event(), c.timing_event()};
                 BSG_CUDA(cudaEventRecord(sp.a, c.s_comp));
                 if (!cnt_.active) fail(BSG_EARG, "internal error: streaming decode without a counting call");
-                launch_decode(DecodeBatch{d_raw, d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
+                launch_decode(DecodeBatch{d_raw, d_offs, res_->n_rows, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
                               c.scalars.as<DeviceScalars>(), c.s_comp);
                 BSG_CUDA(cudaEventRecord(sp.b, c.s_comp));
                 BSG_CUDA(cudaEventRecord(c.ev_free[slot], c.s_comp));
                 kt_.decode.push_back(sp); kt_.launches += n > 0;
             }
             h2d_ms += now_ms() - t0;
-            n_rows_ += n;
+            res_->n_rows += n;
         }
         } catch (...) {
             // workers still reference this Session and the staging slots: wait for every submitted batch
@@ -1351,9 +1443,9 @@ private:
             throw;
         }
         BSG_CUDA(cudaStreamSynchronize(c.s_copy));
-        if (keep_raw_) build_resident_table();
+        if (res_->keep_raw) build_resident_table();
         tm_.ms_h2d = h2d_ms;
-        tm_.records = n_rows_;
+        tm_.records = res_->n_rows;
     }
 
     // GPU-inflate pipeline: host ships compressed bytes; inflate, record walk and decode run on the device.
@@ -1368,8 +1460,8 @@ private:
     void run_pipeline_gpu(uint64_t max_batch, size_t max_offs) {
         DeviceCtx& c = *ctx_;
         const size_t nb = batches_.size();
-        resident_.clear();
-        n_rows_ = 0;
+        res_->batches.clear();
+        res_->n_rows = 0;
         const std::vector<uint64_t>& ent = bam_.entry_points();
         uint64_t raw_base = 0; int64_t offs_base = 0;
         struct Up {             // what compute() and finish() need to know about an uploaded batch
@@ -1378,7 +1470,7 @@ private:
         };
         std::vector<Up> ups(nb);
         // the high-priority stream starts behind everything already queued on the compute stream (scalars reset, tiles)
-        hi_prio_ = !keep_raw_;
+        hi_prio_ = !res_->keep_raw;
         BSG_CUDA(cudaEventRecord(c.ev_order, c.s_comp));
         BSG_CUDA(cudaStreamWaitEvent(c.s_hi, c.ev_order, 0));
         std::vector<Span> inflate_spans, walk_spans, h2d_spans, crc_spans;
@@ -1458,9 +1550,9 @@ private:
             c.g_base[slot].ensure(walkers.size() * 4 + 64);
             c.g_wscr[slot].ensure(walk_scratch_words(int(blocks.size()), int(walkers.size())) * 4);
             c.g_spec[slot].ensure(inflate_spec_words(int(blocks.size())) * 4);
-            if (keep_raw_) {
-                up.d_raw = raw_all_.as<uint8_t>() + raw_base;
-                up.d_offs = offs_all_.as<uint32_t>() + offs_base;
+            if (res_->keep_raw) {
+                up.d_raw = res_->raw_all.as<uint8_t>() + raw_base;
+                up.d_offs = res_->offs_all.as<uint32_t>() + offs_base;
             } else {
                 // the raw buffer of the slot may still be read by the decode kernel of batch bi - 2; this batch's inflate
                 // writes it next: a device-side dependency (ev_gfree in compute()), not a reason to hold the upload back
@@ -1550,7 +1642,7 @@ private:
             h2d_spans.push_back(sph);
             nvtxRangePop();
             t_copy += now_ms() - tt;
-            if (keep_raw_) {
+            if (res_->keep_raw) {
                 raw_base += (b->bytes + 64 + 255) & ~255ull;
                 offs_base += int64_t((b->bytes) / kMinRecord) + 2;
             }
@@ -1561,7 +1653,7 @@ private:
             const Up& up = ups[bi];
             nvtxRangePushA("bsg:launch inflate + crc + walk");
             BSG_CUDA(cudaStreamWaitEvent(c.s_comp, c.ev_up[slot], 0));
-            if (!keep_raw_) BSG_CUDA(cudaStreamWaitEvent(c.s_comp, c.ev_gfree[rslot], 0));      // decode (+ CRC) of batch bi - 2
+            if (!res_->keep_raw) BSG_CUDA(cudaStreamWaitEvent(c.s_comp, c.ev_gfree[rslot], 0));      // decode (+ CRC) of batch bi - 2
             Span sp{c.timing_event(), c.timing_event()};
             BSG_CUDA(cudaEventRecord(sp.a, c.s_comp));
             launch_inflate(c.g_blocks[slot].as<InflateBlock>(), up.n_blocks, c.g_comp[slot].as<uint8_t>(), up.d_raw,
@@ -1610,9 +1702,9 @@ private:
             nvtxRangePushA("bsg:decode batch + stream out");
             BSG_CUDA(cudaEventSynchronize(c.ev_total[slot]));
             const int64_t n = int64_t(c.h_total.as<uint32_t>()[slot]);
-            if (n_rows_ + n > rows_cap_) fail(BSG_EFORMAT, "record count exceeds the planned table capacity");
-            if (keep_raw_) {
-                resident_.push_back(ResidentBatch{up.raw_base, up.offs_base, n});
+            if (res_->n_rows + n > res_->rows_cap) fail(BSG_EFORMAT, "record count exceeds the planned table capacity");
+            if (res_->keep_raw) {
+                res_->batches.push_back(ResidentBatch{up.raw_base, up.offs_base, n});
             } else {
                 // decode on the high-priority stream as soon as the walk of this batch is done (ev_total): it goes ahead of
                 // whatever of the next batches has not started yet
@@ -1620,7 +1712,7 @@ private:
                 Span sp{c.timing_event(), c.timing_event()};
                 BSG_CUDA(cudaEventRecord(sp.a, c.s_hi));
                 if (!cnt_.active) fail(BSG_EARG, "internal error: streaming decode without a counting call");
-                launch_decode(DecodeBatch{up.d_raw, up.d_offs, n_rows_, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
+                launch_decode(DecodeBatch{up.d_raw, up.d_offs, res_->n_rows, int32_t(n), 0}, table(), cnt_.mode == MODE_COVERAGE, cnt_.ss != 0, cnt_.fp,
                               c.scalars.as<DeviceScalars>(), c.s_hi);
                 BSG_CUDA(cudaEventRecord(sp.b, c.s_hi));
                 kt_.decode.push_back(sp); kt_.launches += n > 0;
@@ -1634,13 +1726,13 @@ private:
                     // (Polling for the frontier between upload chunks instead of blocking here was measured: no gain.)
                     ReadTable t = table();
                     int32_t* f = c.h_front.as<int32_t>();
-                    launch_publish_pair(t.tid + (n_rows_ + n - 1), t.pos + (n_rows_ + n - 1), f, c.s_hi);      // not a memcpy: see compute()
+                    launch_publish_pair(t.tid + (res_->n_rows + n - 1), t.pos + (res_->n_rows + n - 1), f, c.s_hi);      // not a memcpy: see compute()
                     BSG_CUDA(cudaEventRecord(c.ev_front[0], c.s_hi));
                     BSG_CUDA(cudaEventSynchronize(c.ev_front[0]));
-                    advance(n_rows_ + n, uint32_t(f[0]), f[1]);
+                    advance(res_->n_rows + n, uint32_t(f[0]), f[1]);
                 }
             }
-            n_rows_ += n;
+            res_->n_rows += n;
             nvtxRangePop();
         };
 
@@ -1682,7 +1774,7 @@ private:
             for (size_t k = 0; k < nb && !h2d_spans.empty(); ++k) {
                 fprintf(stderr, "[bsg]   batch %zu: h2d %.2f-%.2f inflate %.2f-%.2f walk %.2f-%.2f", k, rel(h2d_spans[k].a), rel(h2d_spans[k].b),
                         rel(inflate_spans[k].a), rel(inflate_spans[k].b), rel(walk_spans[k].a), rel(walk_spans[k].b));
-                if (!keep_raw_ && k < dec_first + nb && dec_first + k < kt_.decode.size())
+                if (!res_->keep_raw && k < dec_first + nb && dec_first + k < kt_.decode.size())
                     fprintf(stderr, " decode %.2f-%.2f", rel(kt_.decode[dec_first + k].a), rel(kt_.decode[dec_first + k].b));
                 if (k < crc_spans.size()) fprintf(stderr, " crc %.2f-%.2f", rel(crc_spans[k].a), rel(crc_spans[k].b));
                 fprintf(stderr, "\n");
@@ -1694,8 +1786,8 @@ private:
         BSG_CUDA(cudaMemcpyAsync(c.h_scalars.p, c.scalars.p, sizeof(DeviceScalars), cudaMemcpyDeviceToHost, c.s_comp));
         BSG_CUDA(cudaStreamSynchronize(c.s_comp));
         check_status(c.h_scalars.as<DeviceScalars>()->status);
-        if (keep_raw_) build_resident_table();
-        tm_.records = n_rows_;
+        if (res_->keep_raw) build_resident_table();
+        tm_.records = res_->n_rows;
     }
 
     void build_resident_table() {
@@ -1703,17 +1795,17 @@ private:
         std::vector<DecodeBatch> tab;
         int chunks = 0;
         int64_t row0 = 0;
-        for (auto& rb : resident_) {
+        for (auto& rb : res_->batches) {
             if (rb.n > 0) {
-                tab.push_back(DecodeBatch{raw_all_.as<uint8_t>() + rb.raw_base, offs_all_.as<uint32_t>() + rb.offs_base, row0, int32_t(rb.n), chunks});
+                tab.push_back(DecodeBatch{res_->raw_all.as<uint8_t>() + rb.raw_base, res_->offs_all.as<uint32_t>() + rb.offs_base, row0, int32_t(rb.n), chunks});
                 chunks += int((rb.n + kDecodeChunk - 1) / kDecodeChunk);
             }
             row0 += rb.n;
         }
-        resident_.resize(tab.size());
-        resident_chunks_ = chunks;
-        batch_table_.ensure(tab.size() * sizeof(DecodeBatch) + 64);
-        if (!tab.empty()) BSG_CUDA(cudaMemcpy(batch_table_.p, tab.data(), tab.size() * sizeof(DecodeBatch), cudaMemcpyHostToDevice));
+        res_->batches.resize(tab.size());
+        res_->chunks = chunks;
+        res_->batch_table.ensure(tab.size() * sizeof(DecodeBatch) + 64);
+        if (!tab.empty()) BSG_CUDA(cudaMemcpy(res_->batch_table.p, tab.data(), tab.size() * sizeof(DecodeBatch), cudaMemcpyHostToDevice));
         BSG_CUDA(cudaStreamSynchronize(c.s_comp));
         build_resident_index(row0);
     }
@@ -1728,54 +1820,54 @@ private:
     // The status bits do not fail the open: every staged call raises them, as K1 does on the table path.
     void build_resident_index(int64_t n_rows) {
         DeviceCtx& c = *ctx_;
-        idx_ = ResidentIndexHost();
-        const int nb = int(resident_.size());
+        res_->idx = ResidentIndexHost();
+        const int nb = int(res_->batches.size());
         if (n_rows <= 0 || nb == 0) return;
-        idx_.n = n_rows;
+        res_->idx.n = n_rows;
         const int64_t n_keys = (n_rows + kIndexStride - 1) / kIndexStride;
-        idx_keys_.ensure(size_t(n_keys) * sizeof(uint64_t));
-        idx_scal_.ensure(sizeof(IndexScalars));
-        IndexScalars* isc = idx_scal_.as<IndexScalars>();
+        res_->idx_keys.ensure(size_t(n_keys) * sizeof(uint64_t));
+        res_->idx_scal.ensure(sizeof(IndexScalars));
+        IndexScalars* isc = res_->idx_scal.as<IndexScalars>();
         cudaStream_t st = c.s_comp;
         Span sp0{c.timing_event(), c.timing_event()};
         BSG_CUDA(cudaMemsetAsync(isc, 0, sizeof(IndexScalars), st));
         BSG_CUDA(cudaEventRecord(sp0.a, st));
-        launch_resident_index(batch_table_.as<DecodeBatch>(), nb, resident_chunks_, 0, 0, idx_keys_.as<unsigned long long>(), nullptr,
+        launch_resident_index(res_->batch_table.as<DecodeBatch>(), nb, res_->chunks, 0, 0, res_->idx_keys.as<unsigned long long>(), nullptr,
                               nullptr, isc, st);
         BSG_CUDA(cudaEventRecord(sp0.b, st));
         kt_.decode.push_back(sp0); kt_.launches += 1;
         IndexScalars hs;
         BSG_CUDA(cudaMemcpyAsync(&hs, isc, sizeof hs, cudaMemcpyDeviceToHost, st));
         BSG_CUDA(cudaStreamSynchronize(st));
-        idx_.n_keys = n_keys;
-        idx_.status = hs.status;
-        idx_.reach = int64_t(hs.reach);
+        res_->idx.n_keys = n_keys;
+        res_->idx.status = hs.status;
+        res_->idx.reach = int64_t(hs.reach);
         int k = 6;
         for (; k < kSpanBuckets; ++k) {
             uint64_t above = 0;
             for (int b = k; b < kSpanBuckets; ++b) above += hs.bucket_n[b];
             if (above * 64 <= uint64_t(n_rows)) break;
         }
-        idx_.long_span = k < kSpanBuckets ? (1u << k) - 1u : ~0u;
+        res_->idx.long_span = k < kSpanBuckets ? (1u << k) - 1u : ~0u;
         uint64_t n_long = 0;
         for (int b = 0; b < kSpanBuckets; ++b) {
-            if (b < k) idx_.short_max = std::max(idx_.short_max, int64_t(hs.bucket_max[b]));
-            else { idx_.long_max = std::max(idx_.long_max, int64_t(hs.bucket_max[b])); n_long += hs.bucket_n[b]; }
+            if (b < k) res_->idx.short_max = std::max(res_->idx.short_max, int64_t(hs.bucket_max[b]));
+            else { res_->idx.long_max = std::max(res_->idx.long_max, int64_t(hs.bucket_max[b])); n_long += hs.bucket_n[b]; }
         }
         if (n_long) {
-            idx_long_key_.ensure(size_t(n_long) * sizeof(uint64_t));
-            idx_long_row_.ensure(size_t(n_long) * sizeof(int2));
+            res_->idx_long_key.ensure(size_t(n_long) * sizeof(uint64_t));
+            res_->idx_long_row.ensure(size_t(n_long) * sizeof(int2));
             Span sp1{c.timing_event(), c.timing_event()};
             BSG_CUDA(cudaMemsetAsync(&isc->n_long, 0, sizeof(uint32_t), st));
             BSG_CUDA(cudaEventRecord(sp1.a, st));
-            launch_resident_index(batch_table_.as<DecodeBatch>(), nb, resident_chunks_, 1, idx_.long_span, nullptr,
-                                  idx_long_key_.as<unsigned long long>(), idx_long_row_.as<int2>(), isc, st);
+            launch_resident_index(res_->batch_table.as<DecodeBatch>(), nb, res_->chunks, 1, res_->idx.long_span, nullptr,
+                                  res_->idx_long_key.as<unsigned long long>(), res_->idx_long_row.as<int2>(), isc, st);
             BSG_CUDA(cudaEventRecord(sp1.b, st));
             kt_.decode.push_back(sp1); kt_.launches += 1;
             std::vector<uint64_t> lk(n_long);
             std::vector<int2> lr(n_long);
-            BSG_CUDA(cudaMemcpyAsync(lk.data(), idx_long_key_.p, n_long * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            BSG_CUDA(cudaMemcpyAsync(lr.data(), idx_long_row_.p, n_long * sizeof(int2), cudaMemcpyDeviceToHost, st));
+            BSG_CUDA(cudaMemcpyAsync(lk.data(), res_->idx_long_key.p, n_long * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+            BSG_CUDA(cudaMemcpyAsync(lr.data(), res_->idx_long_row.p, n_long * sizeof(int2), cudaMemcpyDeviceToHost, st));
             BSG_CUDA(cudaStreamSynchronize(st));
             // pass 1 appends in CTA completion order: sort into row order (key, then batch and record for equal keys)
             std::vector<uint32_t> ord(n_long);
@@ -1787,15 +1879,15 @@ private:
             std::vector<uint64_t> keys(n_long);
             std::vector<int2> rows(n_long);
             for (size_t j = 0; j < n_long; ++j) { keys[j] = lk[ord[j]]; rows[j] = lr[ord[j]]; }
-            idx_.n_long = int64_t(n_long);
-            BSG_CUDA(cudaMemcpy(idx_long_key_.p, keys.data(), n_long * sizeof(uint64_t), cudaMemcpyHostToDevice));
-            BSG_CUDA(cudaMemcpy(idx_long_row_.p, rows.data(), n_long * sizeof(int2), cudaMemcpyHostToDevice));
+            res_->idx.n_long = int64_t(n_long);
+            BSG_CUDA(cudaMemcpy(res_->idx_long_key.p, keys.data(), n_long * sizeof(uint64_t), cudaMemcpyHostToDevice));
+            BSG_CUDA(cudaMemcpy(res_->idx_long_row.p, rows.data(), n_long * sizeof(int2), cudaMemcpyHostToDevice));
         }
     }
 
     ResidentView resident_view() const {
-        return ResidentView{batch_table_.as<DecodeBatch>(), int(resident_.size()), idx_.n, idx_keys_.as<unsigned long long>(),
-                            idx_.n_keys, idx_long_key_.as<unsigned long long>(), idx_long_row_.as<int2>(), idx_.n_long, idx_.long_span};
+        return ResidentView{res_->batch_table.as<DecodeBatch>(), int(res_->batches.size()), res_->idx.n, res_->idx_keys.as<unsigned long long>(),
+                            res_->idx.n_keys, res_->idx_long_key.as<unsigned long long>(), res_->idx_long_row.as<int2>(), res_->idx.n_long, res_->idx.long_span};
     }
 
     // Key ranges around a tile that hold every read the call can count there, in int64 from the session's spans and the
@@ -1812,14 +1904,14 @@ private:
             omax = amax / 2 + p.shift;
         }
         const int64_t big = int64_t(1) << 40;
-        if (std::max(std::abs(omin), std::abs(omax)) + idx_.reach + 2 > INT32_MAX) return FusedHalos{big, big, big, big};
+        if (std::max(std::abs(omin), std::abs(omax)) + res_->idx.reach + 2 > INT32_MAX) return FusedHalos{big, big, big, big};
         auto halo = [&](int64_t smax, int64_t* lo, int64_t* hi) {
             *lo = std::max(omax, std::max<int64_t>(smax, 1) - 1 - omin);
             *hi = std::max(-omin, omax);
         };
         FusedHalos h;
-        halo(idx_.short_max, &h.s_lo, &h.s_hi);
-        halo(idx_.long_max, &h.l_lo, &h.l_hi);
+        halo(res_->idx.short_max, &h.s_lo, &h.s_hi);
+        halo(res_->idx.long_max, &h.l_lo, &h.l_hi);
         return h;
     }
 
@@ -1853,7 +1945,7 @@ public:
         FusedHalos h{};
         if (scheme != 1) {
             h = fused_halos(fp);
-            if (scheme != 2) fused = double(fused_rows_estimate(h)) <= kFusedShare * double(idx_.n);
+            if (scheme != 2) fused = double(fused_rows_estimate(h)) <= kFusedShare * double(res_->idx.n);
         }
         if (!fused) { decode_resident(mode, fp); return; }
         BSG_CUDA(cudaMemsetAsync(ctx_->scalars.p, 0, sizeof(DeviceScalars), ctx_->s_comp));
@@ -1862,17 +1954,6 @@ public:
     }
 
 private:
-    struct ResidentIndexHost {
-        int64_t n = 0;                          // resident rows
-        uint32_t status = 0;                    // STATUS_* bits of the resident records
-        int64_t reach = 0;                      // max(pos + span)
-        uint32_t long_span = ~0u;               // T: rows with span > T are on the long list
-        int64_t short_max = 0, long_max = 0;    // largest span at most T / above T
-        int64_t n_keys = 0, n_long = 0;         // sampled keys (device), long-list rows (device)
-    };
-
-    struct ResidentBatch { uint64_t raw_base; int64_t offs_base; int64_t n; };
-
     std::thread setup_thread_;
     Error setup_err_{0, ""};
     int32_t* prefault_out_ = nullptr;
@@ -1885,20 +1966,16 @@ private:
     Pool* pool_ = nullptr;
     std::vector<Segment> segs_;
     std::vector<std::unique_ptr<Batch>> batches_;
-    std::vector<ResidentBatch> resident_;
-    DevBuf raw_all_, offs_all_, batch_table_;   // a staged session OWNS its resident raw bytes, offsets and batch table
+    std::shared_ptr<StagedRecords> res_ = std::make_shared<StagedRecords>();
+    bool is_view_ = false;
+    int64_t view_halo_ = 0;
     uint64_t my_tiles_gen_ = 0;
-    int64_t rows_cap_ = 0, n_rows_ = 0;
-    bool keep_raw_ = false;
-    int64_t staged_ext_ = 0;
     std::thread plan_thread_;
     Error plan_err_{0, ""};
     int64_t plan_ext_ = 0;
     double plan_ms_ = 0;
-    int resident_chunks_ = 0;
     // the fused pileup step of staged sessions (build_resident_index, prepare_resident_pileup)
-    ResidentIndexHost idx_;
-    DevBuf idx_keys_, idx_long_key_, idx_long_row_, idx_scal_, fused_rng_;
+    DevBuf fused_rng_;
     bool fused_ = false;                 // this call counts through K3f + K4f
     FusedHalos fused_h_{};
     struct EstEntry { uint64_t gen; FusedHalos h; int64_t rows; };
@@ -2340,6 +2417,27 @@ int bsg_stage_open(bsg_stage** st, const char* bampath, int64_t R, const char* c
         h->s->kick_page_locking();
         g_stages.push_back(h.get());
         *st = h.release();
+    });
+}
+
+int bsg_stage_view(bsg_stage** view, const bsg_stage* st, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                   const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand) {
+    if (!view) { g_err = "null view pointer"; return BSG_EARG; }
+    *view = nullptr;
+    if (!st) { g_err = "null stage"; return BSG_EARG; }
+    return guarded([&] {
+        if (!st->s) fail(BSG_EARG, "this staged session was ended by bsg_shutdown()");
+        const double t0 = now_ms();
+        const Session& s = *st->s;
+        Regions rg;
+        resolve_regions(s.bam(), R, seq_levels, n_levels, seq_idx, loc, width, strand, &rg);
+        const int64_t halo = s.view_halo(rg);
+        auto h = std::make_unique<bsg_stage>();
+        h->s.reset(new Session(s, std::move(rg), halo));
+        memset(&g_tm, 0, sizeof g_tm);
+        g_tm.ms_total = now_ms() - t0;
+        g_stages.push_back(h.get());
+        *view = h.release();
     });
 }
 

@@ -162,11 +162,11 @@ void scan_segments(const BamFile& bam, Segment* segs, int64_t a, int64_t b) {
 }  // namespace
 
 void plan_fetch(const BamFile& bam, const Regions& rg, int64_t ext, uint64_t seg_cbytes, Pool& pool,
-                std::vector<Segment>* segs) {
+                std::vector<Segment>* segs, std::vector<QueryInterval>* queries) {
     const bool dbg = getenv("BSG_DEBUG") != nullptr;
     double t0 = now_ms();
     auto lap = [&](const char* what) { if (dbg) { const double t = now_ms(); fprintf(stderr, "[bsg]   plan: %s %.1f ms\n", what, t - t0); t0 = t; } };
-    struct Q { int32_t rid; int64_t beg, end; };
+    using Q = QueryInterval;
     std::vector<Q> qs;
     qs.reserve(rg.R);
     for (int64_t i : rg.sorted_order()) {                        // (rid, loc) order == (rid, beg) order: ext is constant
@@ -183,6 +183,7 @@ void plan_fetch(const BamFile& bam, const Regions& rg, int64_t ext, uint64_t seg
         const int64_t gap = 16384;
         for (; j < qs.size() && qs[j].rid == cur.rid && qs[j].beg <= cur.end + gap; ++j) cur.end = std::max(cur.end, qs[j].end);
         bam.query(cur.rid, cur.beg, cur.end, &ranges);
+        if (queries) queries->push_back(cur);
         i = j;
     }
     lap("index queries");

@@ -49,9 +49,16 @@ struct Segment {            // an independently inflatable + walkable piece of t
     uint64_t csize = 0;                // compressed bytes
 };
 
+struct QueryInterval {      // one index query of the planner, after the merge: [beg, end) on contig rid
+    int32_t rid;
+    int64_t beg, end;
+};
+
 // Regions (+/- ext) -> merged index queries -> record-aligned virtual-offset ranges -> segments of roughly
 // seg_cbytes compressed bytes, cut at index entry points; BGZF block headers are scanned on the pool.
+// queries (optional) receives the merged index queries in (rid, beg) order: every record that overlaps one of them
+// is inside the planned segments.
 void plan_fetch(const BamFile& bam, const Regions& rg, int64_t ext, uint64_t seg_cbytes, Pool& pool,
-                std::vector<Segment>* segs);
+                std::vector<Segment>* segs, std::vector<QueryInterval>* queries = nullptr);
 
 }  // namespace bsg

@@ -195,6 +195,27 @@ int bsg_coverage_staged_device(bsg_stage* st, const int32_t* tlen_filter, int32_
                                int32_t filteredF, int32_t tspan, int32_t* d_out, const int64_t* out_offsets, void* stream);
 void bsg_stage_close(bsg_stage* st);
 
+/* ---- region views of a staged session: count another region set against the same resident records ----------------
+ * bsg_stage_view() binds the region set (the region arrays of bsg_stage_open) to the records `st` already holds on the
+ * device.  It reads no BAM or index bytes and launches nothing: names are looked up in the BAM header the session
+ * holds (BSG_ENOCHROM with the reference's message for an unknown name, BSG_EARG for malformed region arrays).  *view
+ * is a bsg_stage handle: every bsg_*_staged* entry point accepts it as it accepts the session it came from, with the
+ * session's options and device.  `st` may itself be a view; its view counts the same resident records.
+ * Coverage rule.  The session records the index queries its open sent (each region +/- ext_hint, clamped at 0, with
+ * queries less than 16 kb apart merged into one): every record overlapping such a query is resident.  A view region
+ * with width > 0 needs a halo a >= 0 such that [max(0, loc - a), loc + width + a) lies inside one query; a view with a
+ * region that has none is refused with BSG_EARG, naming the 1-based region.  The view's halo is the smallest a over its
+ * regions (unbounded without non-empty regions), and a staged call on the view that needs more (the ext of
+ * bsg_stage_open's ext_hint rule: |shift| + tlen_filter[1] with pe_mid for pileups, tlen_filter[1] with tspan for
+ * coverage) is BSG_EARG instead of silently missing reads.
+ * Lifetime.  A session and its views share the resident records: bsg_stage_close() on any handle frees that handle's own
+ * tables, and the resident device memory goes with the last handle, in whatever order they are closed.
+ * bsg_shutdown() ends views as it ends sessions (later calls BSG_EARG, bsg_stage_close stays valid).
+ * Cost.  A view owns only its tile table and per-call scratch on the device; its calls report the session's
+ * bytes_compressed, bytes_inflated and n_batches.  bsg_stage_view itself reports only ms_total. */
+int bsg_stage_view(bsg_stage** view, const bsg_stage* st, int64_t R, const char* const* seq_levels, int32_t n_levels,
+                   const int32_t* seq_idx, const int32_t* loc, const int32_t* width, const int8_t* strand);
+
 /* ---- bamCoverage as runs: run-length (length, value) pairs counted on the GPU ------------------------------------------
  * Coverage is piecewise constant; these calls return it as runs instead of one int32 per base, without ever holding the
  * dense result.  Region i's coverage, in region orientation (a '-' region's runs describe the reversed vector), is
